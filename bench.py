@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 3                # our arm, 1 GPU
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N   # our arm, N GPUs (weak scaling)
     python bench.py --impl reference --steps K --warmup W          # the reference's CPU path (oracle port)
+    python bench.py --steps 20 --warmup 3 --dump-outputs DIR       # also writes the last timed call's outputs as DIR/*.npy
 
 Metric (BASELINE.json): PDE-residual query points/sec for forward + Jacobian + residual + backward on the
 0.25 degree configuration (145x257 grid geometry, batch 8, 65 536 query points per sample).  A "step" is one
@@ -234,6 +235,26 @@ def _emit(line):
     os.write(_JSON_FD if _JSON_FD is not None else 1, (json.dumps(line) + "\n").encode())
 
 
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as path/<name>.npy, float64 where the call returns float64 and float32 otherwise, DUMP_BYTES at most
+    in all.  Over that budget the smaller arrays are kept whole and each larger one is replaced by a sample of its flattened
+    elements at sorted indices drawn from a fixed seed, so two runs with the same arguments store the same elements."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    budget = DUMP_BYTES - 1024 * len(arrays)                         # room for the .npy headers
+    for i, (name, a) in enumerate(sorted(arrays.items(), key=lambda kv: (kv[1].nbytes, kv[0]))):
+        share = budget // (len(arrays) - i)
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a)
+        budget -= a.nbytes
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -252,7 +273,14 @@ def main():
     ap.add_argument("--no-sustained", action="store_true", help="skip the 60-step power-capped steady-state timing of the same call")
     ap.add_argument("--no-graph", action="store_true", help="time the eager place_one_batch call instead of its CUDA-graph capture")
     ap.add_argument("--e2e-breakdown", action="store_true", help="print per-phase times of the e2e step to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed call returned on rank 0 (total loss, per-sample loss "
+                         "terms, gradients of the 13 decoder weight tensors) as DIR/<name>.npy, %d MB at most" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     _claim_stdout()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -347,6 +375,14 @@ def main():
     if not (last_total == last_total and abs(last_total) < float("inf")) or abs(last_total - first_total) > 1e-6 * abs(first_total):
         raise SystemExit("timed operator returned loss %r, first call %r" % (last_total, first_total))
     checksum = {"total": last_total, "terms_mean_over_samples": terms_mean, "first_call_total": first_total}
+    if args.dump_outputs and rank == 0:
+        # the gradients are those backward() hands a caller of the last timed call (the call computed them already).  The inputs
+        # are bit-identical from run to run, the outputs are not: the kernels accumulate with atomics, and two runs of the
+        # default workload differed by up to 2.5e-7 of each gradient tensor's largest element (B200, 1000 W power limit)
+        grads = torch.autograd.grad(holder["last_total"], leaves)
+        outs = {"total": holder["last_total"], "terms": holder["last_terms"]}
+        outs.update(("grad_" + n, g) for n, g in zip(Nat.WEIGHT_FIELDS, grads))
+        dump_outputs(args.dump_outputs, {k: v.detach().cpu().numpy() for k, v in outs.items()})
 
     # ---- the same operator SUSTAINED: the B200 runs this call at its board power cap; after ~0.3 s of load the SM clock settles at
     # 1.4-1.5 GHz and a step takes ~8 % longer than in the first 20 steps after idle that `value` is timed over.  Reported beside it. ----
