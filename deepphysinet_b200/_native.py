@@ -61,11 +61,18 @@ class DpnSampler(C.Structure):
                 ("t_step", C.c_double), ("begin_lat", C.c_double), ("deg_per_cell", C.c_double), ("omega", C.c_double)]
 
 
+class DpnLattice(C.Structure):
+    _fields_ = [("nx", C.c_int32), ("ny", C.c_int32), ("nt", C.c_int32), ("pad_", C.c_int32),
+                ("x0", C.c_double), ("y0", C.c_double), ("t0", C.c_double),
+                ("sx", C.c_double), ("sy", C.c_double), ("st", C.c_double)]
+
+
 _lib = None
 
 ABI_VERSION = 2
 EXPORTS = ("dpn_abi_version", "dpn_last_error", "dpn_workspace_bytes", "dpn_pde_fwd_bwd", "dpn_pde_margin_fwd_bwd",
-           "dpn_decoder_fwd", "dpn_decoder_bwd", "dpn_sample_field", "dpn_generate_queries", "dpn_last_launch_count")
+           "dpn_decoder_fwd", "dpn_decoder_bwd", "dpn_sample_field", "dpn_generate_queries", "dpn_last_launch_count",
+           "dpn_lattice_workspace_bytes", "dpn_decoder_lattice")
 
 
 def lib():
@@ -93,6 +100,9 @@ def lib():
                                       C.c_void_p, C.c_size_t, C.c_void_p]
         L.dpn_sample_field.argtypes = [C.POINTER(DpnSampler)] + [C.c_void_p] * 7
         L.dpn_last_launch_count.restype = C.c_int
+        L.dpn_lattice_workspace_bytes.argtypes = [C.POINTER(DpnShape), C.POINTER(C.c_size_t)]
+        L.dpn_decoder_lattice.argtypes = [C.POINTER(DpnShape), C.POINTER(DpnConsts), C.POINTER(DpnLattice), C.POINTER(DpnSampler),
+                                          C.c_void_p, C.POINTER(DpnWeights), C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
         if L.dpn_abi_version() != ABI_VERSION:
             raise RuntimeError("libdpn_b200.so ABI version mismatch")
         _lib = L
@@ -144,8 +154,9 @@ def stream_ptr():
 _ws = {}
 
 
-def workspace(shape: DpnShape, device):
-    """Caller-owned scratch for one library call on the CURRENT stream (torch caching-allocator memory).
+def workspace(shape: DpnShape, device, nbytes=None):
+    """Caller-owned scratch for one library call on the CURRENT stream (torch caching-allocator memory): dpn_workspace_bytes(shape)
+    bytes, or `nbytes` when given (dpn_lattice_workspace_bytes for dpn_decoder_lattice).
 
     * Outside CUDA-graph capture: one buffer per (device, stream), grown on demand.  A dropped buffer returns to the caching
       allocator, which only re-issues it in stream order, so kernels already enqueued on that stream stay safe; two streams
@@ -154,7 +165,10 @@ def workspace(shape: DpnShape, device):
       kernel nodes, so the memory must belong to the graph - it then lives exactly as long as the graph does, whatever later
       eager calls (a larger shape, another mode) do to the cached buffers."""
     need = C.c_size_t(0)
-    check(lib().dpn_workspace_bytes(C.byref(shape), C.byref(need)), "dpn_workspace_bytes")
+    if nbytes is None:
+        check(lib().dpn_workspace_bytes(C.byref(shape), C.byref(need)), "dpn_workspace_bytes")
+    else:
+        need.value = int(nbytes)
     nbytes = max(need.value, 256)
     if device.type == "cuda" and torch.cuda.is_current_stream_capturing():
         return torch.empty(nbytes, dtype=torch.uint8, device=device), need.value

@@ -1,4 +1,5 @@
 // extern "C" surface of libdpn_b200.so (include/dpn_b200.h): argument validation, mode dispatch.
+#include <math.h>
 #include <stdarg.h>
 
 #include <atomic>
@@ -72,11 +73,16 @@ static size_t ws_bytes(const DpnShape& s) {
   return tc::workspace_bytes(tc_chunk(s), s.K, s.B, planes(s));
 }
 
+static size_t lattice_ws_bytes(const DpnShape& s) {
+  if (s.mode == DPN_MODE_FP32) return f32::lattice_workspace_bytes(f32_chunk(s), s.K, s.B);
+  return tc::lattice_workspace_bytes(tc_chunk(s), s.K, s.B, planes(s));
+}
+
 static int dispatch(Job& job, void* stream) {
   g_launches = 0;
   int rc = check_device();
   if (rc) return rc;
-  const size_t need = ws_bytes(job.shape);
+  const size_t need = job.kind == JOB_LATTICE ? lattice_ws_bytes(job.shape) : ws_bytes(job.shape);
   if (!job.workspace || job.workspace_bytes < need) {
     set_error("workspace too small: have %zu bytes, need %zu", job.workspace_bytes, need);
     return DPN_E_WORKSPACE;
@@ -93,15 +99,41 @@ static int dispatch(Job& job, void* stream) {
   return tensor ? tc::run(job, st) : f32::run(job, st);
 }
 
+static int check_weights(const DpnWeights* w) {
+  const void* ws[] = {w->W1, w->b1, w->W2, w->b2, w->e, w->Wd, w->bd, w->Wa, w->ba, w->Wb, w->bb, w->wo, w->bo};
+  for (const void* q : ws)
+    if (!q || (reinterpret_cast<uintptr_t>(q) & 15)) { set_error("a weight pointer is NULL or not 16-byte aligned"); return DPN_E_INVALID; }
+  return 0;
+}
+
 static int check_common(const DpnShape* s, const DpnConsts* c, const DpnPoints* p, const DpnWeights* w) {
   int rc = check_shape(s);
   if (rc) return rc;
   if (!c || !p || !w) { set_error("consts / points / weights is NULL"); return DPN_E_INVALID; }
-  const void* ws[] = {w->W1, w->b1, w->W2, w->b2, w->e, w->Wd, w->bd, w->Wa, w->ba, w->Wb, w->bb, w->wo, w->bo};
-  for (const void* q : ws)
-    if (!q || (reinterpret_cast<uintptr_t>(q) & 15)) { set_error("a weight pointer is NULL or not 16-byte aligned"); return DPN_E_INVALID; }
+  if ((rc = check_weights(w))) return rc;
   if (!p->coord_data) { set_error("coord_data is NULL"); return DPN_E_INVALID; }
   if (!p->coord_pe && !(p->x && p->y && p->t)) { set_error("need either coord_pe or x,y,t"); return DPN_E_INVALID; }
+  return 0;
+}
+
+static bool sampler_ok(const DpnSampler* s) {
+  return s->B > 0 && s->N > 0 && s->Tt >= 2 && s->Hc >= 2 && s->Wc >= 2 && s->cells_per_coarse > 0 && s->t_step > 0 &&
+         s->dx > 0 && s->dy > 0;
+}
+
+// The first and last node of one lattice axis, in fp64, must lie in the coarse stack [0, (n - 1) cell] with the tolerance of
+// sample_point (1e-9 coarse cells); the fp32 box the kernel clamps to is [0, largest float <= the far edge].
+static int check_axis(const char* name, double v0, double step, int n, double cell, int ncoarse, float* lo, float* hi) {
+  const double first = v0, last = v0 + (double)(n - 1) * step, edge = (double)(ncoarse - 1) * cell;
+  constexpr double EPS = 1e-9;
+  if (!(first / cell >= -EPS && last / cell <= (double)(ncoarse - 1) + EPS)) {
+    set_error("dpn_decoder_lattice: lattice %s range [%.9g, %.9g] lies outside the coarse stack [0, %.9g]", name, first, last, edge);
+    return DPN_E_INVALID;
+  }
+  float e = (float)edge;
+  if ((double)e > edge) e = nextafterf(e, 0.f);
+  *lo = 0.f;
+  *hi = e;
   return 0;
 }
 
@@ -191,6 +223,55 @@ int dpn_decoder_bwd(const DpnShape* shape, const DpnConsts* consts, const DpnPoi
   memset(&job, 0, sizeof(job));
   job.kind = JOB_DEC_BWD; job.shape = *shape; job.dc = make_dev_consts(*consts);
   job.pts = pts; job.w = w; job.d_o = d_o; job.grads = grads;
+  job.workspace = workspace; job.workspace_bytes = workspace_bytes;
+  return dispatch(job, cuda_stream);
+}
+
+int dpn_lattice_workspace_bytes(const DpnShape* shape, size_t* bytes) {
+  int rc = check_shape(shape);
+  if (rc) return rc;
+  if (!bytes) { set_error("bytes is NULL"); return DPN_E_INVALID; }
+  *bytes = lattice_ws_bytes(*shape);
+  return 0;
+}
+
+int dpn_decoder_lattice(const DpnShape* shape, const DpnConsts* consts, const DpnLattice* g, const DpnSampler* s,
+                        const float* coarse, const DpnWeights* w, float* out, void* workspace, size_t workspace_bytes,
+                        void* cuda_stream) {
+  int rc = check_shape(shape);
+  if (rc) return rc;
+  if (!consts || !g || !s || !coarse || !w || !out) { set_error("dpn_decoder_lattice: NULL argument"); return DPN_E_INVALID; }
+  if ((rc = check_weights(w))) return rc;
+  if (shape->K != 6) { set_error("dpn_decoder_lattice: needs K = 6 nets (u,v,p,T,q,rho), got %d", shape->K); return DPN_E_INVALID; }
+  if (g->nx <= 0 || g->ny <= 0 || g->nt <= 0) {
+    set_error("dpn_decoder_lattice: lattice sizes must be positive, got nx=%d ny=%d nt=%d", g->nx, g->ny, g->nt);
+    return DPN_E_INVALID;
+  }
+  if (!(g->sx > 0 && g->sy > 0 && g->st > 0) || !isfinite(g->sx) || !isfinite(g->sy) || !isfinite(g->st)) {
+    set_error("dpn_decoder_lattice: lattice spacing must be positive and finite, got sx=%g sy=%g st=%g", g->sx, g->sy, g->st);
+    return DPN_E_INVALID;
+  }
+  const long long n = (long long)g->nx * g->ny * g->nt;
+  if (n > 2147483647LL) { set_error("dpn_decoder_lattice: nx ny nt = %lld nodes does not fit int32", n); return DPN_E_INVALID; }
+  if (n != shape->N) { set_error("dpn_decoder_lattice: shape N = %d but the lattice has nx ny nt = %lld nodes", shape->N, n); return DPN_E_INVALID; }
+  if (!sampler_ok(s)) {
+    set_error("dpn_decoder_lattice: bad sampler shape B=%d N=%d T=%d H=%d W=%d", s->B, s->N, s->Tt, s->Hc, s->Wc);
+    return DPN_E_INVALID;
+  }
+  if (s->B != shape->B || s->N != shape->N) {
+    set_error("dpn_decoder_lattice: sampler B=%d N=%d does not match shape B=%d N=%d", s->B, s->N, shape->B, shape->N);
+    return DPN_E_INVALID;
+  }
+  Job job;
+  memset(&job, 0, sizeof(job));
+  LatticeJob& L = job.lat;
+  if ((rc = check_axis("x", g->x0, g->sx, g->nx, s->dx * s->cells_per_coarse, s->Wc, &L.lo[0], &L.hi[0]))) return rc;
+  if ((rc = check_axis("y", g->y0, g->sy, g->ny, s->dy * s->cells_per_coarse, s->Hc, &L.lo[1], &L.hi[1]))) return rc;
+  if ((rc = check_axis("t", g->t0, g->st, g->nt, s->t_step, s->Tt, &L.lo[2], &L.hi[2]))) return rc;
+  L.g = *g; L.s = *s; L.coarse = coarse;
+  for (int k = 0; k < 6; ++k) { L.sd[k] = (float)consts->std[k]; L.mu[k] = (float)consts->mean[k]; }
+  job.kind = JOB_LATTICE; job.shape = *shape; job.dc = make_dev_consts(*consts);
+  job.w = w; job.o = out;
   job.workspace = workspace; job.workspace_bytes = workspace_bytes;
   return dispatch(job, cuda_stream);
 }

@@ -461,24 +461,37 @@ __global__ void copy_seed_kernel(size_t n, const float* __restrict__ src, float 
 // ------------------------------------------------------------------------------------------------
 static inline size_t al(size_t n) { return (n + 255) & ~(size_t)255; }
 
-Workspace carve(char* base, int P, int Kn, int B) {
+// What a values-only pass touches comes first; what only the reverse sweep, the residual or the backward touches follows.
+// values_only: the prefix plus the staging of the lattice job's per-point inputs (one sample's chunk), in place of the rest.
+Workspace carve(char* base, int P, int Kn, int B, bool values_only = false) {
   Workspace w;
+  memset(&w, 0, sizeof(w));
   size_t off = 0;
   auto take = [&](size_t floats) { float* p = reinterpret_cast<float*>(base + off); off += al(floats * 4); return p; };
   w.pe = take((size_t)P * C);
   w.pe6 = take((size_t)P * C);
   w.o = take((size_t)P * Kn);
-  w.od = take((size_t)P * Kn * 3);
-  w.dov = take((size_t)P * Kn);
-  w.dod = take((size_t)P * Kn * 3);
-  float** hs[] = {&w.H1, &w.CC, &w.GG, &w.UM, &w.YT, &w.QM, &w.HT, &w.CT, &w.ZH, &w.ZC, &w.GZ};
-  for (auto h : hs) *h = take((size_t)Kn * P * H);
-  float** cs[] = {&w.JIN, &w.ZP, &w.ZD};
-  for (auto c : cs) *c = take((size_t)Kn * P * C);
+  float** vs[] = {&w.H1, &w.CC, &w.GG};
+  for (auto h : vs) *h = take((size_t)Kn * P * H);
   w.uvec = take((size_t)Kn * H);
   w.wo2 = take((size_t)Kn * H);
   w.cst = take(Kn);
   w.bsum = take((size_t)B * Kn * H);
+  if (values_only) {
+    w.lx = take(P);
+    w.ly = take(P);
+    w.lt = take(P);
+    w.lcd = take((size_t)P * 6);
+    w.bytes = off;
+    return w;
+  }
+  w.od = take((size_t)P * Kn * 3);
+  w.dov = take((size_t)P * Kn);
+  w.dod = take((size_t)P * Kn * 3);
+  float** hs[] = {&w.UM, &w.YT, &w.QM, &w.HT, &w.CT, &w.ZH, &w.ZC, &w.GZ};
+  for (auto h : hs) *h = take((size_t)Kn * P * H);
+  float** cs[] = {&w.JIN, &w.ZP, &w.ZD};
+  for (auto c : cs) *c = take((size_t)Kn * P * C);
   w.vc = take((size_t)Kn * H);
   w.vg = take((size_t)Kn * H);
   w.sdo = take(Kn);
@@ -487,6 +500,7 @@ Workspace carve(char* base, int P, int Kn, int B) {
 }
 
 size_t workspace_bytes(int P, int Kn, int B) { return carve(nullptr, P, Kn, B).bytes; }
+size_t lattice_workspace_bytes(int P, int Kn, int B) { return carve(nullptr, P, Kn, B, true).bytes; }
 
 // ------------------------------------------------------------------------------------------------
 // Driver
@@ -504,7 +518,8 @@ int run(const Job& J, cudaStream_t st) {
   const int B = J.shape.B, N = J.shape.N, Kn = J.shape.K;
   const int chunk = J.chunk;
   const DevConsts& DC = J.dc;
-  Workspace w = carve(reinterpret_cast<char*>(J.workspace), chunk, Kn, B);
+  const bool lattice = J.kind == JOB_LATTICE;
+  Workspace w = carve(reinterpret_cast<char*>(J.workspace), chunk, Kn, B, lattice);
   const DpnWeights& Wt = *J.w;
   const bool pde = J.kind == JOB_PDE;
   const bool want_bwd = J.grads != nullptr;
@@ -541,7 +556,11 @@ int run(const Job& J, cudaStream_t st) {
       const size_t sH = (size_t)P * H, sC = (size_t)P * C;
       const unsigned gp = (P + 7) / 8;
       const float* pe = w.pe;
-      if (J.pts->coord_pe) {
+      int rc;
+      if (lattice) {                                                 // staged inputs of this (sample, chunk)
+        if ((rc = launch_lattice(J.lat, b, 1, p0, P, w.lx, w.ly, w.lt, w.lcd, st))) return rc;
+        encode_kernel<<<gp, pb, 0, st>>>(DC, P, w.lx, w.ly, w.lt, w.lcd, w.pe, w.pe6);
+      } else if (J.pts->coord_pe) {
         pe = J.pts->coord_pe + q0 * C;
         encode_kernel<<<gp, pb, 0, st>>>(DC, P, nullptr, nullptr, nullptr, J.pts->coord_data + q0 * 6, nullptr, w.pe6);
       } else {
@@ -549,7 +568,6 @@ int run(const Job& J, cudaStream_t st) {
                                          J.pts->coord_data + q0 * 6, w.pe, w.pe6);
       }
       DPN_LAUNCH_OK();
-      int rc;
       // G1: H1 = relu(PE W1^T + b1)
       Gemm g = mk(P, H, C, pe, C, 0, Wt.W1 + gW1, C, (size_t)H * C, w.H1, sH);
       g.bias = Wt.b1 + gb; g.sBias = H; g.relu = 1;
@@ -567,11 +585,12 @@ int run(const Job& J, cudaStream_t st) {
       if ((rc = launch_gemm(g, NT, Kn, st))) return rc;
       // outputs
       float* o_dst = (J.kind == JOB_DEC_FWD) ? J.o + q0 * Kn : w.o;
-      const float* ref = J.pts->ref ? J.pts->ref + q0 * Kn : J.pts->coord_data + q0 * 6;
-      const int ref_ld = J.pts->ref ? Kn : 6;
+      const float* ref = lattice ? w.lcd : (J.pts->ref ? J.pts->ref + q0 * Kn : J.pts->coord_data + q0 * 6);
+      const int ref_ld = !lattice && J.pts->ref ? Kn : 6;
       out_kernel<<<dim3(gp, Kn), pb, 0, st>>>(P, Kn, w.CC, w.GG, w.wo2, w.uvec, w.cst, ref, ref_ld, o_dst,
                                               need_sweep ? w.UM : nullptr);
       DPN_LAUNCH_OK();
+      if (lattice && (rc = launch_lattice_emit(J.lat, 1, P, w.o, (size_t)P, J.o + q0 * 6, (size_t)N * 6, st))) return rc;
       if (!need_sweep) continue;
       // G4: YT = UM Wa + 2wo ; G5: QM = (YT W2) * [H1>0] ; G6: JIN = QM W1
       g = mk(P, H, H, w.UM, H, sH, Wt.Wa, H, (size_t)H * H, w.YT, sH);

@@ -4,7 +4,21 @@
 
 namespace dpn {
 
-enum JobKind { JOB_PDE = 0, JOB_DEC_FWD = 1, JOB_DEC_BWD = 2 };
+enum JobKind { JOB_PDE = 0, JOB_DEC_FWD = 1, JOB_DEC_BWD = 2, JOB_LATTICE = 3 };
+
+// dpn_decoder_lattice, validated by dpn_api.cu: the lattice, the coarse stack it samples and the de-normalisation of the output.
+struct LatticeJob {
+  DpnLattice g;
+  DpnSampler s;
+  const float* coarse;       // [B][Tt][Hc][Wc][6]
+  float lo[3], hi[3];        // x, y, t are clamped to this fp32 box inside the coarse stack (the validated domain)
+  float sd[6], mu[6];        // std, mean rounded double -> fp32: out = o * sd + mu with two roundings, as torch's o * std + mean
+};
+
+// Per chunk (dpn_sampler.cu): staged x, y, t [nb][P] and coord_data [nb][P][6] of nodes p0 .. p0 + P - 1 of samples b0 .. b0 + nb - 1;
+// then out[b * out_bstride + p * 6 + k] = o[(b * srow + p) * 6 + k] * sd[k] + mu[k] for the same nodes (out at sample b0, node p0).
+int launch_lattice(const LatticeJob& L, int b0, int nb, int p0, int P, float* x, float* y, float* t, float* coord_data, cudaStream_t st);
+int launch_lattice_emit(const LatticeJob& L, int nb, int P, const float* o, size_t srow, float* out, size_t out_bstride, cudaStream_t st);
 
 // One library call, validated and normalised by dpn_api.cu.
 struct Job {
@@ -16,7 +30,8 @@ struct Job {
   const DpnPdeOut* out;     // JOB_PDE
   const DpnMargin* margin;  // JOB_PDE, optional: supervised SmoothL1 data loss on the same points
   const DpnGrads* grads;    // JOB_PDE (optional), JOB_DEC_BWD
-  float* o;                 // JOB_DEC_FWD
+  float* o;                 // JOB_DEC_FWD: normalised [B*N][K];  JOB_LATTICE: physical [B][N][6]
+  LatticeJob lat;           // JOB_LATTICE
   const float* d_o;         // JOB_DEC_BWD
   void* workspace;
   size_t workspace_bytes;
@@ -45,12 +60,14 @@ struct Workspace {
   float *H1, *CC, *GG, *UM, *YT, *QM, *HT, *CT, *ZH, *ZC, *GZ;
   float *JIN, *ZP, *ZD;
   float *uvec, *wo2, *cst, *bsum, *vc, *vg, *sdo;
+  float *lx, *ly, *lt, *lcd;  // lattice staging (values-only carve only)
   size_t bytes;
 };
 
 constexpr int DEFAULT_CHUNK = 16384;
 
 size_t workspace_bytes(int P, int Kn, int B);
+size_t lattice_workspace_bytes(int P, int Kn, int B);
 int launch_gemm(const Gemm& g, int layout, int batches, cudaStream_t st);
 int run(const Job& job, cudaStream_t st);
 

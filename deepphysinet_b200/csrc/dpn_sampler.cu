@@ -3,7 +3,7 @@
 // :406-415 (margin points) and :567-576 (dense grid): point-wise trilinear interpolation of the normalised coarse
 // (1 degree, 6-hourly) field stack at continuous (lon, lat, hour) queries, plus the Coriolis parameter of :521-526.
 // Values only - the reference does not differentiate through this interpolation (SURVEY D1) and neither do we.
-#include "dpn_common.cuh"
+#include "dpn_fp32.cuh"
 
 namespace dpn {
 
@@ -103,6 +103,63 @@ __global__ void __launch_bounds__(256) query_kernel(const DpnQueryGen G, const i
     }
     if (f && valid) f[i] = coriolis(S, yv);
   }
+}
+
+// Lattice inference (dpn_decoder_lattice): one thread per node of a chunk of every sample.  The node's coordinates are computed in
+// fp64 and rounded once to fp32, then clamped into the validated fp32 box: with a spacing that is not representable the last node
+// could otherwise land one ulp outside the coarse stack and sample NaN; at exact lattices the clamp changes nothing.  coord_data
+// comes from the same sample_point as dpn_sample_field's and leaves through the same shared-memory transpose.
+__global__ void __launch_bounds__(256) lattice_kernel(const LatticeJob L, const int b0, const int nb, const int p0, const int P,
+                                                      float* __restrict__ x, float* __restrict__ y, float* __restrict__ t,
+                                                      float* __restrict__ coord_data) {
+  __shared__ float stage[8][32 * 6];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const size_t total = (size_t)nb * P;
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  float acc[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  if (i < total) {
+    const size_t b = i / P, node = (size_t)p0 + (i - b * P);
+    const size_t row = node / L.g.nx;
+    const double ix = (double)(node - row * L.g.nx), iy = (double)(row % L.g.ny), it = (double)(row / L.g.ny);
+    const float xv = fminf(fmaxf((float)__dadd_rn(L.g.x0, __dmul_rn(ix, L.g.sx)), L.lo[0]), L.hi[0]);
+    const float yv = fminf(fmaxf((float)__dadd_rn(L.g.y0, __dmul_rn(iy, L.g.sy)), L.lo[1]), L.hi[1]);
+    const float tv = fminf(fmaxf((float)__dadd_rn(L.g.t0, __dmul_rn(it, L.g.st)), L.lo[2]), L.hi[2]);
+    x[i] = xv; y[i] = yv; t[i] = tv;
+    sample_point(L.s, L.coarse + ((size_t)b0 + b) * L.s.Tt * L.s.Hc * L.s.Wc * 6, xv, yv, tv, acc);
+  }
+#pragma unroll
+  for (int c = 0; c < 6; ++c) stage[warp][lane * 6 + c] = acc[c];
+  __syncwarp();
+  const size_t w0 = ((size_t)blockIdx.x * blockDim.x + warp * 32) * 6;
+#pragma unroll
+  for (int c = 0; c < 6; ++c) {
+    const size_t word = w0 + c * 32 + lane;
+    if (word < total * 6) coord_data[word] = stage[warp][c * 32 + lane];
+  }
+}
+
+// out = o * std + mean, one thread per output word: the chunk's output is contiguous per sample, and so are the rows of o.
+__global__ void __launch_bounds__(256) lattice_emit_kernel(const LatticeJob L, const int nb, const int P, const float* __restrict__ o,
+                                                           const size_t srow, float* __restrict__ out, const size_t out_bstride) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, per = (size_t)P * 6;
+  if (i >= (size_t)nb * per) return;
+  const size_t b = i / per, r = i - b * per;
+  const int k = (int)(r % 6);
+  out[b * out_bstride + r] = __fadd_rn(__fmul_rn(o[b * srow * 6 + r], L.sd[k]), L.mu[k]);
+}
+
+int launch_lattice(const LatticeJob& L, int b0, int nb, int p0, int P, float* x, float* y, float* t, float* coord_data, cudaStream_t st) {
+  const size_t total = (size_t)nb * P;
+  lattice_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(L, b0, nb, p0, P, x, y, t, coord_data);
+  DPN_LAUNCH_OK();
+  return 0;
+}
+
+int launch_lattice_emit(const LatticeJob& L, int nb, int P, const float* o, size_t srow, float* out, size_t out_bstride, cudaStream_t st) {
+  const size_t total = (size_t)nb * P * 6;
+  lattice_emit_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(L, nb, P, o, srow, out, out_bstride);
+  DPN_LAUNCH_OK();
+  return 0;
 }
 
 int run_sampler(const DpnSampler& S, const float* coarse, const float* x, const float* y, const float* t,

@@ -1693,6 +1693,7 @@ __global__ void gather_o_kernel(const Work w, float* __restrict__ o_out) {
 struct Carve {
   uint8_t *img_gen, *img_sta, *pe_blob, *pe6_blob, *blobs;
   float *pet, *o, *od, *dov, *dod, *uvec, *wo2, *cst, *bsum, *vc, *vg, *sdo;
+  float *lx, *ly, *lt, *lcd;    // lattice staging (values-only carve only)
   long long* dbg;
   NetScales* sc;
   int* seedmax;
@@ -1701,8 +1702,11 @@ struct Carve {
 
 static inline size_t al(size_t n) { return (n + 1023) & ~(size_t)1023; }
 
-static Carve carve(uint8_t* base, int chunk, int Kn, int B, int pl) {
+// What a values-only pass (sweep 0) touches comes first; what only the reverse sweep, the residual or the backward touches follows.
+// values_only: the prefix plus the staging of the lattice job's per-point inputs, in place of the rest.
+static Carve carve(uint8_t* base, int chunk, int Kn, int B, int pl, bool values_only = false) {
   Carve c;
+  memset(&c, 0, sizeof(c));
   const size_t T = ((size_t)(chunk + TP - 1) / TP + CLUSTER - 1) / CLUSTER * CLUSTER, rows = (size_t)B * T * TP;
   size_t off = 0;
   auto take = [&](size_t bytes) { uint8_t* p = base + off; off += al(bytes); return p; };
@@ -1711,20 +1715,29 @@ static Carve carve(uint8_t* base, int chunk, int Kn, int B, int pl) {
   c.pe_blob = take((size_t)B * T * BLOB_C * pl);
   c.pe6_blob = take((size_t)B * T * BLOB_C * pl);
   c.pet = reinterpret_cast<float*>(take((size_t)B * T * C * TP * 4));
-  c.blobs = take((size_t)B * Kn * T * (pl == 2 ? Geo<2>::NET_TILE : Geo<1>::NET_TILE));
   c.o = reinterpret_cast<float*>(take(rows * Kn * 4));
-  c.od = reinterpret_cast<float*>(take(rows * Kn * 12));
-  c.dov = reinterpret_cast<float*>(take(rows * Kn * 4));
-  c.dod = reinterpret_cast<float*>(take(rows * Kn * 12));
   c.uvec = reinterpret_cast<float*>(take((size_t)Kn * H * 4));
   c.wo2 = reinterpret_cast<float*>(take((size_t)Kn * H * 4));
   c.cst = reinterpret_cast<float*>(take((size_t)Kn * 4));
   c.bsum = reinterpret_cast<float*>(take((size_t)B * Kn * H * 4));
+  c.dbg = reinterpret_cast<long long*>(take(16 * 8));
+  c.sc = reinterpret_cast<NetScales*>(take((size_t)B * Kn * sizeof(NetScales)));
+  if (values_only) {
+    const size_t pts = (size_t)B * chunk;
+    c.lx = reinterpret_cast<float*>(take(pts * 4));
+    c.ly = reinterpret_cast<float*>(take(pts * 4));
+    c.lt = reinterpret_cast<float*>(take(pts * 4));
+    c.lcd = reinterpret_cast<float*>(take(pts * 24));
+    c.bytes = off;
+    return c;
+  }
+  c.blobs = take((size_t)B * Kn * T * (pl == 2 ? Geo<2>::NET_TILE : Geo<1>::NET_TILE));
+  c.od = reinterpret_cast<float*>(take(rows * Kn * 12));
+  c.dov = reinterpret_cast<float*>(take(rows * Kn * 4));
+  c.dod = reinterpret_cast<float*>(take(rows * Kn * 12));
   c.vc = reinterpret_cast<float*>(take((size_t)Kn * H * 4));
   c.vg = reinterpret_cast<float*>(take((size_t)Kn * H * 4));
   c.sdo = reinterpret_cast<float*>(take((size_t)Kn * 4));
-  c.dbg = reinterpret_cast<long long*>(take(16 * 8));
-  c.sc = reinterpret_cast<NetScales*>(take((size_t)B * Kn * sizeof(NetScales)));
   c.seedmax = reinterpret_cast<int*>(take((size_t)B * Kn * 2 * sizeof(int)));
   c.bytes = off;
   return c;
@@ -1737,6 +1750,7 @@ int default_chunk(int B, int planes) {
 }
 
 size_t workspace_bytes(int chunk, int Kn, int B, int planes) { return carve(nullptr, chunk, Kn, B, planes).bytes; }
+size_t lattice_workspace_bytes(int chunk, int Kn, int B, int planes) { return carve(nullptr, chunk, Kn, B, planes, true).bytes; }
 
 template <int PL, bool F16>
 static int make_images(const DpnWeights& Wt, const Carve& c, int B, int Kn, cudaStream_t st) {
@@ -1778,7 +1792,8 @@ static int run_planes(const Job& J, cudaStream_t st) {
       if (dev >= 0 && dev < 64) attr_done_mask.fetch_or(1ull << dev, std::memory_order_release);
     }
   }
-  Carve c = carve(reinterpret_cast<uint8_t*>(J.workspace), chunk, Kn, B, PL);
+  const bool lattice = J.kind == JOB_LATTICE;
+  Carve c = carve(reinterpret_cast<uint8_t*>(J.workspace), chunk, Kn, B, PL, lattice);
   const DpnWeights& Wt = *J.w;
   const bool pde = J.kind == JOB_PDE;
   const bool want_bwd = J.grads != nullptr;
@@ -1827,7 +1842,16 @@ static int run_planes(const Job& J, cudaStream_t st) {
     w.B = B; w.Kn = Kn; w.T = T; w.P = P; w.N = N; w.p0 = p0;
     w.img_gen = c.img_gen; w.img_sta = c.img_sta;
     w.b1 = Wt.b1; w.bsum = c.bsum; w.ba = Wt.ba; w.uvec = c.uvec; w.wo2 = c.wo2; w.cst = c.cst;
-    w.coord_data = J.pts->coord_data; w.ref = J.pts->ref;
+    const float *px, *py, *pt, *ppe = nullptr;
+    if (lattice) {                                                    // staged inputs of this chunk: [B][P], so q = b P + p_local
+      if ((rc = launch_lattice(J.lat, 0, B, p0, P, c.lx, c.ly, c.lt, c.lcd, st))) return rc;
+      w.N = P; w.p0 = 0;
+      w.coord_data = c.lcd; w.ref = nullptr;
+      px = c.lx; py = c.ly; pt = c.lt;
+    } else {
+      w.coord_data = J.pts->coord_data; w.ref = J.pts->ref;
+      px = J.pts->x; py = J.pts->y; pt = J.pts->t; ppe = J.pts->coord_pe;
+    }
     w.pe_blob = c.pe_blob; w.pe6_blob = c.pe6_blob; w.pet = c.pet; w.blobs = c.blobs;
     w.o = c.o; w.od = c.od; w.dov = c.dov; w.dod = c.dod;
     w.vc = c.vc; w.vg = c.vg; w.sdo = c.sdo;
@@ -1839,7 +1863,7 @@ static int run_planes(const Job& J, cudaStream_t st) {
 #endif
     memcpy(w.band, J.dc.band, sizeof(w.band));
     const int tiles = B * T;
-    encode_kernel<PL, F16><<<tiles, TP, 0, st>>>(J.dc, w, J.pts->x, J.pts->y, J.pts->t, J.pts->coord_pe);
+    encode_kernel<PL, F16><<<tiles, TP, 0, st>>>(J.dc, w, px, py, pt, ppe);
     DPN_LAUNCH_OK();
     if constexpr (PL == 2) {
       if (w.xfirst) pass1_ts_kernel<PL, F16, true><<<tiles, Geo<PL>::THREADS, ts::Cfg<PL>::SMEM, st>>>(w, sweep);
@@ -1848,6 +1872,10 @@ static int run_planes(const Job& J, cudaStream_t st) {
       pass1_ts_kernel<PL, F16, false><<<tiles, Geo<PL>::THREADS, ts::Cfg<PL>::SMEM, st>>>(w, sweep);
     }
     DPN_LAUNCH_OK();
+    if (lattice) {
+      if ((rc = launch_lattice_emit(J.lat, B, P, c.o, (size_t)T * TP, J.o + (size_t)p0 * 6, (size_t)N * 6, st))) return rc;
+      continue;
+    }
     if (J.kind == JOB_DEC_FWD) {
       gather_o_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(w, J.o);
       DPN_LAUNCH_OK();

@@ -10,6 +10,7 @@ constexpr int DEFAULT_POINTS_IN_FLIGHT = 1048576;  // B * chunk * planes: bounds
 
 int default_chunk(int B, int planes);              // points per sample per pass (multiple of 128)
 size_t workspace_bytes(int chunk, int Kn, int B, int planes);
+size_t lattice_workspace_bytes(int chunk, int Kn, int B, int planes);   // the values-only prefix of the carve + lattice staging
 int run(const Job& job, cudaStream_t st);
 
 }  // namespace tc

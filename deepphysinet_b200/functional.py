@@ -289,3 +289,59 @@ def sample_field(coarse, x, y, t, consts: Optional[PhysicsConsts] = None, cells_
     N.check(N.lib().dpn_sample_field(C.byref(S), N.ptr(cz), N.ptr(xs[0]), N.ptr(xs[1]), N.ptr(xs[2]), N.ptr(cd), N.ptr(f),
                                      N.stream_ptr()), "dpn_sample_field")
     return cd, f
+
+
+class Lattice(NamedTuple):
+    """Regular space-time lattice (DpnLattice, include/dpn_b200.h): node (k, j, i) sits at x = x0 + i sx, y = y0 + j sy (metres,
+    the units of pde_residual) and t = t0 + k st (seconds); decoder_lattice returns [B, nt, ny, nx, 6].  A sub-region is a lattice
+    with another origin and fewer nodes, e.g. Lattice.domain(consts, refine=4)._replace(x0=..., nx=...)."""
+    nx: int
+    ny: int
+    nt: int
+    x0: float
+    y0: float
+    t0: float
+    sx: float
+    sy: float
+    st: float
+
+    @classmethod
+    def domain(cls, consts: PhysicsConsts, refine=1, t0=0.0, st=3600.0, nt=25):
+        """The full lat_size x lon_size domain at `refine` times the training spacing, `nt` leads `st` seconds apart from t0."""
+        return cls(nx=(int(consts.lon_size) - 1) * int(refine) + 1, ny=(int(consts.lat_size) - 1) * int(refine) + 1, nt=int(nt),
+                   x0=0.0, y0=0.0, t0=float(t0), sx=float(consts.dx) / refine, sy=float(consts.dy) / refine, st=float(st))
+
+
+@torch.no_grad()
+def decoder_lattice(coarse, W: DecoderWeights, lattice: Lattice, consts: Optional[PhysicsConsts] = None, mode=None,
+                    cells_per_coarse=4.0, t_step=6 * 3600.0):
+    """Physical fields [B, nt, ny, nx, 6] (u,v,p,T,q,rho; inverse_norm without clip, interface_physics.py:533) of the six
+    decoders on `lattice` for the B samples of W, with coord_data sampled from `coarse` [B,Tt,Hc,Wc,6] as sample_field does.
+    One library call: coordinates and coord_data are generated on the GPU per chunk, and the workspace holds a values-only pass.
+    Values only, like sample_field (no grad_fn)."""
+    consts = consts or PhysicsConsts()
+    Bw, K = _check_weights(W)
+    if K != 6:
+        raise ValueError("decoder_lattice needs all six nets (u,v,p,T,q,rho)")
+    cz = _prep(coarse)
+    if cz.dim() != 5 or cz.shape[-1] != 6 or cz.shape[0] != Bw:
+        raise ValueError("coarse must be [B,Tt,Hc,Wc,6] with B = %d samples, got %s" % (Bw, tuple(cz.shape)))
+    g = N.DpnLattice(nx=int(lattice.nx), ny=int(lattice.ny), nt=int(lattice.nt), pad_=0, x0=float(lattice.x0), y0=float(lattice.y0),
+                     t0=float(lattice.t0), sx=float(lattice.sx), sy=float(lattice.sy), st=float(lattice.st))
+    Np = g.nx * g.ny * g.nt
+    if Np >= 2 ** 31:
+        raise ValueError("the lattice has %d nodes per sample; at most 2**31 - 1 fit one call" % Np)
+    _, Tt, Hc, Wc, _ = cz.shape
+    S = N.DpnSampler(B=Bw, N=Np, Tt=Tt, Hc=Hc, Wc=Wc, pad_=0, dx=consts.dx, dy=consts.dy, cells_per_coarse=float(cells_per_coarse),
+                     t_step=float(t_step), begin_lat=0.0, deg_per_cell=0.0, omega=0.0)
+    shape = _shape(Bw, Np, 6, mode or _DEFAULT_MODE)
+    ws = [_prep(w) for w in W]
+    out = torch.empty(Bw, g.nt, g.ny, g.nx, 6, device=cz.device)
+    need = C.c_size_t(0)
+    N.check(N.lib().dpn_lattice_workspace_bytes(C.byref(shape), C.byref(need)), "dpn_lattice_workspace_bytes")
+    with torch.cuda.device(cz.device):
+        wsbuf, nbytes = N.workspace(shape, cz.device, need.value)
+        N.check(N.lib().dpn_decoder_lattice(C.byref(shape), C.byref(N.make_consts(consts)), C.byref(g), C.byref(S), N.ptr(cz),
+                                            C.byref(_weights_struct(ws)), N.ptr(out), N.ptr(wsbuf), nbytes, N.stream_ptr()),
+                "dpn_decoder_lattice")
+    return out

@@ -196,3 +196,13 @@ class InterfacePhysics(nn.Module):
         std = torch.tensor(consts.std, device=dev, dtype=o.dtype)
         phys = o * std + mean
         return phys.reshape(len(time_ids), Ww, Hh, 6).permute(0, 2, 1, 3).contiguous()
+
+    @torch.no_grad()
+    def predict_lattice(self, field_data, coarse, forecast_h, lattice, weights=None):
+        """Lattice inference for B samples at once: physical fields [B, nt, ny, nx, 6] of every sample on `lattice`
+        (functional.Lattice; Lattice.domain(self.consts(...), refine, ...) covers the whole grid at `refine` times the training
+        spacing), coord_data from its own coarse stack coarse[b] [Tt,Hc,Wc,6], inverse_norm without clip as predict_grid.
+        The encoder and hyper-network run once for all samples (or not at all with cached `weights`), then one library call
+        evaluates every node; the workspace holds a values-only pass (dpn_lattice_workspace_bytes)."""
+        W = weights if weights is not None else self.physics_net.decoder_weights(field_data, forecast_h)
+        return Fn.decoder_lattice(coarse, W, lattice, consts=self.consts(self._last_factor()), mode=self.mode)

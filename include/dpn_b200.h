@@ -209,6 +209,34 @@ typedef struct DpnQueryGen {
 int dpn_generate_queries(const DpnQueryGen *g, const DpnSampler *sampler, const float *coarse, float *x, float *y,
                          float *t, float *coord_data, float *f, void *cuda_stream);
 
+/* Lattice inference: the six decoders on a regular space-time lattice, for B samples, as physical fields.  Generalises the
+ * dense forward of interface_physics.py:538-606 and physics_dataset.get_margin_grid :528-588 to any spacing, sub-region and
+ * lead times.  Node (k, j, i) of every sample sits at
+ *   x = x0 + i sx,  y = y0 + j sy  (metres, DpnPoints units),  t = t0 + k st  (seconds);  i < nx, j < ny, k < nt.
+ * Output order is [B, nt, ny, nx, 6]: t slowest, x fastest. */
+typedef struct DpnLattice {
+  int32_t nx, ny, nt, pad_;
+  double x0, y0, t0;
+  double sx, sy, st;
+} DpnLattice;
+
+/* Bytes of device workspace dpn_decoder_lattice needs for this shape: the values-only part of the dpn_workspace_bytes carve
+ * (weight images, coordinate / data features, outputs) plus per-point staging of x, y, t and coord_data - about 2.3 KB per point
+ * in flight in the split modes against 41 KB for dpn_workspace_bytes. */
+int dpn_lattice_workspace_bytes(const DpnShape *shape, size_t *bytes);
+
+/* out[b, k, j, i, :] = o * std + mean (inverse_norm WITHOUT clip, as the reference's dense forward :533) of the six nets at node
+ * (k, j, i) of sample b.  Per chunk of nodes the library generates the coordinates (fp64, rounded once to fp32) and samples
+ * coord_data from coarse [B,Tt,Hc,Wc,6] with dpn_sample_field's interpolation; nothing per point exists on the host.
+ *   shape  B samples, N = nx ny nt (must fit int32), K = 6, any mode; chunk honoured as elsewhere
+ *   s      coarse-stack geometry exactly as in dpn_sample_field; s->B, s->N must equal shape->B, shape->N; Coriolis fields unused
+ *   w      generated weights per sample, as everywhere;  out [B, nt, ny, nx, 6] physical values
+ * DPN_E_INVALID (with dpn_last_error text) for zero sizes, non-positive spacing, a first or last node outside the coarse stack in
+ * x, y or t, B / N mismatches and NULL pointers.  Values only. */
+int dpn_decoder_lattice(const DpnShape *shape, const DpnConsts *consts, const DpnLattice *g, const DpnSampler *s,
+                        const float *coarse, const DpnWeights *w, float *out,
+                        void *workspace, size_t workspace_bytes, void *cuda_stream);
+
 /* Introspection for tests and bench: number of kernels the last call on this thread launched. */
 int dpn_last_launch_count(void);
 
