@@ -246,12 +246,6 @@ __device__ __forceinline__ uint32_t gp_off(const int KC, const int r, const int 
   return (uint32_t)(r >> 5) * (uint32_t)(KC * 512) + (uint32_t)kc * 512u + (uint32_t)(r & 31) * 16u;
 }
 
-__device__ __forceinline__ void mbar_wait_t(uint64_t* bar, uint32_t parity, long long& acc) {
-  const long long t0 = clock64();
-  mbar_wait(bar, parity);
-  acc += clock64() - t0;
-}
-
 // Column sums over the 32 rows a warp owns: after the exchange lane l holds sum_rows v[row][l].  31 shuffles.
 __device__ __forceinline__ float warp_colsum32(float (&v)[32], int lane) {
 #pragma unroll
@@ -274,6 +268,233 @@ __device__ __forceinline__ float warp_colsum32(float (&v)[32], int lane) {
 template <int PL> __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, %0;" ::"n"(Geo<PL>::ET) : "memory"); }   // the epilogue warps only
 
 // ------------------------------------------------------------------------------------------------
+// The tcgen05 pipeline of pass1_ts_kernel and pass2z_kernel (DESIGN.md section 5).  A producer warp streams the K = 16 weight chunks
+// through a ring of stages (`full` / `empty` mbarriers; with a cluster, every chunk is read from L2 once and multicast); one MMA warp
+// issues split contractions; two 256-column TMEM regions are ping-pong accumulators that the epilogue warps convert in place, block
+// by block, into the A operand of the next GEMM (`blk[4]`: block cb of both column halves is converted, one arrival per epilogue
+// warp; `acc_ready[2]`: the GEMM into region 0 / 1 has completed).  A kernel brings its ring geometry (Cfg: NS stages of STAGE bytes,
+// the weight chunk first, W_BYTES at most), its barrier struct (full, empty, blk, acc_ready, tmem_base and whatever only it needs)
+// and its schedule.
+// ------------------------------------------------------------------------------------------------
+namespace pp {
+constexpr uint32_t REGION = 256;                // TMEM columns of one ping-pong region
+constexpr int A_PLANE = 2 * CORE_STRIDE;        // A slice [128 x 16] of one plane that rides in a stage behind its weight chunk: 4 KB
+constexpr uint16_t MC_MASK = (uint16_t)((1u << CLUSTER) - 1);
+static_assert(2 * REGION == 512 && REGION == H, "TMEM map: two [128 x 256] fp32 accumulators, each converted in place into 2 x 16-bit planes");
+// which of the products of a split contraction a chunk issues: all three | exact A operand (B_lo, B_hi) | the two cross terms | the main term
+enum { P_ALL = 0, P_EXACT = 1, P_CROSS = 2, P_MAIN = 3 };
+
+// K-chunk order of a TS-form GEMM: the two epilogue warp groups finish block cb of their column halves together, i.e. chunks
+// 2cb, 2cb+1 (half 0) and 8+2cb, 9+2cb (half 1)
+__host__ __device__ constexpr int block_order(int i) { return ((i >> 2) << 1) + (i & 1) + ((i >> 1) & 1) * 8; }
+// TMEM column of the hi plane of K-chunk c of a converted region a (the lo plane is 16 columns further)
+__device__ __forceinline__ uint32_t chunk_col(uint32_t a, int c) { return a + 32u * (uint32_t)(c >> 1) + 8u * (uint32_t)(c & 1); }
+
+// mbarrier wait; with the cycle counters on (debug builds, DPN_PHASE_DEBUG=1), the cycles spent waiting are added to acc
+__device__ __forceinline__ void wait(uint64_t* bar, uint32_t parity, const bool timed, long long& acc) {
+  if (timed) {
+    const long long t0 = clock64();
+    mbar_wait(bar, parity);
+    acc += clock64() - t0;
+  } else {
+    mbar_wait(bar, parity);
+  }
+}
+
+struct Block {
+  uint32_t tmem;    // base of the 512 TMEM columns
+  uint32_t rank;    // rank of this CTA in its cluster
+};
+// Thread 0 initialises the ring and hand-off barriers (a kernel initialises its own extra barriers before this call), the MMA warp
+// allocates all 512 TMEM columns, and no CTA goes on before the barriers of every CTA of its cluster exist (multicast copies and
+// commits arrive on them).
+template <int PL, int NS, class Pipe>
+__device__ __forceinline__ Block block_start(Pipe& p, const int tid, const int warp) {
+  if (tid == 0) {
+    for (int s = 0; s < NS; ++s) { mbar_init(&p.full[s], 1); mbar_init(&p.empty[s], CLUSTER); }
+    for (int i = 0; i < 4; ++i) mbar_init(&p.blk[i], Geo<PL>::EW);
+    mbar_init(&p.acc_ready[0], 1); mbar_init(&p.acc_ready[1], 1);
+    fence_barrier_init();
+  }
+  if (warp == Geo<PL>::W_MMA) tmem_alloc(&p.tmem_base, 512);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  if (CLUSTER > 1) cluster_sync_all();
+  return Block{p.tmem_base, cluster_ctarank()};
+}
+// No CTA leaves, and no TMEM column is freed, while MMAs or the multicast commits of a peer may still arrive
+template <int PL>
+__device__ __forceinline__ void block_end(const uint32_t tmem, const int warp) {
+  tc_fence_before();
+  __syncthreads();
+  if (CLUSTER > 1) cluster_sync_all();
+  if (warp == Geo<PL>::W_MMA) tmem_dealloc(tmem, 512);
+}
+
+// The weight ring as one warp (producer or MMA issuer) walks it: its stage and that stage's phase
+template <int PL, class Cfg>
+struct Ring {
+  uint8_t* ring;
+  uint64_t *full, *empty;
+  uint32_t rank = 0;                // producer: this CTA's rank in the cluster
+  uint64_t pol = 0;                 // producer: L2 policy of the weights (evict_last: every tile of a sample re-reads them)
+  uint32_t s = 0, ph = 0;
+  __device__ __forceinline__ void advance() { if (++s == Cfg::NS) { s = 0; ph ^= 1; } }
+  // Producer: wait for the stage to be free, then one lane starts the copies into it: the weight chunk wsrc of wbytes (with a cluster,
+  // each CTA fetches 1 / CLUSTER of it and multicasts that slice) and, if asrc, the A slice of the same K-chunk behind it.
+  // hi_only: only the hi planes (the first half of the chunk, one plane of the A slice).
+  __device__ __forceinline__ void put(const uint8_t* wsrc, uint32_t wbytes, const uint8_t* asrc, const bool hi_only = false) {
+    if (hi_only) wbytes /= 2;
+    const int a_planes = hi_only ? 1 : PL;
+    mbar_wait(&empty[s], ph ^ 1);
+    if (elect_one()) {
+      uint8_t* stg = ring + s * Cfg::STAGE;
+      mbar_arrive_expect_tx(&full[s], wbytes + (asrc ? a_planes * A_PLANE : 0));
+      if (CLUSTER == 1) {
+        bulk_g2s_hint(stg, wsrc, wbytes, &full[s], pol);
+      } else {
+        const uint32_t slice = wbytes / CLUSTER;
+        bulk_g2s_mc_hint(stg + rank * slice, wsrc + rank * slice, slice, &full[s], MC_MASK, pol);
+      }
+      if (asrc) {
+        for (int p = 0; p < a_planes; ++p) bulk_g2s_hint(stg + Cfg::W_BYTES + p * A_PLANE, asrc + p * BLOB_C, A_PLANE, &full[s], pol);
+      }
+    }
+    advance();
+  }
+  // MMA issuer (elected lane): the stage is free once the MMAs issued so far have read it, in every CTA of the cluster
+  __device__ __forceinline__ void release() { if (CLUSTER == 1) mma_commit(&empty[s]); else mma_commit_mc(&empty[s], MC_MASK); }
+};
+
+// The MMA warp: consumer of the ring and of the epilogues' converted blocks
+template <int PL, bool F16, class Cfg>
+struct Mma {
+  Ring<PL, Cfg> ring;
+  uint64_t *blk, *acc_ready;
+  uint32_t ring_addr;               // shared-memory address of stage 0
+  bool timed;
+  bool no_mma;                      // debug builds: the barrier protocol without the MMAs
+  uint32_t bp = 0;                  // parity of the blk barriers
+  long long t_full = 0, t_epi = 0;  // cycles waited for weight chunks / for converted blocks
+
+  // One K = 16 chunk: the weights of the next stage (N = Nn) against an A operand, into the accumulator at d.  PL = 2: lo*hi + hi*lo
+  // + hi*hi (`part` selects a subset); PL = 1: one product.
+  // TS form: A planes in tensor memory, hi at a_hi, lo at a_lo.
+  __device__ __forceinline__ void ts(const uint32_t d, const int Nn, const uint32_t a_hi, const uint32_t a_lo, const uint32_t first, const int part = P_ALL) {
+    chunk(Nn, [&](const uint32_t idesc, const uint64_t bd, const uint64_t bl) {
+      if (PL == 1) {
+        mma_ts(d, a_hi, bd, idesc, first);
+      } else {
+        if (part == P_ALL || part == P_CROSS) mma_ts(d, a_lo, bd, idesc, first);   // (an exact 16-bit A operand - the 0 / 1 mask of G4 - has no lo plane)
+        if (part != P_MAIN) mma_ts(d, a_hi, bl, idesc, part == P_EXACT ? first : 1u);
+        if (part != P_CROSS) mma_ts(d, a_hi, bd, idesc, part == P_MAIN ? first : 1u);
+      }
+    });
+  }
+  // SS form: A planes in shared memory, descriptor ad, the lo plane al_off (>> 4) further; in_stage: the A slice rides in the stage
+  // behind the weight chunk, so ad is the descriptor of stage 0's slice.  The hi plane of A is fetched once for its two MMAs.
+  __device__ __forceinline__ void ss(const uint32_t d, const int Nn, const uint64_t a0, const uint32_t al_off, const bool in_stage, const uint32_t first, const int part = P_ALL) {
+    const uint64_t ad = a0 + (in_stage ? ring.s * (uint32_t)(Cfg::STAGE >> 4) : 0u), al = ad + al_off;
+    chunk(Nn, [&](const uint32_t idesc, const uint64_t bd, const uint64_t bl) {
+      if (PL == 1 || part == P_MAIN) {
+        mma_bf16(d, ad, bd, idesc, first);
+      } else {
+        mma_bf16(d, al, bd, idesc, first);
+        if (part == P_CROSS) {
+          mma_bf16(d, ad, bl, idesc, 1u);
+        } else {
+          mma_f16_c<REUSE_A ? A_FILL : A_DISCARD>(d, ad, bl, idesc, 1u);
+          mma_f16_c<REUSE_A ? A_LAST : A_DISCARD>(d, ad, bd, idesc, 1u);
+        }
+      }
+    });
+  }
+  // K = 256 GEMM into d whose A operand is region a, converted in place by the running epilogue: each block as soon as it is converted
+  __device__ __forceinline__ void gemm_ts(const uint32_t d, const uint32_t a, const int Nn, const bool accumulate, const int part = P_ALL) {
+    for (int cb = 0; cb < 4; ++cb) {
+      wait_blk(cb);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int c = 2 * cb + (j & 1) + (j >> 1) * 8;              // block_order(4 cb + j)
+        const uint32_t ah = chunk_col(a, c);
+        ts(d, Nn, ah, ah + 16, (accumulate || cb > 0 || j > 0) ? 1u : 0u, part);
+      }
+    }
+    bp ^= 1u;
+  }
+  __device__ __forceinline__ void wait_blk(const int cb) { wait(&blk[cb], bp, timed, t_epi); tc_fence_after(); }
+  // the GEMM into `region` is complete once the MMAs issued so far are
+  __device__ __forceinline__ void ready(const uint32_t region) { if (elect_one()) mma_commit(&acc_ready[region]); }
+
+  template <class F>
+  __device__ __forceinline__ void chunk(const int Nn, F&& mmas) {
+    const uint32_t idesc = idesc_16(F16, Nn, 0, 0, 128);
+    const uint64_t b_base = smem_desc(ring_addr, Nn * 16, 128);
+    const uint32_t b_lo = (uint32_t)(Nn * 32) >> 4;
+    wait(&ring.full[ring.s], ring.ph, timed, t_full);
+    tc_fence_after();
+    const uint64_t bd = b_base + ring.s * (uint32_t)(Cfg::STAGE >> 4), bl = bd + b_lo;
+    if (elect_one()) {
+      if (!no_mma) mmas(idesc, bd, bl);
+      ring.release();
+    }
+    ring.advance();
+  }
+};
+
+// An epilogue thread (point r of the tile = TMEM lane, one column half): its side of the hand-offs
+template <int PL, bool F16>
+struct Epi {
+  uint64_t *blk, *acc_ready;
+  uint32_t lane_base;               // this warp's TMEM lanes, column 0
+  int r, lane;
+  bool timed;
+  bool no_stores;                   // debug builds: no workspace tile stores
+  uint32_t ar0 = 0, ar1 = 0;        // waits on acc_ready[0] / [1] so far
+  long long t_acc = 0;              // cycles waited for accumulators
+
+  // waits for the GEMM into `region`; returns this thread's lane address of that region
+  __device__ __forceinline__ uint32_t acc_wait(const uint32_t region) {
+    const uint32_t par = (region ? ar1 : ar0) & 1u;
+    wait(&acc_ready[region], par, timed, t_acc);
+    if (region) ++ar1; else ++ar0;
+    tc_fence_after();
+    return lane_base + region * REGION;
+  }
+  // this warp's part of block cb is in tensor memory (proxy: and its generic-proxy stores to shared memory are visible to the tensor
+  // core): one arrival per warp
+  __device__ __forceinline__ void blk_done(const int cb, const bool proxy = false) {
+    tmem_st_wait(); tc_fence_before();
+    if (proxy) fence_proxy_async();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&blk[cb]);
+  }
+  // 32 columns of this row (32-column block cg): split into the planes once, then -> the workspace tile blob (if any) and / or, with
+  // to_a, IN PLACE over the accumulator block they came from (blk_addr): the next A operand
+  __device__ __forceinline__ void emit(const int cg, const float (&v)[32], uint8_t* blob, const bool to_a, const uint32_t blk_addr) {
+    uint32_t hi[16], lo[16];
+#pragma unroll
+    for (int qd = 0; qd < 4; ++qd) {
+      uint4 pq[PL];
+      split8<PL, F16>(v + qd * 8, pq);
+      if (blob && !no_stores) {
+        const uint32_t off = gp_off(32, r, cg * 4 + qd);
+        __stcs(reinterpret_cast<uint4*>(blob + off), pq[0]);
+        if (PL == 2) __stcs(reinterpret_cast<uint4*>(blob + BLOB_H + off), pq[PL - 1]);
+      }
+      hi[qd * 4 + 0] = pq[0].x; hi[qd * 4 + 1] = pq[0].y; hi[qd * 4 + 2] = pq[0].z; hi[qd * 4 + 3] = pq[0].w;
+      lo[qd * 4 + 0] = pq[PL - 1].x; lo[qd * 4 + 1] = pq[PL - 1].y; lo[qd * 4 + 2] = pq[PL - 1].z; lo[qd * 4 + 3] = pq[PL - 1].w;
+    }
+    if (to_a) {
+      tmem_st16(blk_addr, hi);
+      if (PL == 2) tmem_st16(blk_addr + 16, lo);
+    }
+  }
+};
+}  // namespace pp
+
+// ------------------------------------------------------------------------------------------------
 // Pass 1 of the split modes: A operands in TENSOR MEMORY (DESIGN.md section 5).
 // The A operand of every GEMM but G1 / G2b is written by the epilogues with tcgen05.st and read by the TS form of tcgen05.mma; the
 // PE / PE6 tiles of G1 / G2b travel through the ring as K = 16 slices next to their weight chunks; tiles kept for the backward pass
@@ -289,14 +510,12 @@ template <int PL> __device__ __forceinline__ void epi_bar() { asm volatile("bar.
 // accumulator of GEMM j + 1.
 // ------------------------------------------------------------------------------------------------
 namespace ts {
-constexpr int A_PLANE = 2 * CORE_STRIDE;        // A slice [128 x 16] of one plane: 4 KB
-constexpr uint32_t REGION = 256;               // TMEM columns of one ping-pong region
 constexpr int NS_MAX = 16;
 template <int PL>
 struct Cfg {                                    // ring geometry for PL operand planes
   static constexpr int NS = PL == 2 ? 9 : 16;
   static constexpr int W_BYTES = PL * STAGE_BYTES;         // weight chunk [256 x 16]: 8 KB per plane, hi | lo  ([192 x 16]: 6 KB per plane)
-  static constexpr int STAGE = W_BYTES + PL * A_PLANE;     // 24 KB / 12 KB
+  static constexpr int STAGE = W_BYTES + PL * pp::A_PLANE; // 24 KB / 12 KB
   static constexpr int SMEM = NS * STAGE + NVEC * H * 4 + TP * 4 * 4;
 };
 struct PipeTS {
@@ -307,10 +526,6 @@ struct PipeTS {
   uint32_t tmem_base;
 };
 static_assert(Cfg<2>::SMEM + (int)sizeof(PipeTS) + 1024 <= 227 * 1024 && Cfg<1>::SMEM <= Cfg<2>::SMEM, "pass1_ts_kernel: ring + vectors + row sums + barriers must fit one SM's 227 KB");
-static_assert(2 * REGION == 512 && REGION == H, "TMEM map: two [128 x 256] fp32 accumulators, each converted in place into 2 x 16-bit planes");
-// K-chunk order of a TS-form GEMM: the two epilogue warp groups finish block cb of their column halves together, i.e. chunks
-// 2cb, 2cb+1 (half 0) and 8+2cb, 9+2cb (half 1)
-__host__ __device__ constexpr int block_order(int i) { return ((i >> 2) << 1) + (i & 1) + ((i >> 1) & 1) * 8; }
 }  // namespace ts
 
 template <int PL, bool F16, bool XF>             // PL operand planes; XF: cross-first accumulation of G1 - G3 (DPN_MODE_F16X3A)
@@ -325,21 +540,9 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int b = blockIdx.x / w.T, tl = blockIdx.x % w.T;
   const size_t g = blockIdx.x;
-  if (tid == 0) {
-    for (int s = 0; s < TS::NS; ++s) { mbar_init(&pipe.full[s], 1); mbar_init(&pipe.empty[s], CLUSTER); }
-    for (int i = 0; i < 4; ++i) mbar_init(&pipe.blk[i], Geo<PL>::EW);
-    mbar_init(&pipe.acc_ready[0], 1); mbar_init(&pipe.acc_ready[1], 1);
-    mbar_init(&pipe.drained, Geo<PL>::EW);
-    fence_barrier_init();
-  }
-  if (warp == Geo<PL>::W_MMA) tmem_alloc(&pipe.tmem_base, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  if (CLUSTER > 1) cluster_sync_all();
-  const uint32_t tmem = pipe.tmem_base;
-  const uint32_t rank = cluster_ctarank();
-  constexpr uint16_t MC_MASK = (uint16_t)((1u << CLUSTER) - 1);
+  if (tid == 0) mbar_init(&pipe.drained, Geo<PL>::EW);
+  const pp::Block cta = pp::block_start<PL, TS::NS>(pipe, tid, warp);
+  const uint32_t tmem = cta.tmem;
   // DPN_MODE_F16X3A: CROSS-FIRST accumulation of the three GEMMs that decide the ReLU masks (G1 -> m1; G2, G3 -> m3).  The tensor core adds every MMA
   // into the fp32 accumulator with round-toward-zero at the accumulator's CURRENT magnitude, so the 2 x 16 cross-term MMAs of a split
   // contraction cost as much accuracy as its 16 main-term MMAs when they are interleaved.  Issued FIRST - while the accumulator holds
@@ -351,28 +554,8 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
 
   if (warp == Geo<PL>::W_PROD) {
     // ---------------- producer: weight chunks (multicast slices) + this tile's PE slices ----------------
-    uint32_t s = 0, ph = 0;
-    const uint64_t pol = l2_policy_evict_last();
-    // hi_only: the main-term phase of a cross-first GEMM needs only the hi plane of the chunk (first half) and of the A slice
-    auto put = [&](const uint8_t* wsrc, uint32_t wbytes, const uint8_t* asrc, const bool hi_only = false) {
-      if (hi_only) wbytes /= 2;
-      const int a_planes = hi_only ? 1 : PL;
-      mbar_wait(&pipe.empty[s], ph ^ 1);
-      if (elect_one()) {
-        uint8_t* stg = ring + s * TS::STAGE;
-        mbar_arrive_expect_tx(&pipe.full[s], wbytes + (asrc ? a_planes * ts::A_PLANE : 0));
-        if (CLUSTER == 1) {
-          bulk_g2s_hint(stg, wsrc, wbytes, &pipe.full[s], pol);
-        } else {
-          const uint32_t slice = wbytes / CLUSTER;
-          bulk_g2s_mc_hint(stg + rank * slice, wsrc + rank * slice, slice, &pipe.full[s], MC_MASK, pol);
-        }
-        if (asrc) {
-          for (int p = 0; p < a_planes; ++p) bulk_g2s_hint(stg + TS::W_BYTES + p * ts::A_PLANE, asrc + p * BLOB_C, ts::A_PLANE, &pipe.full[s], pol);
-        }
-      }
-      if (++s == TS::NS) { s = 0; ph ^= 1; }
-    };
+    // (the main-term phase of a cross-first GEMM needs only the hi planes of its chunks and A slices: hi_only)
+    pp::Ring<PL, TS> wr{ring, pipe.full, pipe.empty, cta.rank, l2_policy_evict_last()};
     const uint8_t* pe_src = w.pe_blob + g * Geo<PL>::BC;
     const uint8_t* pe6_src = w.pe6_blob + g * Geo<PL>::BC;
     for (int k = 0; k < w.Kn; ++k) {
@@ -383,164 +566,86 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       // the MMA warp's order: G1 | G2b (PE6 slices: no dependence on an epilogue, issued first) | TS-form GEMMs in block order.
       // Cross-first GEMMs (G1 - G3 when masks matter, see the MMA warp) read every chunk twice: whole chunks for the cross terms,
       // then the hi planes again for the main terms.
-      for (int c = 0; c < 12; ++c) put(iW1 + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe_src + (size_t)c * ts::A_PLANE);
-      if (xfirst) for (int c = 0; c < 12; ++c) put(iW1 + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe_src + (size_t)c * ts::A_PLANE, true);
-      for (int c = 0; c < 12; ++c) put(iWd + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe6_src + (size_t)c * ts::A_PLANE);
-      for (int i = 0; i < 16; ++i) put(iW2 + (size_t)ts::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
+      for (int c = 0; c < 12; ++c) wr.put(iW1 + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe_src + (size_t)c * pp::A_PLANE);
+      if (xfirst) for (int c = 0; c < 12; ++c) wr.put(iW1 + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe_src + (size_t)c * pp::A_PLANE, true);
+      for (int c = 0; c < 12; ++c) wr.put(iWd + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe6_src + (size_t)c * pp::A_PLANE);
+      for (int i = 0; i < 16; ++i) wr.put(iW2 + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
       if (xfirst) {
-        for (int c = 0; c < 12; ++c) put(iWd + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe6_src + (size_t)c * ts::A_PLANE, true);
-        for (int c = 0; c < 16; ++c) put(iW2 + (size_t)c * TS::W_BYTES, TS::W_BYTES, nullptr, true);
+        for (int c = 0; c < 12; ++c) wr.put(iWd + (size_t)c * TS::W_BYTES, TS::W_BYTES, pe6_src + (size_t)c * pp::A_PLANE, true);
+        for (int c = 0; c < 16; ++c) wr.put(iW2 + (size_t)c * TS::W_BYTES, TS::W_BYTES, nullptr, true);
       }
-      for (int i = 0; i < 16; ++i) put(iWa + (size_t)ts::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
-      if (xfirst) for (int c = 0; c < 16; ++c) put(iWa + (size_t)c * TS::W_BYTES, TS::W_BYTES, nullptr, true);
+      for (int i = 0; i < 16; ++i) wr.put(iWa + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
+      if (xfirst) for (int c = 0; c < 16; ++c) wr.put(iWa + (size_t)c * TS::W_BYTES, TS::W_BYTES, nullptr, true);
       if (sweep) {
-        for (int i = 0; i < 16; ++i) put(iWaT + (size_t)ts::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
-        for (int i = 0; i < 16; ++i) put(iW2T + (size_t)ts::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
+        for (int i = 0; i < 16; ++i) wr.put(iWaT + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
+        for (int i = 0; i < 16; ++i) wr.put(iW2T + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
         if (sweep > 1)
-          for (int i = 0; i < 16; ++i) put(iW1T + (size_t)ts::block_order(i) * (PL * 6144), PL * 6144, nullptr);
+          for (int i = 0; i < 16; ++i) wr.put(iW1T + (size_t)pp::block_order(i) * (PL * 6144), PL * 6144, nullptr);
       }
     }
   } else if (warp == Geo<PL>::W_MMA) {
     // ---------------- MMA issuer ----------------
-    uint32_t s = 0, ph = 0, bp = 0, dr = 0, cur = 0;
-    long long t_full = 0, t_epi = 0;
-    const bool timed = w.phase_dbg != nullptr;
+    pp::Mma<PL, F16, TS> mma{{ring, pipe.full, pipe.empty}, pipe.blk, pipe.acc_ready, smem_u32(ring), w.phase_dbg != nullptr, DPN_DBG(w, 1)};
+    uint32_t dr = 0, cur = 0;
     const long long t_begin = clock64();
-    const uint32_t ring_addr = smem_u32(ring);
-    const uint64_t a_base = smem_desc(ring_addr + TS::W_BYTES, CORE_STRIDE, 128);
-    // one K = 16 chunk: lo*hi + hi*lo + hi*hi into the accumulator at column d; A planes from tensor memory (a_hi) or from the stage
-    // which of the products of a split contraction a chunk issues: all three | exact A operand (B_lo, B_hi) | the two cross terms | the main term
-    enum { P_ALL = 0, P_EXACT = 1, P_CROSS = 2, P_MAIN = 3 };
-    auto chunk = [&](const uint32_t d, const int Nn, const bool a_in_tmem, const uint32_t a_hi, const uint32_t first, const int part = P_ALL) {
-      const uint32_t idesc = idesc_16(F16, Nn, 0, 0, 128);
-      const uint64_t b_base = smem_desc(ring_addr, Nn * 16, 128);
-      const uint32_t b_lo = (uint32_t)(Nn * 32) >> 4;
-      if (timed) mbar_wait_t(&pipe.full[s], ph, t_full); else mbar_wait(&pipe.full[s], ph);
-      tc_fence_after();
-      const uint64_t bd = b_base + s * (uint32_t)(TS::STAGE >> 4), bl = bd + b_lo;
-      if (elect_one()) {
-        if (DPN_DBG(w, 1)) {                             // (debug builds: no MMAs, barrier protocol intact)
-        } else if (a_in_tmem) {
-          if (PL == 1) {                                   // one plane: one product
-            mma_ts(d, a_hi, bd, idesc, first);
-          } else {
-            if (part == P_ALL || part == P_CROSS) mma_ts(d, a_hi + 16, bd, idesc, first);   // (an exact 16-bit A operand - the 0 / 1 mask of G4 - has no lo plane)
-            if (part != P_MAIN) mma_ts(d, a_hi, bl, idesc, part == P_EXACT ? first : 1u);
-            if (part != P_CROSS) mma_ts(d, a_hi, bd, idesc, part == P_MAIN ? first : 1u);
-          }
-        } else {                                         // the A slice of this chunk sits behind the weights in the same stage
-          const uint64_t ad = a_base + s * (uint32_t)(TS::STAGE >> 4), al = ad + (ts::A_PLANE >> 4);
-          if (PL == 1 || part == P_MAIN) {
-            mma_bf16(d, ad, bd, idesc, first);
-          } else {
-            mma_bf16(d, al, bd, idesc, first);
-            if (part == P_CROSS) {
-              mma_bf16(d, ad, bl, idesc, 1u);
-            } else {
-              mma_f16_c<REUSE_A ? A_FILL : A_DISCARD>(d, ad, bl, idesc, 1u);
-              mma_f16_c<REUSE_A ? A_LAST : A_DISCARD>(d, ad, bd, idesc, 1u);
-            }
-          }
-        }
-        if (CLUSTER == 1) mma_commit(&pipe.empty[s]); else mma_commit_mc(&pipe.empty[s], MC_MASK);
-      }
-      if (++s == TS::NS) { s = 0; ph ^= 1; }
-    };
+    const uint64_t a_base = smem_desc(smem_u32(ring) + TS::W_BYTES, CORE_STRIDE, 128);      // the A slice of stage 0
     // G over the PE / PE6 slices of the ring into region `cur`
-    auto gemm_ss = [&](const int nchunks, const int part = P_ALL, const bool accumulate = false) {
-      for (int c = 0; c < nchunks; ++c) chunk(tmem + cur * ts::REGION, H, false, 0u, (accumulate || c > 0) ? 1u : 0u, part);
+    auto gemm_ss = [&](const int nchunks, const int part = pp::P_ALL, const bool accumulate = false) {
+      for (int c = 0; c < nchunks; ++c) mma.ss(tmem + cur * pp::REGION, H, a_base, pp::A_PLANE >> 4, true, (accumulate || c > 0) ? 1u : 0u, part);
     };
     // G whose A operand is the other region, converted in place by the running epilogue: block by block
-    auto gemm_ts = [&](const int Nn, const bool accumulate, const int part = P_ALL) {
-      const uint32_t d = tmem + cur * ts::REGION, a = tmem + (cur ^ 1u) * ts::REGION;
-      for (int cb = 0; cb < 4; ++cb) {
-        if (timed) mbar_wait_t(&pipe.blk[cb], bp, t_epi); else mbar_wait(&pipe.blk[cb], bp);
-        tc_fence_after();
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int c = 2 * cb + (j & 1) + (j >> 1) * 8;
-          chunk(d, Nn, true, a + 32u * (uint32_t)(c >> 1) + 8u * (uint32_t)(c & 1), (accumulate || cb > 0 || j > 0) ? 1u : 0u, part);
-        }
-      }
-      bp ^= 1u;
+    auto gemm_ts = [&](const int Nn, const bool accumulate, const int part = pp::P_ALL) {
+      mma.gemm_ts(tmem + cur * pp::REGION, tmem + (cur ^ 1u) * pp::REGION, Nn, accumulate, part);
     };
     // main terms of a cross-first K = 256 GEMM: every block of the A operand has arrived (its cross terms are in), natural chunk order
     auto gemm_ts_main = [&]() {
-      const uint32_t d = tmem + cur * ts::REGION, a = tmem + (cur ^ 1u) * ts::REGION;
-      for (int c = 0; c < 16; ++c) chunk(d, H, true, a + 32u * (uint32_t)(c >> 1) + 8u * (uint32_t)(c & 1), 1u, P_MAIN);
+      const uint32_t d = tmem + cur * pp::REGION, a = tmem + (cur ^ 1u) * pp::REGION;
+      for (int c = 0; c < 16; ++c) mma.ts(d, H, pp::chunk_col(a, c), pp::chunk_col(a, c) + 16, 1u, pp::P_MAIN);
     };
-    auto ready = [&]() { if (elect_one()) mma_commit(&pipe.acc_ready[cur]); cur ^= 1u; };
+    auto ready = [&]() { mma.ready(cur); cur ^= 1u; };
     for (int k = 0; k < w.Kn; ++k) {
-      if (xfirst) { gemm_ss(12, P_CROSS); gemm_ss(12, P_MAIN, true); } else gemm_ss(12);
+      if (xfirst) { gemm_ss(12, pp::P_CROSS); gemm_ss(12, pp::P_MAIN, true); } else gemm_ss(12);
       ready();                                                             // G1 (A = PE slices); its region was the A operand of the previous GEMM
       if (k > 0) {                                                         // the last epilogue of the previous net has drained this region
-        if (timed) mbar_wait_t(&pipe.drained, dr & 1, t_epi); else mbar_wait(&pipe.drained, dr & 1);
+        pp::wait(&pipe.drained, dr & 1, mma.timed, mma.t_epi);
         ++dr; tc_fence_after();
       }
       if (xfirst) {                                                        // G2b (A = PE6 slices) + G2a (A = h1): all cross terms, then all main terms
-        gemm_ss(12, P_CROSS); gemm_ts(H, true, P_CROSS); gemm_ss(12, P_MAIN, true); gemm_ts_main(); ready();
+        gemm_ss(12, pp::P_CROSS); gemm_ts(H, true, pp::P_CROSS); gemm_ss(12, pp::P_MAIN, true); gemm_ts_main(); ready();
       } else {
         gemm_ss(12); gemm_ts(H, true); ready();
       }
-      if (xfirst) { gemm_ts(H, false, P_CROSS); gemm_ts_main(); } else gemm_ts(H, false);
+      if (xfirst) { gemm_ts(H, false, pp::P_CROSS); gemm_ts_main(); } else gemm_ts(H, false);
       ready();                                                             // G3 (A = c)
       if (sweep) {
-        gemm_ts(H, false, P_EXACT); ready();                               // G4 (A = the m3 mask, B = diag(u) Wa: two MMAs per chunk)
+        gemm_ts(H, false, pp::P_EXACT); ready();                             // G4 (A = the m3 mask, B = diag(u) Wa: two MMAs per chunk)
         gemm_ts(H, false); ready();                                        // G5 (A = y)
         if (sweep > 1) { gemm_ts(C, false); ready(); }                     // G6 (A = qm, N = 192)
       }
     }
-    if (timed && lane == 0) {
+    if (mma.timed && lane == 0) {
       atomicAdd((unsigned long long*)w.phase_dbg + 0, (unsigned long long)(clock64() - t_begin));
-      atomicAdd((unsigned long long*)w.phase_dbg + 1, (unsigned long long)t_full);
-      atomicAdd((unsigned long long*)w.phase_dbg + 2, (unsigned long long)t_epi);
+      atomicAdd((unsigned long long*)w.phase_dbg + 1, (unsigned long long)mma.t_full);
+      atomicAdd((unsigned long long*)w.phase_dbg + 2, (unsigned long long)mma.t_epi);
     }
   } else if (warp < Geo<PL>::EW) {
     // ---------------- epilogue: thread = (point r, column half) ----------------
     constexpr int NB = Geo<PL>::NB;
     const int half = warp >> 2, r = (warp & 3) * 32 + lane, c0 = half * NB;
-    const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+    pp::Epi<PL, F16> epi{pipe.blk, pipe.acc_ready, tmem + ((uint32_t)((warp & 3) * 32) << 16), r, lane, w.phase_dbg != nullptr, DPN_DBG(w, 4)};
     const int p_local = tl * TP + r;
     const bool valid = p_local < w.P;
     const size_t q = (size_t)b * w.N + w.p0 + p_local;
     const size_t row = g * TP + r;
     const float* pet = w.pet + g * (size_t)(C * TP) + r;
     const uint64_t pol_keep = l2_policy_evict_last();
-    uint32_t arc0 = 0u, arc1 = 0u, cur = 0u;
-    // 32 columns of this row: split into the two planes once, then -> workspace tile (if any) and / or IN PLACE over the accumulator
-    // block they came from (blk_addr): the next A operand
-    auto emit = [&](const int cg, const float (&v)[32], uint8_t* blob, const bool to_a, const uint32_t blk_addr) {
-      uint32_t hi[16], lo[16];
-#pragma unroll
-      for (int qd = 0; qd < 4; ++qd) {
-        uint4 pq[PL];
-        split8<PL, F16>(v + qd * 8, pq);
-        if (blob && !DPN_DBG(w, 4)) {
-          const uint32_t off = gp_off(32, r, cg * 4 + qd);
-          __stcs(reinterpret_cast<uint4*>(blob + off), pq[0]);
-          if (PL == 2) __stcs(reinterpret_cast<uint4*>(blob + BLOB_H + off), pq[PL - 1]);
-        }
-        hi[qd * 4 + 0] = pq[0].x; hi[qd * 4 + 1] = pq[0].y; hi[qd * 4 + 2] = pq[0].z; hi[qd * 4 + 3] = pq[0].w;
-        lo[qd * 4 + 0] = pq[PL - 1].x; lo[qd * 4 + 1] = pq[PL - 1].y; lo[qd * 4 + 2] = pq[PL - 1].z; lo[qd * 4 + 3] = pq[PL - 1].w;
-      }
-      if (to_a) {
-        tmem_st16(blk_addr, hi);
-        if (PL == 2) tmem_st16(blk_addr + 16, lo);
-      }
-    };
-    // this warp's part of block cb is in tensor memory / this warp has read the last accumulator of the net: one arrival per warp
-    auto blk_done = [&](const int cb) { tmem_st_wait(); tc_fence_before(); __syncwarp(); if (lane == 0) mbar_arrive(&pipe.blk[cb]); };
+    uint32_t cur = 0u;
+    // this warp has read the last accumulator of the net: one arrival per warp
     auto net_done = [&]() { tc_fence_before(); __syncwarp(); if (lane == 0) mbar_arrive(&pipe.drained); };
-    long long t_acc = 0;
     const long long t_begin = clock64();
-    const bool timed = w.phase_dbg != nullptr;
     // waits for the GEMM into the current region; returns this thread's lane address of that region and flips the region
     auto acc_wait = [&]() -> uint32_t {
-      const uint32_t par = (cur ? arc1 : arc0) & 1u;
-      if (timed) mbar_wait_t(&pipe.acc_ready[cur], par, t_acc); else mbar_wait(&pipe.acc_ready[cur], par);
-      if (cur) ++arc1; else ++arc0;
-      tc_fence_after();
-      const uint32_t a = lane_base + cur * ts::REGION;
+      const uint32_t a = epi.acc_wait(cur);
       cur ^= 1u;
       return a;
     };
@@ -593,8 +698,8 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         }
 #pragma unroll
         for (int i = 0; i < NB; ++i) m1w[i] = (cb == i) ? bits : m1w[i];
-        emit(cg, v, nullptr, true, ra + cg * 32);                     // h1 itself is not kept: pass 2 needs only its mask
-        blk_done(cb);
+        epi.emit(cg, v, nullptr, true, ra + cg * 32);                     // h1 itself is not kept: pass 2 needs only its mask
+        epi.blk_done(cb);
       }
       // ---- epilogue 2: c = acc + (b2 + bd + e);  oc = 2wo.c ----
       float os0 = 0.f, os1 = 0.f;
@@ -616,8 +721,8 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
             v[j4 * 4 + e] = cc;
           }
         }
-        emit(cg, v, nullptr, true, ra + cg * 32);
-        blk_done(cb);
+        epi.emit(cg, v, nullptr, true, ra + cg * 32);
+        epi.blk_done(cb);
       }
       // ---- epilogue 3: g = relu(a3 + ba);  o = oc + u.g + cst + ref;  the mask m3 = [a3 > 0] is the A operand of G4 ----
       uint32_t m3w[NB];
@@ -652,7 +757,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
 #pragma unroll
           for (int i = 0; i < 16; ++i) mk[i] = (((bits >> (2 * i)) & 1u) ? ONE : 0u) | (((bits >> (2 * i + 1)) & 1u) ? (ONE << 16) : 0u);
           tmem_st16(ra + cg * 32, mk);
-          blk_done(cb);
+          epi.blk_done(cb);
         }
       }
       if (!sweep) net_done();
@@ -683,8 +788,8 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
 #pragma unroll
           for (int e = 0; e < 4; ++e) v[j4 * 4 + e] = F16 ? fmaf(v[j4 * 4 + e], k4, ww[e]) : v[j4 * 4 + e] + ww[e];
         }
-        emit(cg, v, blob_h<PL>(nt, B_YT), true, ra + cg * 32);
-        blk_done(cb);
+        epi.emit(cg, v, blob_h<PL>(nt, B_YT), true, ra + cg * 32);
+        epi.blk_done(cb);
       }
       // ---- epilogue 5: qm = acc * m1 ----
       ra = acc_wait();
@@ -698,8 +803,8 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         for (int i = 0; i < NB; ++i) bits = (cb == i) ? m1w[i] : bits;
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = ((bits >> j) & 1u) ? (F16 ? v[j] * i5 : v[j]) : 0.f;
-        emit(cg, v, blob_h<PL>(nt, B_QM), sweep > 1, ra + cg * 32);
-        if (sweep > 1) blk_done(cb);
+        epi.emit(cg, v, blob_h<PL>(nt, B_QM), sweep > 1, ra + cg * 32);
+        if (sweep > 1) epi.blk_done(cb);
       }
       if (sweep < 2) { net_done(); continue; }
       // ---- epilogue 6: do/dz_c = sum_j jin_j dPE_j  (j % 3 == c); N = 192: each half takes one 96-column group ----
@@ -734,18 +839,15 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         }
       }
     }
-    if (timed && tid == 0) {
+    if (epi.timed && tid == 0) {
       const long long tot = clock64() - t_begin;
       atomicAdd((unsigned long long*)w.phase_dbg + 4, (unsigned long long)tot);
-      atomicAdd((unsigned long long*)w.phase_dbg + 5, (unsigned long long)t_acc);
-      atomicAdd((unsigned long long*)w.phase_dbg + 7, (unsigned long long)(tot - t_acc));
+      atomicAdd((unsigned long long*)w.phase_dbg + 5, (unsigned long long)epi.t_acc);
+      atomicAdd((unsigned long long*)w.phase_dbg + 7, (unsigned long long)(tot - epi.t_acc));
       atomicAdd((unsigned long long*)w.phase_dbg + 6, 1ull);
     }
   }
-  tc_fence_before();
-  __syncthreads();
-  if (CLUSTER > 1) cluster_sync_all();
-  if (warp == Geo<PL>::W_MMA) tmem_dealloc(tmem, 512);
+  pp::block_end<PL>(tmem, warp);
 }
 
 // 8 consecutive values of a stored tile: sum of its planes
@@ -788,10 +890,11 @@ template <int PL>
 struct Cfg {
   static constexpr int NS = PL == 2 ? 7 : 14;
   static constexpr int W_BYTES = PL * STAGE_BYTES;       // one K = 16 chunk of a [256 x K] image: 8 KB per plane, hi | lo
+  static constexpr int STAGE = W_BYTES;
   static constexpr int ZD_BYTES = PL * BLOB_C;           // zd staging: one [128 x 192] tile per plane, layout (*)
-  static constexpr int SMEM = NS * W_BYTES + ZD_BYTES + NV2 * H * 4 + H * 4 + 16;        // + column sums of zc + sum of dov
+  static constexpr int SMEM = NS * STAGE + ZD_BYTES + NV2 * H * 4 + H * 4 + 16;        // + column sums of zc + sum of dov
 };
-constexpr uint32_t REGION = 256, ZP_LO = 96;   // TMEM: regions R0 | R1; zp planes inside R1: hi [0,96) | lo [96,192)
+constexpr uint32_t ZP_LO = 96;                 // zp planes inside TMEM region R1: hi [0,96) | lo [96,192)
 struct PipeZ {
   uint64_t full[NS_MAX], empty[NS_MAX];
   uint64_t blk[4];          // block i of both column halves of the next A operand is in tensor memory (one arrival per epilogue warp)
@@ -810,46 +913,19 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ p2z::PipeZ pipe;
   uint8_t* ring = smem;
-  uint8_t* zdt = smem + PZ::NS * PZ::W_BYTES;
+  uint8_t* zdt = smem + PZ::NS * PZ::STAGE;
   float* svec = reinterpret_cast<float*>(zdt + PZ::ZD_BYTES);
   float* csum = svec + p2z::NV2 * H;                               // [H] + sdo
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int b = blockIdx.x / w.T, tl = blockIdx.x % w.T;
   const size_t g = blockIdx.x;
-  if (tid == 0) {
-    for (int s = 0; s < PZ::NS; ++s) { mbar_init(&pipe.full[s], 1); mbar_init(&pipe.empty[s], CLUSTER); }
-    for (int i = 0; i < 4; ++i) mbar_init(&pipe.blk[i], Geo<PL>::EW);
-    mbar_init(&pipe.acc_ready[0], 1); mbar_init(&pipe.acc_ready[1], 1);
-    fence_barrier_init();
-  }
-  if (warp == Geo<PL>::W_MMA) tmem_alloc(&pipe.tmem_base, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  if (CLUSTER > 1) cluster_sync_all();
-  const uint32_t tmem = pipe.tmem_base;
-  const uint32_t rank = cluster_ctarank();
-  constexpr uint16_t MC_MASK = (uint16_t)((1u << CLUSTER) - 1);
+  const pp::Block cta = pp::block_start<PL, PZ::NS>(pipe, tid, warp);
+  const uint32_t tmem = cta.tmem;
 
   if (warp == Geo<PL>::W_PROD) {
     // ---------------- producer: weight chunks (multicast slices) ----------------
-    uint32_t s = 0, ph = 0;
-    const uint64_t pol = l2_policy_evict_last();
-    auto put = [&](const uint8_t* wsrc) {
-      mbar_wait(&pipe.empty[s], ph ^ 1);
-      if (elect_one()) {
-        uint8_t* stg = ring + s * PZ::W_BYTES;
-        mbar_arrive_expect_tx(&pipe.full[s], PZ::W_BYTES);
-        if (CLUSTER == 1) {
-          bulk_g2s_hint(stg, wsrc, PZ::W_BYTES, &pipe.full[s], pol);
-        } else {
-          constexpr uint32_t slice = PZ::W_BYTES / CLUSTER;
-          bulk_g2s_mc_hint(stg + rank * slice, wsrc + rank * slice, slice, &pipe.full[s], MC_MASK, pol);
-        }
-      }
-      if (++s == PZ::NS) { s = 0; ph ^= 1; }
-    };
+    pp::Ring<PL, PZ> wr{ring, pipe.full, pipe.empty, cta.rank, l2_policy_evict_last()};
     for (int k = 0; k < w.Kn; ++k) {
       const uint8_t* gen = w.img_gen + ((size_t)b * w.Kn + k) * Geo<PL>::GEN;
       const uint8_t* sta = w.img_sta + (size_t)k * Geo<PL>::STA;
@@ -857,119 +933,49 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       // the MMA warp's order: G7' in prologue-block order | zd Wd^T (no dependence on an epilogue) | G8' in block order
       for (int i = 0; i < 4; ++i)
         for (int h = 0; h < 2; ++h)
-          for (int j = 0; j < p2z::zp_count(i); ++j) put(iW1 + (size_t)(6 * h + p2z::zp_first(i) + j) * PZ::W_BYTES);
-      for (int c = 0; c < 12; ++c) put(iWd + (size_t)c * PZ::W_BYTES);
-      for (int i = 0; i < 16; ++i) put(iW2 + (size_t)ts::block_order(i) * PZ::W_BYTES);
+          for (int j = 0; j < p2z::zp_count(i); ++j) wr.put(iW1 + (size_t)(6 * h + p2z::zp_first(i) + j) * PZ::W_BYTES, PZ::W_BYTES, nullptr);
+      for (int c = 0; c < 12; ++c) wr.put(iWd + (size_t)c * PZ::W_BYTES, PZ::W_BYTES, nullptr);
+      for (int i = 0; i < 16; ++i) wr.put(iW2 + (size_t)pp::block_order(i) * PZ::W_BYTES, PZ::W_BYTES, nullptr);
     }
   } else if (warp == Geo<PL>::W_MMA) {
     // ---------------- MMA issuer ----------------
-    uint32_t s = 0, ph = 0, bp = 0;
-    long long t_full = 0, t_epi = 0;
-    const bool timed = w.phase_dbg != nullptr;
+    pp::Mma<PL, F16, PZ> mma{{ring, pipe.full, pipe.empty}, pipe.blk, pipe.acc_ready, smem_u32(ring), w.phase_dbg != nullptr, false};
     const long long t_begin = clock64();
-    const uint32_t ring_addr = smem_u32(ring);
-    const uint32_t idesc = idesc_16(F16, H, 0, 0, 128);
-    const uint64_t b_base = smem_desc(ring_addr, H * 16, 128);
     const uint64_t zd_base = smem_desc(smem_u32(zdt), CORE_STRIDE, 128);
-    constexpr uint32_t b_lo = (uint32_t)(H * 32) >> 4, zd_lo = BLOB_C >> 4, zd_step = (2 * CORE_STRIDE) >> 4;
-    const uint32_t R0 = tmem, R1 = tmem + p2z::REGION;
-    // one K = 16 chunk: lo*hi + hi*lo + hi*hi into the accumulator at d; A planes from tensor memory (a_hi / a_lo) or K-slice zc of the zd tile
-    auto chunk = [&](const uint32_t d, const bool a_in_tmem, const uint32_t a_hi, const uint32_t a_lo, const int zc, const uint32_t first) {
-      if (timed) mbar_wait_t(&pipe.full[s], ph, t_full); else mbar_wait(&pipe.full[s], ph);
-      tc_fence_after();
-      const uint64_t bd = b_base + s * (uint32_t)(PZ::W_BYTES >> 4), bl = bd + b_lo;
-      if (elect_one()) {
-        if (a_in_tmem) {
-          if (PL == 2) { mma_ts(d, a_lo, bd, idesc, first); mma_ts(d, a_hi, bl, idesc, 1u); }
-          mma_ts(d, a_hi, bd, idesc, PL == 2 ? 1u : first);
-        } else {
-          const uint64_t ad = zd_base + (uint32_t)zc * zd_step, al = ad + zd_lo;
-          if (PL == 2) {
-            mma_bf16(d, al, bd, idesc, first);
-            mma_f16_c<REUSE_A ? A_FILL : A_DISCARD>(d, ad, bl, idesc, 1u);
-            mma_f16_c<REUSE_A ? A_LAST : A_DISCARD>(d, ad, bd, idesc, 1u);
-          } else {
-            mma_bf16(d, ad, bd, idesc, first);
-          }
-        }
-        if (CLUSTER == 1) mma_commit(&pipe.empty[s]); else mma_commit_mc(&pipe.empty[s], MC_MASK);
-      }
-      if (++s == PZ::NS) { s = 0; ph ^= 1; }
-    };
-    auto wait_blk = [&](const int i) { if (timed) mbar_wait_t(&pipe.blk[i], bp, t_epi); else mbar_wait(&pipe.blk[i], bp); tc_fence_after(); };
-    // K = 256 GEMM whose A operand is region a, converted in place by the running epilogue
-    auto gemm_ts = [&](const uint32_t d, const uint32_t a, const bool accumulate) {
-      for (int cb = 0; cb < 4; ++cb) {
-        wait_blk(cb);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int c = 2 * cb + (j & 1) + (j >> 1) * 8;
-          const uint32_t ah = a + 32u * (uint32_t)(c >> 1) + 8u * (uint32_t)(c & 1);
-          chunk(d, true, ah, ah + 16, 0, (accumulate || cb > 0 || j > 0) ? 1u : 0u);
-        }
-      }
-      bp ^= 1u;
-    };
-    auto ready = [&](const int region) { if (elect_one()) mma_commit(&pipe.acc_ready[region]); };
+    constexpr uint32_t zd_lo = BLOB_C >> 4, zd_step = (2 * CORE_STRIDE) >> 4;
+    const uint32_t R0 = tmem, R1 = tmem + pp::REGION;
     for (int k = 0; k < w.Kn; ++k) {
       for (int i = 0; i < 4; ++i) {                                        // G7' = zp W1^T -> R0, under the prologue
-        wait_blk(i);
+        mma.wait_blk(i);
         for (int h = 0; h < 2; ++h)
           for (int j = 0; j < p2z::zp_count(i); ++j) {
             const uint32_t c = 6 * h + p2z::zp_first(i) + j;
-            chunk(R0, true, R1 + 8u * c, R1 + p2z::ZP_LO + 8u * c, 0, (i > 0 || h > 0 || j > 0) ? 1u : 0u);
+            mma.ts(R0, H, R1 + 8u * c, R1 + p2z::ZP_LO + 8u * c, (i > 0 || h > 0 || j > 0) ? 1u : 0u);
           }
       }
-      bp ^= 1u;
-      ready(0);
-      for (int c = 0; c < 12; ++c) chunk(R1, false, 0u, 0u, c, c > 0 ? 1u : 0u);   // G8' = zd Wd^T (zd: shared memory, complete with the prologue)
-      gemm_ts(R1, R0, true); ready(1);                                     //       + zh W2^T, under epilogue 7
+      mma.bp ^= 1u;
+      mma.ready(0);
+      for (int c = 0; c < 12; ++c) mma.ss(R1, H, zd_base + (uint32_t)c * zd_step, zd_lo, false, c > 0 ? 1u : 0u);   // G8' = zd Wd^T (zd: shared memory, complete with the prologue)
+      mma.gemm_ts(R1, R0, H, true); mma.ready(1);                          //       + zh W2^T, under epilogue 7
     }
-    if (timed && lane == 0) {
+    if (mma.timed && lane == 0) {
       atomicAdd((unsigned long long*)w.phase_dbg + 8, (unsigned long long)(clock64() - t_begin));
-      atomicAdd((unsigned long long*)w.phase_dbg + 9, (unsigned long long)t_full);
-      atomicAdd((unsigned long long*)w.phase_dbg + 10, (unsigned long long)t_epi);
+      atomicAdd((unsigned long long*)w.phase_dbg + 9, (unsigned long long)mma.t_full);
+      atomicAdd((unsigned long long*)w.phase_dbg + 10, (unsigned long long)mma.t_epi);
     }
   } else if (warp < Geo<PL>::EW) {
     // ---------------- prologue + epilogues: thread = (point r, column half) ----------------
     constexpr int NB = Geo<PL>::NB;
     const int half = warp >> 2, r = (warp & 3) * 32 + lane, c0 = half * NB;
-    const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+    pp::Epi<PL, F16> epi{pipe.blk, pipe.acc_ready, tmem + ((uint32_t)((warp & 3) * 32) << 16), r, lane, w.phase_dbg != nullptr, false};
     const size_t row = g * TP + r;
     const float* pet = w.pet + g * (size_t)(C * TP) + r;
     const uint8_t* pe6 = w.pe6_blob + g * Geo<PL>::BC;
     const uint64_t pol_keep = l2_policy_evict_last();
-    uint32_t ar0 = 0u, ar1 = 0u;
-    const uint32_t R0 = lane_base, R1 = lane_base + p2z::REGION;
-    // this warp's part of block i is in tensor memory (and, for the prologue, in the zd tile in shared memory): one arrival per warp
-    auto blk_done = [&](const int i) { tmem_st_wait(); tc_fence_before(); fence_proxy_async(); __syncwarp(); if (lane == 0) mbar_arrive(&pipe.blk[i]); };
-    long long t_acc = 0, t_pro = 0;
+    const uint32_t R0 = epi.lane_base, R1 = epi.lane_base + pp::REGION;
+    long long t_pro = 0;
     const long long t_begin = clock64();
-    const bool timed = w.phase_dbg != nullptr;
-    auto acc_wait = [&](const int region) {
-      const uint32_t par = (region ? ar1 : ar0) & 1u;
-      if (timed) mbar_wait_t(&pipe.acc_ready[region], par, t_acc); else mbar_wait(&pipe.acc_ready[region], par);
-      if (region) ++ar1; else ++ar0;
-      tc_fence_after();
-    };
-    // 32 columns of this row, already scaled: split once -> workspace tile (wgrad operand) and / or the next A operand in TMEM
-    auto emit = [&](const int cg, const float (&v)[32], uint8_t* blob, const uint32_t blk_addr) {
-      uint32_t hi[16], lo[16];
-#pragma unroll
-      for (int qd = 0; qd < 4; ++qd) {
-        uint4 pq[PL];
-        split8<PL, F16>(v + qd * 8, pq);
-        if (blob) {
-          const uint32_t off = gp_off(32, r, cg * 4 + qd);
-          __stcs(reinterpret_cast<uint4*>(blob + off), pq[0]);
-          if (PL == 2) __stcs(reinterpret_cast<uint4*>(blob + BLOB_H + off), pq[PL - 1]);
-        }
-        hi[qd * 4 + 0] = pq[0].x; hi[qd * 4 + 1] = pq[0].y; hi[qd * 4 + 2] = pq[0].z; hi[qd * 4 + 3] = pq[0].w;
-        lo[qd * 4 + 0] = pq[PL - 1].x; lo[qd * 4 + 1] = pq[PL - 1].y; lo[qd * 4 + 2] = pq[PL - 1].z; lo[qd * 4 + 3] = pq[PL - 1].w;
-      }
-      tmem_st16(blk_addr, hi);                                         // in place: the planes replace the accumulator block they came from
-      if (PL == 2) tmem_st16(blk_addr + 16, lo);
-    };
+    const bool timed = epi.timed;
     for (int i = tid; i < H + 4; i += Geo<PL>::ET) csum[i] = 0.f;
     for (int k = 0; k < w.Kn; ++k) {
       uint8_t* nt = net_tile<PL>(w, b, k, tl);
@@ -1074,11 +1080,11 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         }
         tmem_st8(R1 + it * 12, hi); tmem_st4(R1 + it * 12 + 8, hi + 8);
         if (PL == 2) { tmem_st8(R1 + p2z::ZP_LO + it * 12, lo); tmem_st4(R1 + p2z::ZP_LO + it * 12 + 8, lo + 8); }
-        blk_done(it - half * NB);
+        epi.blk_done(it - half * NB, true);               // (and its part of the zd tile is in shared memory)
       }
       if (timed) t_pro += clock64() - t_p0;
       // ---- epilogue 7: zh = m1 (acc + dov b1) ----
-      acc_wait(0);
+      epi.acc_wait(0);
 #pragma unroll 1
       for (int cb = 0; cb < NB; ++cb) {
         const int cg = c0 + cb;
@@ -1098,11 +1104,11 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
             v[j] = ((bits >> j) & 1u) ? z : 0.f;
           }
         }
-        emit(cg, v, blob_h<PL>(nt, B_ZH), R0 + cg * 32);
-        blk_done(cb);
+        epi.emit(cg, v, blob_h<PL>(nt, B_ZH), true, R0 + cg * 32);
+        epi.blk_done(cb, true);
       }
       // ---- epilogue 8: zc = acc + dov (b2 + bd + e) -> workspace (Z operand of dWa);  column sum -> vc ----
-      acc_wait(1);
+      epi.acc_wait(1);
 #pragma unroll 1
       for (int cb = 0; cb < NB; ++cb) {
         const int cg = c0 + cb;
@@ -1147,16 +1153,13 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
     if (timed && tid == 0) {
       const long long tot = clock64() - t_begin;
       atomicAdd((unsigned long long*)w.phase_dbg + 12, (unsigned long long)tot);
-      atomicAdd((unsigned long long*)w.phase_dbg + 13, (unsigned long long)t_acc);
-      atomicAdd((unsigned long long*)w.phase_dbg + 15, (unsigned long long)(tot - t_acc));
+      atomicAdd((unsigned long long*)w.phase_dbg + 13, (unsigned long long)epi.t_acc);
+      atomicAdd((unsigned long long*)w.phase_dbg + 15, (unsigned long long)(tot - epi.t_acc));
       atomicAdd((unsigned long long*)w.phase_dbg + 11, (unsigned long long)t_pro);
       atomicAdd((unsigned long long*)w.phase_dbg + 14, 1ull);
     }
   }
-  tc_fence_before();
-  __syncthreads();
-  if (CLUSTER > 1) cluster_sync_all();
-  if (warp == Geo<PL>::W_MMA) tmem_dealloc(tmem, 512);
+  pp::block_end<PL>(tmem, warp);
 }
 
 // ------------------------------------------------------------------------------------------------
