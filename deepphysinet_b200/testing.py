@@ -48,7 +48,8 @@ def run_library(W, pts, consts=None, mode="fp32", want_fields=True, n_norm=0):
 
 
 def oracle_reference(W, pts, consts=None):
-    """fp64 CPU oracle (autograd restatement of the reference) on the same inputs; mean over samples."""
+    """fp64 CPU oracle (autograd restatement of the reference) on the same inputs and every constant of `consts`; mean over
+    samples."""
     from oracle import dpn_oracle as O
     consts = consts or PhysicsConsts()
     B = W.W1.shape[0]
@@ -64,6 +65,7 @@ def oracle_reference(W, pts, consts=None):
         tb, tt, v, j = O.place_generated(col("x"), col("y"), col("t"), col("f"), pts["coord_data"][b].detach().double().cpu(),
                                          Wb, dx=consts.dx, dy=consts.dy, lat_size=consts.lat_size, lon_size=consts.lon_size,
                                          pred_t_span=consts.pred_t_span, with_clip=consts.with_clip, factors=factors,
+                                         norm=O.norm_of(consts), c_p=consts.c_p, L=consts.L, R_v=consts.R_v, R_d=consts.R_d,
                                          return_fields=True)
         total = total + tb / B
         terms.append(torch.stack([a.detach() for a in tt]))

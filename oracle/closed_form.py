@@ -59,12 +59,21 @@ def coord_features(x, y, t, dx, dy, lat_size, lon_size, t_span):
     return pe, dpe
 
 
-def residual_and_seeds(o, od, f, n_total, scales, with_clip=True, fact=FACT):
-    """o [N,6] normalised outputs, od [N,6,3] z-space derivatives, f [N,1].
+def kwargs_of(consts):
+    """pde_fwd_bwd keywords carrying every constant of a deepphysinet_b200.config.PhysicsConsts."""
+    return dict(dx=consts.dx, dy=consts.dy, lat_size=consts.lat_size, lon_size=consts.lon_size, t_span=consts.pred_t_span,
+                with_clip=consts.with_clip,
+                phys=dict(mean=consts.mean, std=consts.std, lo=consts.lo, hi=consts.hi, fact=consts.factor, c_p=consts.c_p,
+                          L=consts.L, R_v=consts.R_v, R_d=consts.R_d))
+
+
+def residual_and_seeds(o, od, f, n_total, scales, with_clip=True, fact=FACT, mean=MEAN, std=STD, lo=LO, hi=HI,
+                       c_p=1005.0, L=2.5e6, R_v=461.5, R_d=287.0):
+    """o [N,6] normalised outputs, od [N,6,3] z-space derivatives, f [N,1]; the constants default to the reference config.
     Returns loss sums [6] (already * factor / n_total), seeds dov [N,6], dod [N,6,3], vals, jac(physical)."""
     dt = o.dtype
-    mean, std = torch.tensor(MEAN, dtype=dt), torch.tensor(STD, dtype=dt)
-    lo, hi = torch.tensor(LO, dtype=dt), torch.tensor(HI, dtype=dt)
+    mean, std = torch.tensor(mean, dtype=dt), torch.tensor(std, dtype=dt)
+    lo, hi = torch.tensor(lo, dtype=dt), torch.tensor(hi, dtype=dt)
     raw = o * std + mean
     kap = torch.ones_like(raw)
     vals = raw.clone()
@@ -78,7 +87,7 @@ def residual_and_seeds(o, od, f, n_total, scales, with_clip=True, fact=FACT):
     gy = lambda i: jac[:, i, 1:2]
     gt = lambda i: jac[:, i, 2:3]
     D = lambda i: gt(i) + u * gx(i) + v * gy(i)
-    c_p, L, R_v, R_d, eps = 1005.0, 2.5e6, 461.5, 287.0, 1e-6
+    eps = 1e-6
     r1 = D(0) + gx(2) / r - f * v
     r2 = D(1) + gy(2) / r + f * u
     r3 = D(5) + r * (gx(0) + gy(1))
@@ -121,10 +130,11 @@ def residual_and_seeds(o, od, f, n_total, scales, with_clip=True, fact=FACT):
 
 
 def pde_fwd_bwd(x, y, t, f, coord_data, W, *, dx=27000.0, dy=27000.0, lat_size=145, lon_size=257,
-                t_span=86400.0, with_clip=True, rnd=lambda a: a, n_total=None, return_stages=False):
+                t_span=86400.0, with_clip=True, rnd=lambda a: a, n_total=None, phys=None, return_stages=False):
     """One sample.  W: dict of stacked per-net tensors
        W1 [6,256,192] b1 [6,256] W2 [6,256,256] b2 [6,256] e [6,256]
        Wd [6,256,192] bd [6,256] Wa [6,256,256] ba [6,256] Wb [6,256,256] bb [6,256] wo [6,256] bo [6].
+    phys: keywords of residual_and_seeds (normalisation, factors, physical constants); kwargs_of(consts) gives all of them.
     Returns (loss_terms[6], grads dict, vals [N,6], jac [N,6,3]) (+ stages dict)."""
     N = x.shape[0]
     n_total = n_total or N
@@ -151,7 +161,7 @@ def pde_fwd_bwd(x, y, t, f, coord_data, W, *, dx=27000.0, dy=27000.0, lat_size=1
         jin = rnd(qm) @ w1                                              # [N,192] = do/dPE
         od[:, k, :] = (jin * dpe).reshape(N, 64, 3).sum(1)
         st.append(dict(h1=h1, c=c, g=g, um=um, yv=yv, qm=qm, m1=m1, m3=m3, uvec=uvec, jin=jin))
-    losses, dov, dod, vals, jac = residual_and_seeds(o, od, f, n_total, scales, with_clip)
+    losses, dov, dod, vals, jac = residual_and_seeds(o, od, f, n_total, scales, with_clip, **(phys or {}))
     G = {k_: torch.zeros_like(v) for k_, v in W.items()}
     for k in range(6):
         s = st[k]

@@ -137,11 +137,17 @@ def physics_net_decode(meta_out, coord_pe, coord_data, fore_h, params):
     return decode_generated(coord_pe, coord_data, stack_generated(meta_out, fore_h, params))
 
 
-def inverse_norm(outs: Sequence[torch.Tensor], with_clip: bool):
-    """interface/interface_physics.py:232-262: mean_norm de-normalisation; clip on P,T,q,rio only."""
+def norm_of(consts) -> Dict[str, tuple]:
+    """OBS_NORM-shaped {key: (mean, std, lo, hi)} of a deepphysinet_b200.config.PhysicsConsts."""
+    return {k: (consts.mean[i], consts.std[i], consts.lo[i], consts.hi[i]) for i, k in enumerate(OBS_KEYS)}
+
+
+def inverse_norm(outs: Sequence[torch.Tensor], with_clip: bool, norm: Dict[str, tuple] = OBS_NORM):
+    """interface/interface_physics.py:232-262: mean_norm de-normalisation; clip on P,T,q,rio only.
+    norm: {key: (mean, std, lo, hi)} of the config's obs_norm_cfg (default: the reference config)."""
     res = []
     for i, key in enumerate(OBS_KEYS):
-        mu, sd, lo, hi = OBS_NORM[key]
+        mu, sd, lo, hi = norm[key]
         v = outs[i] * sd + mu
         if with_clip and i >= 2:
             v = torch.clip(v, lo, hi)
@@ -203,10 +209,12 @@ def residual_losses(x, y, t, f, u, v, p, T, q, rio, factors=LOSS_FACTOR, c_p=100
 
 
 def place_generated(x, y, t, f, coord_data, W, *, dx=27000.0, dy=27000.0, lat_size=145, lon_size=257,
-                    pred_t_span=86400.0, with_clip=True, factors=LOSS_FACTOR, return_fields=False):
+                    pred_t_span=86400.0, with_clip=True, factors=LOSS_FACTOR, norm=OBS_NORM, c_p=1005, L=2.5e6, R_v=461.5, R_d=287,
+                    return_fields=False):
     """interface/interface_physics.py:271-320 for ONE sample, from the fused operator's own inputs.
 
     x, y, t, f: [N,1]; coord_data [N,6]; W = stack_generated(...) (tensors may require grad).
+    norm, factors, c_p, L, R_v, R_d: the constants of inverse_norm and residual_losses (defaults: the reference's).
     Returns (total, [6 terms]) and, with return_fields, also (vals [N,6] physical, jac [N,6,3] d/dx,dy,dt).
     """
     x = x.detach().clone().requires_grad_(True)
@@ -214,8 +222,8 @@ def place_generated(x, y, t, f, coord_data, W, *, dx=27000.0, dy=27000.0, lat_si
     t = t.detach().clone().requires_grad_(True)
     pe = encoding_coord(x, y, t, dx, dy, lat_size, lon_size, pred_t_span)
     outs = decode_generated(pe, coord_data, W)
-    u, v, p, T, q, rio = inverse_norm(outs, with_clip)
-    terms = residual_losses(x, y, t, f, u, v, p, T, q, rio, factors)
+    u, v, p, T, q, rio = inverse_norm(outs, with_clip, norm)
+    terms = residual_losses(x, y, t, f, u, v, p, T, q, rio, factors, c_p, L, R_v, R_d)
     total = terms[0] + terms[1] + terms[3] + terms[2] + terms[4] + terms[5]   # summation order of :301
     if not return_fields:
         return total, terms

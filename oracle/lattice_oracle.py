@@ -20,14 +20,16 @@ def node_coords(lat, k, j, i):
 
 
 def node_values(coarse, W, x, y, t, dx=27000.0, dy=27000.0, lat_size=145, lon_size=257, pred_t_span=86400.0,
-                cells_per_coarse=4.0, t_step=6 * 3600.0):
+                cells_per_coarse=4.0, t_step=6 * 3600.0, consts=None):
     """Physical values [n, 6] (float64) of one sample at points x, y, t: coarse [Tt,Hc,Wc,6], W a dict of that sample's
-    decoder tensors in dpn_oracle layout (W1 [6,256,192], ..., Wd [6,256,192], ...)."""
+    decoder tensors in dpn_oracle layout (W1 [6,256,192], ..., Wd [6,256,192], ...).  consts: the PhysicsConsts whose
+    mean / std de-normalise (default: the reference config); the geometry is given by the keywords."""
     cd = torch.from_numpy(SO.trilinear(np.asarray(coarse), x, y, t, dx=dx, dy=dy, cells_per_coarse=cells_per_coarse, t_step=t_step))
     col = lambda a: torch.from_numpy(np.asarray(a, dtype=np.float64)).reshape(-1, 1)
     pe = O.encoding_coord(col(x), col(y), col(t), dx, dy, lat_size, lon_size, pred_t_span)
     with torch.no_grad():
-        return torch.cat(O.inverse_norm(O.decode_generated(pe, cd, W), with_clip=False), 1)
+        return torch.cat(O.inverse_norm(O.decode_generated(pe, cd, W), with_clip=False,
+                                         norm=O.OBS_NORM if consts is None else O.norm_of(consts)), 1)
 
 
 def lattice_values(coarse, W, lat, **geom):
