@@ -15,14 +15,15 @@
 //   pass 1  G1 a1 = PE W1^T            -> h1 = relu(a1+b1), mask m1
 //           G2 c  = h1 W2^T + PE6 Wd^T -> c + (b2+bd+e);  o += 2wo.c
 //           G3 a3 = c Wa^T             -> g = relu(a3+ba), o += u.g (u = Wb^T wo: out_fc folded through cat_fc1.fc.2), mask m3
-//           G4 y  = (u*m3) Wa + 2wo = m3 (diag(u) Wa) + 2wo    reverse sweep of the scalar output: do/dc   (the bare mask is the A operand)
-//           G5 q  = y W2, qm = q*m1    do/da1
+//           G4 q  = y W2 = m3 P + c2,  qm = q*m1     reverse sweep of the scalar output: do/da1, where y = (u*m3) Wa + 2wo = do/dc is
+//                                         never formed: P = diag(u) Wa W2, c2 = 2 W2^T wo per (sample, net), the bare mask is the A operand
 //           G6 jin = qm W1             do/dPE  -> do/dz_c = jin . dPE_c   (the 3 Jacobian columns)
 //   residual kernel (fp64, shared with the fp32 mode) -> loss terms + seeds dL/do, dL/d(do/dz_c)
 //   pass 2  the Z-side rows  zp = dov PE + sum_c seed_c dPE_c, zd = dov PE6, zh = dov h1 + ht, zc = dov c + ct  as the FORWARD pass of the
 //           combined row zp with frozen masks and dov-scaled biases (G7', G8'); gz = dov g + gt is never formed - its column sum
 //           comes out of the dWa contraction
-//   wgrad   dW1 = qm^T zp, dW2 = y^T zh, dWa = diag(u) (m3^T zc), dWd = y^T zd  : K = points contractions, MN-major operands
+//   wgrad   dW1 = qm^T zp, diag(u) m3^T [zh | zd | zc] : K = points contractions, MN-major operands;  dW2 = y^T zh and dWd = y^T zd
+//           follow after the last chunk as Wa^T (diag(u) m3^T z) + 2wo (x) sum_p z  (unfold_kernel)
 //   colsum  bias gradients and the two vectors the folded output layer needs (vc, vg)
 //
 // Every [128 x Kd] 16-bit operand tile ("blob") is stored in the layout (*) of dpn_umma.cuh in shared memory (and, 32 points at a
@@ -57,9 +58,10 @@ constexpr int CLUSTER = DPN_CLUSTER;                     // CTAs (tiles of the s
 constexpr int AUX_BYTES = TP * 16 * 2;        // 4096   [128 x 16] 16-bit seed tile: col 0/1/2 = the three 16-bit terms of dov
 constexpr int IMG_HC = H * C * 2;             // 98304
 constexpr int IMG_HH = H * H * 2;             // 131072
-constexpr int GEN_IMG = 2 * IMG_HC + 2 * IMG_HH;   // per (sample, net): W1, W1T, W2, W2T
-constexpr int STA_IMG = IMG_HC + 2 * IMG_HH;       // per net: Wd, Wa, (diag(u) Wa)^T
-// Workspace tile of one (net, point tile):  YT QM ZH ZC | ZP ZD | AUX | MASK.  Pass 2 runs as the forward pass of the combined row
+constexpr int GEN_IMG = 2 * IMG_HC + 2 * IMG_HH;   // per (sample, net): W1, W1T, W2, P^T (P = diag(u) Wa W2)
+constexpr int STA_IMG = IMG_HC + 2 * IMG_HH;       // per net: Wd, Wa, one unused [256 x 256] slot (the workspace sizes are pinned)
+// Workspace tile of one (net, point tile):  YT QM ZH ZC | ZP ZD | AUX | MASK.  No kernel writes the YT slot: the first tile of a
+// (sample, net) keeps scratch() there (the workspace sizes are pinned).  Pass 2 runs as the forward pass of the combined row
 // (DESIGN.md section 3) and needs only the ReLU mask m1 of pass 1 (256 bits per point) instead of the h1 / c / g tiles (3 x 1 KB per
 // point), and the weight-gradient kernel builds its J operand [a3 > 0] from the m3 mask bits instead of reading a stored tile.
 constexpr int NBLOB_H = 4, NBLOB_C = 2;
@@ -114,6 +116,8 @@ struct Work {
   float *o, *od, *dov, *dod;   // [B*T*TP][Kn], [..][Kn][3]
   float *vc, *vg, *sdo;        // [Kn][H] column sums of zc / of the never-formed gz, and [Kn] sum of dov
   const NetScales* sc;         // [B][Kn] scaling plan (fp16 variant only)
+  uint8_t* scr;                // per-(sample, net) scratch of the reverse sweep: scr + (b Kn + k) scr_stride (see scratch())
+  size_t scr_stride;
   long long* phase_dbg;        // optional [kernel(2)][8] cycle counters (debug builds with DPN_PHASE_DEBUG=1), summed over CTAs
   int xfirst;                  // cross-first accumulation of G1 - G3 (DPN_MODE_F16X3A)
   int dbg_flags;               // DEBUG BUILDS ONLY (tools/build_debug.sh, DPN_DEBUG_FLAGS): 1 = no MMAs, 2 = empty epilogues, 4 = no tile stores
@@ -134,6 +138,13 @@ template <int PL> __device__ __forceinline__ uint8_t* blob_zp(uint8_t* nt) { ret
 template <int PL> __device__ __forceinline__ uint8_t* blob_zd(uint8_t* nt) { return nt + off_zd<PL>(); }
 template <int PL> __device__ __forceinline__ uint8_t* blob_aux(uint8_t* nt) { return nt + off_aux<PL>(); }
 template <int PL> __device__ __forceinline__ uint8_t* blob_mask(uint8_t* nt) { return nt + off_mask<PL>(); }
+// Per-(sample, net) scratch of the reverse sweep (fp32), in the YT slot of workspace tile index (b Kn + k) Tc, Tc = the tiles per
+// sample of a full chunk: no kernel writes a YT slot (DESIGN.md section 4), and the address is the same for every chunk of a call.
+//   c2 = 2 W2^T wo (pass 1, epilogue 4) | sum_p zh | sum_p dov | (b = 0 only) sum_{b,p} zd  - the last three accumulate over chunks
+// and are turned into dW2, db2 and dWd by unfold_kernel after the last chunk.  P = diag(u) Wa W2 (fp32, [H][H]) is formed in the
+// QM .. ZC slots of the same tile before pass 1 of the first chunk writes them.
+enum { SCR_C2 = 0, SCR_SZH = H, SCR_SDO = 2 * H, SCR_SZD = 2 * H + 32 };   // float offsets
+__host__ __device__ __forceinline__ float* scratch(uint8_t* scr, size_t stride, int bk) { return reinterpret_cast<float*>(scr + (size_t)bk * stride); }
 
 // ------------------------------------------------------------------------------------------------
 // Small helpers
@@ -217,8 +228,8 @@ __device__ __forceinline__ void stg8(uint8_t* tile, uint32_t plane, uint32_t off
 // ------------------------------------------------------------------------------------------------
 struct NetScales {                       // one per (sample, net)
   float sW1, sW2, sWd, sWa;              // weight images (a matrix and its transpose share the factor)
-  float sWaU;                            // the image of diag(u) Wa (B operand of G4, whose A operand is the bare m3 mask)
-  float sH1, sC, sG, sUM, sY, sQ;        // tiles written by pass 1: h1, c, g, u*m3, y, q*m1
+  float sP;                              // the image of P^T, P = diag(u) Wa W2 (B operand of G4, whose A operand is the bare m3 mask)
+  float sH1, sC, sG, spare0, spare1, sQ; // tiles written by pass 1: h1, c, g, q*m1 (spare0 / 1 keep the pinned workspace size)
   float M1, Mc, l1W1, l1W12;             // bounds of |h1|, |c|; L1(W1), L1(W1) L1(W2)
   float rowB;                            // max(1, L1(W1), L1(W1) L1(W2)): growth of the pass-2 tangent row over its chain
   float cap;                             // largest sH1 * sW2 this (sample, net) can carry (plan_kernel takes the min over samples)
@@ -561,8 +572,8 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
     for (int k = 0; k < w.Kn; ++k) {
       const uint8_t* gen = w.img_gen + ((size_t)b * w.Kn + k) * Geo<PL>::GEN;
       const uint8_t* sta = w.img_sta + (size_t)k * Geo<PL>::STA;
-      const uint8_t *iW1 = gen, *iW1T = gen + PL * IMG_HC, *iW2 = gen + PL * 2 * IMG_HC, *iW2T = gen + PL * (2 * IMG_HC + IMG_HH);
-      const uint8_t *iWd = sta, *iWa = sta + PL * IMG_HC, *iWaT = sta + PL * (IMG_HC + IMG_HH);
+      const uint8_t *iW1 = gen, *iW1T = gen + PL * IMG_HC, *iW2 = gen + PL * 2 * IMG_HC, *iPT = gen + PL * (2 * IMG_HC + IMG_HH);
+      const uint8_t *iWd = sta, *iWa = sta + PL * IMG_HC;
       // the MMA warp's order: G1 | G2b (PE6 slices: no dependence on an epilogue, issued first) | TS-form GEMMs in block order.
       // Cross-first GEMMs (G1 - G3 when masks matter, see the MMA warp) read every chunk twice: whole chunks for the cross terms,
       // then the hi planes again for the main terms.
@@ -577,8 +588,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       for (int i = 0; i < 16; ++i) wr.put(iWa + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
       if (xfirst) for (int c = 0; c < 16; ++c) wr.put(iWa + (size_t)c * TS::W_BYTES, TS::W_BYTES, nullptr, true);
       if (sweep) {
-        for (int i = 0; i < 16; ++i) wr.put(iWaT + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
-        for (int i = 0; i < 16; ++i) wr.put(iW2T + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
+        for (int i = 0; i < 16; ++i) wr.put(iPT + (size_t)pp::block_order(i) * TS::W_BYTES, TS::W_BYTES, nullptr);
         if (sweep > 1)
           for (int i = 0; i < 16; ++i) wr.put(iW1T + (size_t)pp::block_order(i) * (PL * 6144), PL * 6144, nullptr);
       }
@@ -618,8 +628,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       if (xfirst) { gemm_ts(H, false, pp::P_CROSS); gemm_ts_main(); } else gemm_ts(H, false);
       ready();                                                             // G3 (A = c)
       if (sweep) {
-        gemm_ts(H, false, pp::P_EXACT); ready();                             // G4 (A = the m3 mask, B = diag(u) Wa: two MMAs per chunk)
-        gemm_ts(H, false); ready();                                        // G5 (A = y)
+        gemm_ts(H, false, pp::P_EXACT); ready();                             // G4 (A = the m3 mask, B = P^T: two MMAs per chunk)
         if (sweep > 1) { gemm_ts(C, false); ready(); }                     // G6 (A = qm, N = 192)
       }
     }
@@ -654,24 +663,25 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       uint8_t* nt = net_tile<PL>(w, b, k, tl);
       // fp16 variant: an accumulator carries (A tile scale) x (weight image scale); k1 .. k6 undo that AND apply the scale of the tile
       // the epilogue produces, and the bias vectors are staged pre-multiplied by the same power of two (exact), so that
-      // value -> next operand is ONE FMA per element:  h1 sH1 = max(acc k1 + b1 sH1, 0),  c sC = acc k2 + bsum sC,  y sY = acc k4 + 2wo sY
-      float k1 = 1.f, k2 = 1.f, i3 = 1.f, k4 = 1.f, i5 = 1.f, i6 = 1.f, sH1 = 1.f, sC = 1.f, sY = 1.f;
+      // value -> next operand is ONE FMA per element:  h1 sH1 = max(acc k1 + b1 sH1, 0),  c sC = acc k2 + bsum sC.
+      // Epilogue 4 takes two steps, q sQ = (acc / sP) sQ + c2 sQ: acc / sP is the real value m3 P (bounded by the fp32 inputs), so
+      // neither step leaves the fp32 range, whereas sQ / sP alone can (both lie in [2^-80, 2^80]).
+      float k1 = 1.f, k2 = 1.f, i3 = 1.f, i4 = 1.f, i6 = 1.f, sH1 = 1.f, sC = 1.f, sQ = 1.f;
       if (F16) {
         const NetScales t = w.sc[b * w.Kn + k];
-        sH1 = t.sH1; sC = t.sC; sY = t.sY;
-        k1 = sH1 / (S_PE * t.sW1); k2 = sC / (t.sH1 * t.sW2); i3 = 1.f / (t.sC * t.sWa); k4 = sY / t.sWaU;
-        i5 = t.sQ / (t.sY * t.sW2); i6 = 1.f / (t.sQ * t.sW1);
+        sH1 = t.sH1; sC = t.sC; sQ = t.sQ;
+        k1 = sH1 / (S_PE * t.sW1); k2 = sC / (t.sH1 * t.sW2); i3 = 1.f / (t.sC * t.sWa); i4 = 1.f / t.sP;
+        i6 = 1.f / (t.sQ * t.sW1);
       }
       epi_bar<PL>();
-      if (tid < H) {                                                   // V_B1: b1 sH1 | V_BSUM: bsum sC | V_BA, V_U | V_WO2: 2wo / sC (epilogue 2) | V_C2: 2wo sY (epilogue 4)
+      if (tid < H) {                                                   // V_B1: b1 sH1 | V_BSUM: bsum sC | V_BA, V_U | V_WO2: 2wo / sC (epilogue 2) | V_C2: c2 sQ (epilogue 4)
         const size_t vb = ((size_t)b * w.Kn + k) * H, vk = (size_t)k * H;
-        const float wo2 = __ldg(w.wo2 + vk + tid);
         svec[V_B1 * H + tid] = __ldg(w.b1 + vb + tid) * sH1;
         svec[V_BSUM * H + tid] = __ldg(w.bsum + vb + tid) * sC;
         svec[V_BA * H + tid] = __ldg(w.ba + vk + tid);
         svec[V_U * H + tid] = __ldg(w.uvec + vk + tid);
-        svec[V_WO2 * H + tid] = wo2 * (1.f / sC);
-        svec[V_C2 * H + tid] = wo2 * sY;
+        svec[V_WO2 * H + tid] = __ldg(w.wo2 + vk + tid) * (1.f / sC);
+        if (sweep) svec[V_C2 * H + tid] = scratch(w.scr, w.scr_stride, b * w.Kn + k)[SCR_C2 + tid] * sQ;
       }
       epi_bar<PL>();
       uint32_t m1w[NB];
@@ -774,24 +784,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         rowsum[r * 4] = 0.f;
       }
       if (!sweep) continue;
-      // ---- epilogue 4: y = acc + 2wo ----
-      ra = acc_wait();
-#pragma unroll 1
-      for (int cb = 0; cb < NB; ++cb) {
-        const int cg = c0 + cb;
-        float v[32];
-        tmem_ld32(ra + cg * 32, v);
-#pragma unroll
-        for (int j4 = 0; j4 < 8; ++j4) {
-          const float4 wv = *reinterpret_cast<const float4*>(svec + V_C2 * H + cg * 32 + j4 * 4);      // 2wo sY
-          const float ww[4] = {wv.x, wv.y, wv.z, wv.w};
-#pragma unroll
-          for (int e = 0; e < 4; ++e) v[j4 * 4 + e] = F16 ? fmaf(v[j4 * 4 + e], k4, ww[e]) : v[j4 * 4 + e] + ww[e];
-        }
-        epi.emit(cg, v, blob_h<PL>(nt, B_YT), true, ra + cg * 32);
-        epi.blk_done(cb);
-      }
-      // ---- epilogue 5: qm = acc * m1 ----
+      // ---- epilogue 4: qm = m1 (acc + c2) ----
       ra = acc_wait();
 #pragma unroll 1
       for (int cb = 0; cb < NB; ++cb) {
@@ -802,7 +795,16 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
 #pragma unroll
         for (int i = 0; i < NB; ++i) bits = (cb == i) ? m1w[i] : bits;
 #pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = ((bits >> j) & 1u) ? (F16 ? v[j] * i5 : v[j]) : 0.f;
+        for (int j4 = 0; j4 < 8; ++j4) {
+          const float4 cv = *reinterpret_cast<const float4*>(svec + V_C2 * H + cg * 32 + j4 * 4);      // c2 sQ
+          const float cc[4] = {cv.x, cv.y, cv.z, cv.w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const int j = j4 * 4 + e;
+            const float qq = F16 ? fmaf(v[j] * i4, sQ, cc[e]) : v[j] + cc[e];
+            v[j] = ((bits >> j) & 1u) ? qq : 0.f;
+          }
+        }
         epi.emit(cg, v, blob_h<PL>(nt, B_QM), sweep > 1, ra + cg * 32);
         if (sweep > 1) epi.blk_done(cb);
       }
@@ -1006,9 +1008,10 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       // the scale of the tile an epilogue produces is folded into its FMA (powers of two: exact): zh sZH = m1 (acc k7 + (dov sZH) b1), ...
       const float k7 = i7 * sZH, k8 = i8 * sZC, dvH = dv * sZH, dvC = dv * sZC, dvP = dv * sZP, inv_sZC = 1.f / sZC;
       const float ddP[3] = {dd[0] * sZP, dd[1] * sZP, dd[2] * sZP};
-      // seed tile for the bias-gradient MMAs of the wgrad kernel: col 0/1/2 = dov split into three 16-bit terms, rest 0
+      // seed tile for the bias-gradient MMAs of the wgrad kernel: col 0/1/2 = dov split into three 16-bit terms, col 3 = an exact 1 on
+      // valid points (the column sums of zh / zd), rest 0
       if (half == 0) {
-        float a8[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        float a8[8] = {0.f, 0.f, 0.f, tl * TP + r < w.P ? 1.f : 0.f, 0.f, 0.f, 0.f, 0.f};
         if (F16) {
           const float x = dv * sDV;
           a8[0] = __half2float(__float2half_rn(x));
@@ -1148,7 +1151,11 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         atomicAdd(w.vc + (size_t)k * H + i, csum[i]);
         csum[i] = 0.f;
       }
-      if (tid == 0) { atomicAdd(w.sdo + k, csum[H]); csum[H] = 0.f; }
+      if (tid == 0) {
+        atomicAdd(w.sdo + k, csum[H]);
+        atomicAdd(scratch(w.scr, w.scr_stride, b * w.Kn + k) + SCR_SDO, csum[H]);
+        csum[H] = 0.f;
+      }
     }
     if (timed && tid == 0) {
       const long long tot = clock64() - t_begin;
@@ -1170,6 +1177,8 @@ struct WgradWork {
   const float* uvec;       // [Kn][H] u = Wb^T wo
   const float *Wa, *ba;    // [Kn][H][H], [Kn][H] fp32 (split modes: vg = sum_p gz from the dWa contraction, see wgrad2_kernel)
   float* vg;               // [Kn][H]
+  uint8_t* scr;            // per-(sample, net) scratch (see scratch()): sum_p zh, sum_p zd
+  size_t scr_stride;
   float *gW1, *gW2, *gWa, *gWd;
   float *gb1, *gb2, *ge, *gbd, *gba;
 };
@@ -1180,10 +1189,12 @@ struct WgradWork {
 // HBM-bound (it reads every operand tile pass 1 / pass 2 wrote), so the structure follows the bytes:
 //   * tiles are stored [point quarter][k-core][32 rows][16 B] (gp_off), so a 32-point quarter of every operand is contiguous; THREE
 //     stages of 73 KB: the bulk loads of quarter-tiles i+1, i+2 run under the MMAs of quarter-tile i;
-//   * three kinds of work item per (sample, net):  0: dW1 = qm^T zp (+ db1);  1: dW2 = y^T zh AND dWd = y^T zd (+ db2) - the two layers
-//     that share J = y run in ONE item with a 256 + 192 column accumulator, so the y tile is read once (-15 % of the kernel's bytes);
-//     2: S = m3^T zc with J = [a3 > 0] as one exact 16-bit plane built from the mask bits of pass 1 (two MMAs per step instead of
-//     three, no stored J tile).  Its epilogue derives three results from S and the seed product sm3 = sum_p m3 dov:
+//   * three kinds of work item per (sample, net):  0: dW1 = qm^T zp (+ db1);  1 and 2 have J = [a3 > 0] as one exact 16-bit plane
+//     built from the mask bits of pass 1 (two MMAs per step and Z plane instead of three, no stored J tile):
+//     1: diag(u) m3^T zh AND diag(u) m3^T zd (+ u sm3) in ONE item with a 256 + 192 column accumulator, plus the column sums
+//     sum_p zh, sum_p zd (the Z half-tiles against the seed tile's column of ones) - y = m3 (diag(u) Wa) + 2wo is never stored, and
+//     unfold_kernel turns these into dW2 = y^T zh, dWd = y^T zd, db2 after the last chunk;
+//     2: S = m3^T zc.  Its epilogue derives three results from S and the seed product sm3 = sum_p m3 dov:
 //     dWa = diag(u) S,  dba = u sm3,  and the column sum of the never-formed tile gz = m3 (zc Wa^T + dov ba):
 //     vg[j] = sum_i Wa[j,i] S[j,i] + ba[j] sm3[j]  - which is why pass 2 has no third GEMM;
 //   * bias gradients are seed-tile products (an N = 16 MMA of the same J planes against the three 16-bit terms of dov);
@@ -1224,13 +1235,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
   int item = blockIdx.x;
   const int mh = item & 1; item >>= 1;                               // output half == cluster rank
   const int split = item % w.splits; item /= w.splits;
-  const int kind = item % wg2::ITEMS; item /= wg2::ITEMS;            // 0: dW1   1: dW2 + dWd   2: dWa (mask)
+  const int kind = item % wg2::ITEMS; item /= wg2::ITEMS;            // 0: dW1   1: dW2 + dWd (mask)   2: dWa (mask)
   const int k = item % w.Kn, b = item / w.Kn;
   const int N1 = kind == 0 ? C : H;                                   // columns of the first Z tile (zp | zh | zc)
   const bool two = kind == 1;                                         // second Z tile: zd, N = 192
-  const bool build_j = kind == 2;
+  const bool build_j = kind > 0;
   const uint32_t z1plane = (uint32_t)wg2::PT * N1 * 2;                // bytes of one plane of a Z1 quarter-tile
-  const int jsel = kind == 0 ? B_QM : B_YT;
+  const int jsel = B_QM;
   const int t0 = (int)((long long)w.T * split / w.splits), t1 = (int)((long long)w.T * (split + 1) / w.splits);
   const int nst = 4 * (t1 - t0);                                      // quarter-tiles
   if (tid == 0) {
@@ -1244,7 +1255,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
   tc_fence_after();
   cluster_sync_all();                                                // the peer's barriers exist before anything is multicast to them
   const uint32_t tmem = tmem_s;
-  constexpr uint32_t COL_D2 = 256, COL_X = 448;                       // TMEM: D1 [0,256) | D2 (dWd) [256,448) | seed product [448,464)
+  // TMEM: D1 [0,256) | D2 (dWd) [256,448) | seed products: J [448,464), zh half-tile [464,480), zd half-tile [480,496)
+  constexpr uint32_t COL_D2 = 256, COL_X = 448, COL_SZH = 464, COL_SZD = 480;
   if (nst > 0) {
     if (warp == 4) {
       for (int i = 0; i < nst; ++i) {
@@ -1272,6 +1284,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
       }
     } else if (warp == 5) {
       const uint32_t idesc1 = idesc_16(F16, N1, 1, 1), idesc2 = idesc_16(F16, C, 1, 1), idesc_x = idesc_16(F16, 16, 1, 1);
+      // the Z half-tile of this CTA as an A operand (the layout of a J plane): zh features 128 mh .., zd features 64 mh ..
+      const uint32_t zh_half = (uint32_t)mh * (wg2::J_PLANE >> 4), zd_half = (uint32_t)mh * (wg2::J_PLANE >> 5);
       // MN-major operands: 8-element groups of the M / N dimension are one k-core block of [32 points][16 B] = 512 bytes apart,
       // 8-point groups of the K dimension 128 bytes; a K = 16-point step adds 256 bytes (>> 4) to the address field
       constexpr uint32_t SBO = wg2::PT * 16;
@@ -1293,25 +1307,27 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
               mma_f16_c<A_FILL>(tmem, ad, b1, idesc1, first);
               if (two) mma_f16_c<A_USE>(tmem + COL_D2, ad, b2, idesc2, first);
               mma_f16_c<A_LAST>(tmem + COL_X, ad, xd, idesc_x, first);
-            } else if (build_j) {                            // exact one-plane J (the mask): J Z_lo + J Z_hi + J seeds
+            } else if (build_j) {                            // exact one-plane J (the mask): J Z_lo + J Z_hi (+ J Z2 likewise) + J seeds
               mma_f16_c<A_FILL>(tmem, ad, b1 + b1_lo, idesc1, first);
               mma_f16_c<A_USE>(tmem, ad, b1, idesc1, 1u);
+              if (two) {
+                mma_f16_c<A_USE>(tmem + COL_D2, ad, b2 + b2_lo, idesc2, first);
+                mma_f16_c<A_USE>(tmem + COL_D2, ad, b2, idesc2, 1u);
+              }
               mma_f16_c<A_LAST>(tmem + COL_X, ad, xd, idesc_x, first);
-            } else if (two) {                                // J = y against zh (D1) and zd (D2)
-              mma_f16_c<A_FILL>(tmem, ad + a_lo, b1, idesc1, first);
-              mma_f16_c<A_USE>(tmem + COL_D2, ad + a_lo, b2, idesc2, first);
-              mma_f16_c<A_LAST>(tmem + COL_X, ad + a_lo, xd, idesc_x, first);
-              mma_f16_c<A_FILL>(tmem, ad, b1 + b1_lo, idesc1, 1u);
-              mma_f16_c<A_USE>(tmem, ad, b1, idesc1, 1u);
-              mma_f16_c<A_USE>(tmem + COL_D2, ad, b2 + b2_lo, idesc2, 1u);
-              mma_f16_c<A_USE>(tmem + COL_D2, ad, b2, idesc2, 1u);
-              mma_f16_c<A_LAST>(tmem + COL_X, ad, xd, idesc_x, 1u);
             } else {
               mma_f16_c<A_FILL>(tmem, ad + a_lo, b1, idesc1, first);
               mma_f16_c<A_LAST>(tmem + COL_X, ad + a_lo, xd, idesc_x, first);
               mma_f16_c<A_FILL>(tmem, ad, b1 + b1_lo, idesc1, 1u);
               mma_f16_c<A_USE>(tmem, ad, b1, idesc1, 1u);
               mma_f16_c<A_LAST>(tmem + COL_X, ad, xd, idesc_x, 1u);
+            }
+            if (two) {                                       // column sums: the Z half-tiles (all planes) against the column of ones
+              const uint64_t zh_a = b1 + zh_half, zd_a = b2 + zd_half;
+              mma_f16_c<A_DISCARD>(tmem + COL_SZH, zh_a, xd, idesc_x, first);
+              if (PL == 2) mma_f16_c<A_DISCARD>(tmem + COL_SZH, zh_a + b1_lo, xd, idesc_x, 1u);
+              mma_f16_c<A_DISCARD>(tmem + COL_SZD, zd_a, xd, idesc_x, first);
+              if (PL == 2) mma_f16_c<A_DISCARD>(tmem + COL_SZD, zd_a + b2_lo, xd, idesc_x, 1u);
             }
           }
           mma_commit_mc(&empty[s], (uint16_t)3);                      // the stage is free in BOTH CTAs' eyes only when both have read it
@@ -1349,11 +1365,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
       float un1 = 1.f, un2 = 1.f, un_x = 1.f;                          // fp16 variant: undo (J tile scale) x (Z tile / seed scale)
       if (F16) {
         const NetScales t = w.sc[gk];
-        const float sj = kind == 0 ? t.sQ : (kind == 2 ? 1.f : t.sY);        // (the mask carries no scale)
+        const float sj = kind == 0 ? t.sQ : 1.f;                       // (the mask carries no scale)
         const float sz1 = kind == 0 ? t.sZP : (kind == 1 ? t.sZH : t.sZC);
-        un1 = (1.f / sj) * (1.f / sz1); un2 = (1.f / sj) * (1.f / t.sZD); un_x = (1.f / sj) * (1.f / t.sDV);   // separately: sj * sz may leave the fp32 range
+        un1 = (1.f / sj) * (1.f / sz1); un2 = 1.f / t.sZD; un_x = (1.f / sj) * (1.f / t.sDV);   // separately: sj * sz may leave the fp32 range
       }
-      // kind 2: this row of S = m3^T zc gives dWa[out,:] = u[out] S and the dot product with Wa[out,:] that vg needs
+      // kinds 1, 2: row `out` of m3^T z is scaled by u[out]; kind 2: this row of S = m3^T zc also gives the dot product with Wa[out,:]
+      // that vg needs
       const float urow = build_j ? __ldg(w.uvec + (size_t)k * H + out) : 1.f;
       const float* warow = w.Wa + ((size_t)k * H + out) * H;
       float dot0 = 0.f, dot1 = 0.f;
@@ -1365,7 +1382,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
         const float sc = un1 * urow;
         for (int cb = 0; cb < N1 / 32; ++cb) {
           tmem_ld32(lane_base + cb * 32, v);
-          if (build_j) {
+          if (kind == 2) {
 #pragma unroll
             for (int j4 = 0; j4 < 8; ++j4) {
               const float4 wv = __ldg(reinterpret_cast<const float4*>(warow + cb * 32) + j4);
@@ -1386,13 +1403,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
       if (two) {                                                       // second output of the merged item: dWd rows (the staging row is reused)
         float* dst = w.gWd + (size_t)k * H * C + (size_t)out * C;
         bulk_wait_read_all();
+        const float sc = un2 * urow;
         for (int cb = 0; cb < C / 32; ++cb) {
           tmem_ld32(lane_base + COL_D2 + cb * 32, v);
 #pragma unroll
           for (int j4 = 0; j4 < 8; ++j4)
-            *reinterpret_cast<float4*>(myrow + cb * 128 + j4 * 16) =
-                F16 ? make_float4(v[j4 * 4] * un2, v[j4 * 4 + 1] * un2, v[j4 * 4 + 2] * un2, v[j4 * 4 + 3] * un2)
-                    : make_float4(v[j4 * 4], v[j4 * 4 + 1], v[j4 * 4 + 2], v[j4 * 4 + 3]);
+            *reinterpret_cast<float4*>(myrow + cb * 128 + j4 * 16) = make_float4(v[j4 * 4] * sc, v[j4 * 4 + 1] * sc, v[j4 * 4 + 2] * sc, v[j4 * 4 + 3] * sc);
         }
         fence_proxy_async();
         bulk_red_add_f32(dst, myrow, (uint32_t)C * 4u);
@@ -1407,10 +1423,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
         } else if (kind == 2) {                                        // bsum = sum_p m3[p,out] dov[p]
           atomicAdd(w.gba + (size_t)k * H + out, urow * bsum);
           atomicAdd(w.vg + (size_t)k * H + out, fmaf(__ldg(w.ba + (size_t)k * H + out), bsum, (dot0 + dot1) * un1));
-        } else {
-          atomicAdd(w.gb2 + gk * H + out, bsum);
-          atomicAdd(w.ge + gk * H + out, bsum);
-          atomicAdd(w.gbd + (size_t)k * H + out, bsum);
+        } else {                                                       // u sm3; and the column sums of zh (features 128 mh + tid) and zd
+          atomicAdd(w.gb2 + gk * H + out, urow * bsum);                // (features 64 mh + tid: CTA 0 keeps [0, 96), CTA 1 [96, 192))
+          tmem_ld16(lane_base + COL_SZH, x);
+          float* scr = scratch(w.scr, w.scr_stride, (int)gk);
+          atomicAdd(scr + SCR_SZH + out, F16 ? x[3] * (1.f / w.sc[gk].sZH) : x[3]);
+          tmem_ld16(lane_base + COL_SZD, x);
+          if (mh == 0 ? tid < C / 2 : tid >= TP - C / 2)
+            atomicAdd(scratch(w.scr, w.scr_stride, k) + SCR_SZD + mh * (C - TP) + tid, F16 ? x[3] * (1.f / w.sc[gk].sZD) : x[3]);
         }
       }
       bulk_wait_read_all();                                            // the engine has read my row: shared memory may go away
@@ -1443,7 +1463,8 @@ __global__ void __launch_bounds__(1024) bounds_kernel(int Kn, const float* __res
                                                      const float* __restrict__ W2, const float* __restrict__ Wd,
                                                      const float* __restrict__ Wa, const float* __restrict__ ba,
                                                      const float* __restrict__ bsum, const float* __restrict__ uvec,
-                                                     const float* __restrict__ wo2, NetScales* __restrict__ tab) {
+                                                     const float* __restrict__ wo2, const uint8_t* __restrict__ Pm, size_t p_stride,
+                                                     NetScales* __restrict__ tab) {   // Pm: fp32 P of (b, k) at Pm + bk p_stride, or nullptr
   __shared__ float red[8];
   __shared__ float srow[8][H];                                       // per matrix row: L1 norm / maximum of W1, Wd, W2, Wa
   // 1024 threads: the block reads ~1.4 MB and one SM's memory-level parallelism is what bounds it (48 blocks on 148 SMs)
@@ -1498,18 +1519,24 @@ __global__ void __launch_bounds__(1024) bounds_kernel(int Kn, const float* __res
   const float mW1 = block_max256(m1, red), mW2 = block_max256(m2, red), mWd = block_max256(md, red), mWa = block_max256(ma, red);
   const float mBs = block_max256(fabsf(bsum[(size_t)bk * H + j]), red), mBa = block_max256(fabsf(ba[(size_t)k * H + j]), red);
   const float Mu = block_max256(fabsf(uvec[(size_t)k * H + j]), red), mWo2 = block_max256(fabsf(wo2[(size_t)k * H + j]), red);
-  const float mWaU = block_max256(fabsf(uvec[(size_t)k * H + j]) * ma, red);       // max |u_j Wa_ji|
+  float mp = 0.f;                                                    // max |P|
+  if (Pm) {
+    const float* pr = reinterpret_cast<const float*>(Pm + (size_t)bk * p_stride);
+    for (int i = 0; i < H; ++i) mp = fmaxf(mp, fabsf(pr[(size_t)i * H + j]));
+  }
+  const float mP = block_max256(mp, red);
   if (j == 0) {
     NetScales t;
     const float Mc = l1W2 * M1 + l1Wd + mBs, Mg = l1Wa * Mc + mBa;
     const float My = Mu * cWa + mWo2, Mq = My * cW2;
     t.sW1 = scale_for(mW1 * 32.f);                   // weights: maximum -> 2^10
     t.sWa = scale_for(mWa * 32.f);
-    t.sWaU = scale_for(mWaU * 32.f);
+    t.sP = scale_for(mP * 32.f);
     t.sWd = scale_for(mWd * 32.f);                   // preliminary: plan_kernel couples sWd, sH1 and sW2
     t.sW2 = scale_for(mW2);                          // preliminary: the LARGEST admissible factor
     t.sH1 = scale_for(M1); t.sC = scale_for(Mc); t.sG = scale_for(Mg);
-    t.sUM = scale_for(Mu); t.sY = scale_for(My); t.sQ = scale_for(Mq);
+    t.spare0 = t.spare1 = 1.f;
+    t.sQ = scale_for(Mq);
     t.M1 = M1; t.Mc = Mc; t.l1W1 = l1W1; t.l1W12 = l1W1 * l1W2;
     t.rowB = fmaxf(1.f, fmaxf(l1W1, l1W1 * l1W2));
     t.cap = t.sH1 * t.sW2;
@@ -1569,13 +1596,101 @@ __global__ void zscale_kernel(int n, const int* __restrict__ seedmax, NetScales*
   t.sDV = scale_for(DV);
 }
 
+// ---- the fold of the reverse sweep (DESIGN.md section 3), fp32 on the CUDA cores ----------------------------------------
+// out[m][n] = rs[m] sum_l A(m, l) X[l][n] + xv[m] yv[n]  for one [H x N] X per batch (blockIdx.y), A = Wa of net batch % Kn:
+// A(m, l) = Wa[m][l] (AT = false: P = diag(u) Wa W2 before pass 1) or Wa[l][m] (AT = true: Wa^T (diag(u) m3^T z) + 2wo (x) sum_p z
+// after the last chunk).  rs, xv: [Kn][H] or nullptr; yv: [N] per batch, sY floats apart.  A CTA owns the 32-column block
+// blockIdx.x of all H rows and has read its whole block of X before it writes, so X may be out (in place).
+template <bool AT>
+__global__ void __launch_bounds__(256) fold_gemm_kernel(int Kn, int N, const float* __restrict__ Wa, const float* X, size_t sX, float* out,
+                                                        size_t sOut, const float* __restrict__ rs, const float* __restrict__ xv,
+                                                        const float* __restrict__ yv, size_t sY) {
+  __shared__ __align__(16) float Xs[H][32];
+  __shared__ __align__(16) float As[16][H];
+  const int tid = threadIdx.x, n0 = blockIdx.x * 32, batch = blockIdx.y, k = batch % Kn;
+  const float* A = Wa + (size_t)k * H * H;
+  const float* Xb = X + (size_t)batch * sX;
+  for (int i = tid; i < H * 8; i += 256)
+    *reinterpret_cast<float4*>(&Xs[i >> 3][(i & 7) * 4]) = *reinterpret_cast<const float4*>(Xb + (size_t)(i >> 3) * N + n0 + (i & 7) * 4);
+  const int ty = tid >> 3, tx = tid & 7;                             // rows 8 ty .. 8 ty + 7, columns n0 + 4 tx .. + 3
+  float acc[8][4];
+#pragma unroll
+  for (int i = 0; i < 8; ++i)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) acc[i][e] = 0.f;
+  for (int l0 = 0; l0 < H; l0 += 16) {
+    __syncthreads();
+    if (AT) {
+      for (int i = tid; i < 4 * H; i += 256)
+        *reinterpret_cast<float4*>(&As[i / (H / 4)][(i % (H / 4)) * 4]) = __ldg(reinterpret_cast<const float4*>(A + (size_t)(l0 + i / (H / 4)) * H) + i % (H / 4));
+    } else {
+      for (int i = tid; i < 4 * H; i += 256) {
+        const int m = i >> 2, q = i & 3;
+        const float4 v = __ldg(reinterpret_cast<const float4*>(A + (size_t)m * H + l0) + q);
+        As[q * 4][m] = v.x; As[q * 4 + 1][m] = v.y; As[q * 4 + 2][m] = v.z; As[q * 4 + 3][m] = v.w;
+      }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int kk = 0; kk < 16; ++kk) {
+      const float4 a0 = *reinterpret_cast<const float4*>(&As[kk][ty * 8]), a1 = *reinterpret_cast<const float4*>(&As[kk][ty * 8 + 4]);
+      const float4 bv = *reinterpret_cast<const float4*>(&Xs[l0 + kk][tx * 4]);
+      const float a[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w}, bb[4] = {bv.x, bv.y, bv.z, bv.w};
+#pragma unroll
+      for (int i = 0; i < 8; ++i)
+#pragma unroll
+        for (int e = 0; e < 4; ++e) acc[i][e] = fmaf(a[i], bb[e], acc[i][e]);
+    }
+  }
+  __syncthreads();                                                   // the whole block of X is read (in place)
+  float y[4] = {0.f, 0.f, 0.f, 0.f};
+  if (yv) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) y[e] = yv[(size_t)batch * sY + n0 + tx * 4 + e];
+  }
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int m = ty * 8 + i;
+    const float r = rs ? rs[(size_t)k * H + m] : 1.f, xm = xv ? xv[(size_t)k * H + m] : 0.f;
+    *reinterpret_cast<float4*>(out + (size_t)batch * sOut + (size_t)m * N + n0 + tx * 4) =
+        make_float4(fmaf(r, acc[i][0], xm * y[0]), fmaf(r, acc[i][1], xm * y[1]), fmaf(r, acc[i][2], xm * y[2]), fmaf(r, acc[i][3], xm * y[3]));
+  }
+}
+
+// Per (sample, net), before pass 1: c2 = 2 W2^T wo, and the sums the weight-gradient kernels accumulate over chunks start at 0
+__global__ void __launch_bounds__(H) c2_kernel(int Kn, const float* __restrict__ W2, const float* __restrict__ wo2, uint8_t* scr, size_t stride) {
+  const int bk = blockIdx.x, k = bk % Kn, i = threadIdx.x;
+  const float* w2 = W2 + (size_t)bk * H * H;
+  float s = 0.f;
+  for (int j = 0; j < H; ++j) s = fmaf(__ldg(wo2 + (size_t)k * H + j), __ldg(w2 + (size_t)j * H + i), s);
+  float* t = scratch(scr, stride, bk);
+  t[SCR_C2 + i] = s;
+  t[SCR_SZH + i] = 0.f;
+  if (i < C) t[SCR_SZD + i] = 0.f;
+  if (i == 0) t[SCR_SDO] = 0.f;
+}
+
+// Per (sample, net), after the last chunk: db2 = Wa^T (u sm3) + 2wo sum_p dov (G.b2 holds u sm3), de = db2, dbd = sum_b db2
+__global__ void __launch_bounds__(H) unfold_b2_kernel(int Kn, const float* __restrict__ Wa, const float* __restrict__ wo2, uint8_t* scr,
+                                                      size_t stride, float* gb2, float* ge, float* gbd) {
+  __shared__ float v[H];
+  const int bk = blockIdx.x, k = bk % Kn, j = threadIdx.x;
+  v[j] = gb2[(size_t)bk * H + j];
+  __syncthreads();
+  const float* wa = Wa + (size_t)k * H * H;
+  float s = __ldg(wo2 + (size_t)k * H + j) * scratch(scr, stride, bk)[SCR_SDO];
+  for (int l = 0; l < H; ++l) s = fmaf(__ldg(wa + (size_t)l * H + j), v[l], s);
+  gb2[(size_t)bk * H + j] = s;
+  ge[(size_t)bk * H + j] = s;
+  atomicAdd(gbd + (size_t)k * H + j, s);
+}
+
 // fp32 weight matrix [R_src x K_src] -> bf16 image in layout (*) ; transpose = image rows are source columns.
 // The image is a sequence of K = 16 chunks (two k-cores, rows*32 bytes per plane); with PL planes a chunk is
 // [hi plane | lo plane], so the producer still fetches one contiguous block per chunk.
 template <int PL, bool F16>
 __global__ void image_kernel(const float* __restrict__ src, size_t src_stride, uint8_t* __restrict__ dst,
-                             size_t dst_stride, int rows, int kd, int transpose, const NetScales* __restrict__ tab, int which,
-                             const float* __restrict__ kscale) {        // kscale [batch][kd]: image of S diag(kscale) (or nullptr)
+                             size_t dst_stride, int rows, int kd, int transpose, const NetScales* __restrict__ tab, int which) {
   const float* S = src + blockIdx.y * src_stride;
   uint8_t* D = dst + blockIdx.y * dst_stride;
   const int q = blockIdx.x * blockDim.x + threadIdx.x;             // 16-byte piece index
@@ -1584,13 +1699,9 @@ __global__ void image_kernel(const float* __restrict__ src, size_t src_stride, u
   float v[8];
 #pragma unroll
   for (int e = 0; e < 8; ++e) v[e] = transpose ? S[(size_t)(kc * 8 + e) * rows + r] : S[(size_t)r * kd + kc * 8 + e];
-  if (kscale) {
-#pragma unroll
-    for (int e = 0; e < 8; ++e) v[e] *= kscale[(size_t)blockIdx.y * kd + kc * 8 + e];
-  }
   if (F16) {                                                         // entry blockIdx.y: (sample, net) for generated weights, (0, net) for static ones
     const NetScales& t = tab[blockIdx.y];
-    const float sc = which == 0 ? t.sW1 : (which == 1 ? t.sW2 : (which == 2 ? t.sWd : (which == 3 ? t.sWa : t.sWaU)));
+    const float sc = which == 0 ? t.sW1 : (which == 1 ? t.sW2 : (which == 2 ? t.sWd : (which == 3 ? t.sWa : t.sP)));
 #pragma unroll
     for (int e = 0; e < 8; ++e) v[e] *= sc;
   }
@@ -1700,6 +1811,7 @@ struct Carve {
   long long* dbg;
   NetScales* sc;
   int* seedmax;
+  size_t scr_stride;            // bytes between the scratch() of consecutive (sample, net): Tc workspace tiles
   size_t bytes;
 };
 
@@ -1734,7 +1846,8 @@ static Carve carve(uint8_t* base, int chunk, int Kn, int B, int pl, bool values_
     c.bytes = off;
     return c;
   }
-  c.blobs = take((size_t)B * Kn * T * (pl == 2 ? Geo<2>::NET_TILE : Geo<1>::NET_TILE));
+  c.scr_stride = T * (pl == 2 ? Geo<2>::NET_TILE : Geo<1>::NET_TILE);
+  c.blobs = take((size_t)B * Kn * c.scr_stride);
   c.od = reinterpret_cast<float*>(take(rows * Kn * 12));
   c.dov = reinterpret_cast<float*>(take(rows * Kn * 4));
   c.dod = reinterpret_cast<float*>(take(rows * Kn * 12));
@@ -1755,25 +1868,23 @@ int default_chunk(int B, int planes) {
 size_t workspace_bytes(int chunk, int Kn, int B, int planes) { return carve(nullptr, chunk, Kn, B, planes).bytes; }
 size_t lattice_workspace_bytes(int chunk, int Kn, int B, int planes) { return carve(nullptr, chunk, Kn, B, planes, true).bytes; }
 
+// Pm: the fp32 P of every (sample, net) (sweep >= 1), or nullptr
 template <int PL, bool F16>
-static int make_images(const DpnWeights& Wt, const Carve& c, int B, int Kn, cudaStream_t st) {
-  struct Spec { const float* src; size_t sstride; size_t doff; size_t dstride; int rows, kd, tr, batches; uint8_t* dst; int which; const float* kscale; };
-  // the transposed Wa image carries u (G4: y = m3 (diag(u) Wa) + 2wo with the bare mask as A operand)
-  const float* ku = c.uvec;
+static int make_images(const DpnWeights& Wt, const Carve& c, const float* Pm, int B, int Kn, cudaStream_t st) {
+  struct Spec { const float* src; size_t sstride; size_t doff; size_t dstride; int rows, kd, tr, batches; uint8_t* dst; int which; };
   const Spec specs[] = {
-      {Wt.W1, (size_t)H * C, 0, GEN_IMG, H, C, 0, B * Kn, c.img_gen, 0, nullptr},              // W1  : rows = out, k = in
-      {Wt.W1, (size_t)H * C, IMG_HC, GEN_IMG, C, H, 1, B * Kn, c.img_gen, 0, nullptr},         // W1T : rows = in,  k = out
-      {Wt.W2, (size_t)H * H, 2 * IMG_HC, GEN_IMG, H, H, 0, B * Kn, c.img_gen, 1, nullptr},
-      {Wt.W2, (size_t)H * H, 2 * IMG_HC + IMG_HH, GEN_IMG, H, H, 1, B * Kn, c.img_gen, 1, nullptr},
-      {Wt.Wd, (size_t)H * C, 0, STA_IMG, H, C, 0, Kn, c.img_sta, 2, nullptr},
-      {Wt.Wa, (size_t)H * H, IMG_HC, STA_IMG, H, H, 0, Kn, c.img_sta, 3, nullptr},
-      {Wt.Wa, (size_t)H * H, IMG_HC + IMG_HH, STA_IMG, H, H, 1, Kn, c.img_sta, ku ? 5 : 3, ku},
+      {Wt.W1, (size_t)H * C, 0, GEN_IMG, H, C, 0, B * Kn, c.img_gen, 0},              // W1  : rows = out, k = in
+      {Wt.W1, (size_t)H * C, IMG_HC, GEN_IMG, C, H, 1, B * Kn, c.img_gen, 0},         // W1T : rows = in,  k = out
+      {Wt.W2, (size_t)H * H, 2 * IMG_HC, GEN_IMG, H, H, 0, B * Kn, c.img_gen, 1},
+      {Pm, c.scr_stride / 4, 2 * IMG_HC + IMG_HH, GEN_IMG, H, H, 1, Pm ? B * Kn : 0, c.img_gen, 4},   // P^T (G4 of the reverse sweep)
+      {Wt.Wd, (size_t)H * C, 0, STA_IMG, H, C, 0, Kn, c.img_sta, 2},
+      {Wt.Wa, (size_t)H * H, IMG_HC, STA_IMG, H, H, 0, Kn, c.img_sta, 3},
   };
   for (const Spec& s : specs) {
     if (s.batches == 0) continue;
     const int pieces = s.rows * s.kd / 8;
     image_kernel<PL, F16><<<dim3((pieces + 255) / 256, s.batches), 256, 0, st>>>(s.src, s.sstride, s.dst + s.doff * PL, s.dstride * PL,
-                                                                                 s.rows, s.kd, s.tr, c.sc, s.which, s.kscale);
+                                                                                 s.rows, s.kd, s.tr, c.sc, s.which);
     DPN_LAUNCH_OK();
   }
   return 0;
@@ -1811,13 +1922,23 @@ static int run_planes(const Job& J, cudaStream_t st) {
   constexpr bool phase_debug = false;
 #endif
   if ((rc = f32::launch_prep(B, Kn, Wt, c.uvec, c.wo2, c.cst, c.bsum, st))) return rc;
+  // the reverse sweep's fold: P = diag(u) Wa W2 (fp32, in workspace tiles pass 1 has not written yet) and c2 = 2 W2^T wo
+  float* Pm = sweep ? reinterpret_cast<float*>(c.blobs + off_h<PL>(B_QM)) : nullptr;
+  if (sweep) {
+    c2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.W2, c.wo2, c.blobs, c.scr_stride);
+    DPN_LAUNCH_OK();
+    fold_gemm_kernel<false><<<dim3(H / 32, B * Kn), 256, 0, st>>>(Kn, H, Wt.Wa, Wt.W2, (size_t)H * H, Pm, c.scr_stride / 4, c.uvec, nullptr,
+                                                                  nullptr, 0);
+    DPN_LAUNCH_OK();
+  }
   if (F16) {                                                          // scaling plan before anything is converted to fp16
-    bounds_kernel<<<B * Kn, 1024, 0, st>>>(Kn, Wt.W1, Wt.b1, Wt.W2, Wt.Wd, Wt.Wa, Wt.ba, c.bsum, c.uvec, c.wo2, c.sc);
+    bounds_kernel<<<B * Kn, 1024, 0, st>>>(Kn, Wt.W1, Wt.b1, Wt.W2, Wt.Wd, Wt.Wa, Wt.ba, c.bsum, c.uvec, c.wo2,
+                                           reinterpret_cast<const uint8_t*>(Pm), c.scr_stride, c.sc);
     DPN_LAUNCH_OK();
     plan_kernel<<<1, 32, 0, st>>>(B, Kn, c.sc);
     DPN_LAUNCH_OK();
   }
-  if ((rc = make_images<PL, F16>(Wt, c, B, Kn, st))) return rc;
+  if ((rc = make_images<PL, F16>(Wt, c, Pm, B, Kn, st))) return rc;
   if (pde) DPN_CUDA_OK(cudaMemsetAsync(J.out->loss_terms, 0, sizeof(double) * 6 * B, st));
   if (pde && J.margin) DPN_CUDA_OK(cudaMemsetAsync(J.margin->loss, 0, sizeof(double) * B, st));
   if (want_bwd) {
@@ -1859,6 +1980,7 @@ static int run_planes(const Job& J, cudaStream_t st) {
     w.o = c.o; w.od = c.od; w.dov = c.dov; w.dod = c.dod;
     w.vc = c.vc; w.vg = c.vg; w.sdo = c.sdo;
     w.sc = c.sc;
+    w.scr = c.blobs; w.scr_stride = c.scr_stride;
     w.xfirst = J.shape.mode == DPN_MODE_F16X3A ? 1 : 0;
     w.phase_dbg = phase_debug ? c.dbg : nullptr;
 #ifdef DPN_DEBUG_BUILD
@@ -1915,6 +2037,7 @@ static int run_planes(const Job& J, cudaStream_t st) {
     WgradWork ww;
     ww.B = B; ww.Kn = Kn; ww.T = T; ww.blobs = c.blobs; ww.sc = c.sc; ww.uvec = c.uvec;
     ww.Wa = Wt.Wa; ww.ba = Wt.ba; ww.vg = c.vg;
+    ww.scr = c.blobs; ww.scr_stride = c.scr_stride;
     ww.gW1 = G.W1; ww.gW2 = G.W2; ww.gWa = G.Wa; ww.gWd = G.Wd;
     ww.gb1 = G.b1; ww.gb2 = G.b2; ww.ge = G.e; ww.gbd = G.bd; ww.gba = G.ba;
     const int items = B * Kn * 2 * wg2::ITEMS;                            // x 2 output halves
@@ -1952,7 +2075,18 @@ static int run_planes(const Job& J, cudaStream_t st) {
   }
 #endif
   if (want_bwd) {
-    if ((rc = f32::launch_finalize(Kn, Wt, c.vc, c.vg, c.sdo, *J.grads, st))) return rc;
+    // dW2 = Wa^T (diag(u) m3^T zh) + 2wo (x) sum_p zh, dWd likewise with zd, db2 = de, dbd (linear: once, after the last chunk)
+    const DpnGrads& G = *J.grads;
+    const float* s0 = scratch(c.blobs, c.scr_stride, 0);
+    fold_gemm_kernel<true><<<dim3(H / 32, B * Kn), 256, 0, st>>>(Kn, H, Wt.Wa, G.W2, (size_t)H * H, G.W2, (size_t)H * H, nullptr, c.wo2,
+                                                                 s0 + SCR_SZH, c.scr_stride / 4);
+    DPN_LAUNCH_OK();
+    fold_gemm_kernel<true><<<dim3(C / 32, Kn), 256, 0, st>>>(Kn, C, Wt.Wa, G.Wd, (size_t)H * C, G.Wd, (size_t)H * C, nullptr, c.wo2,
+                                                             s0 + SCR_SZD, c.scr_stride / 4);
+    DPN_LAUNCH_OK();
+    unfold_b2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.Wa, c.wo2, c.blobs, c.scr_stride, G.b2, G.e, G.bd);
+    DPN_LAUNCH_OK();
+    if ((rc = f32::launch_finalize(Kn, Wt, c.vc, c.vg, c.sdo, G, st))) return rc;
   }
   return 0;
 }
