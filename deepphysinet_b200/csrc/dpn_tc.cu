@@ -19,12 +19,12 @@
 //                                         never formed: P = diag(u) Wa W2, c2 = 2 W2^T wo per (sample, net), the bare mask is the A operand
 //           G6 jin = qm W1             do/dPE  -> do/dz_c = jin . dPE_c   (the 3 Jacobian columns)
 //   residual kernel (fp64, shared with the fp32 mode) -> loss terms + seeds dL/do, dL/d(do/dz_c)
-//   pass 2  the Z-side rows  zp = dov PE + sum_c seed_c dPE_c, zd = dov PE6, zh = dov h1 + ht, zc = dov c + ct  as the FORWARD pass of the
-//           combined row zp with frozen masks and dov-scaled biases (G7', G8'); gz = dov g + gt is never formed - its column sum
-//           comes out of the dWa contraction
-//   wgrad   dW1 = qm^T zp, diag(u) m3^T [zh | zd | zc] : K = points contractions, MN-major operands;  dW2 = y^T zh and dWd = y^T zd
-//           follow after the last chunk as Wa^T (diag(u) m3^T z) + 2wo (x) sum_p z  (unfold_kernel)
-//   colsum  bias gradients and the two vectors the folded output layer needs (vc, vg)
+//   pass 2  the Z-side rows  zp = dov PE + sum_c seed_c dPE_c, zd = dov PE6, zh = dov h1 + ht  as the FORWARD pass of the combined row zp
+//           with frozen masks and dov-scaled biases (G7'); zc = dov c + ct and gz = dov g + gt are never formed
+//   wgrad   dW1 = qm^T zp, m3^T [zh | zd] : K = points contractions, MN-major operands;  after the last chunk, dW2 = y^T zh and
+//           dWd = y^T zd follow as Wa^T diag(u) (m3^T z) + 2wo (x) sum_p z (fold_gemm_kernel), and S = m3^T zc (-> dWa, dba) and the
+//           two vectors the folded output layer needs (vc = sum_p zc, vg = sum_p gz) from S = sum_b (m3^T zh) W2^T + ... (fold_s_kernel)
+//   colsum  bias gradients
 //
 // Every [128 x Kd] 16-bit operand tile ("blob") is stored in the layout (*) of dpn_umma.cuh in shared memory (and, 32 points at a
 // time, in the workspace), so a tile written once by an epilogue is (a) the K-major A operand of the next GEMM and
@@ -60,8 +60,8 @@ constexpr int IMG_HC = H * C * 2;             // 98304
 constexpr int IMG_HH = H * H * 2;             // 131072
 constexpr int GEN_IMG = 2 * IMG_HC + 2 * IMG_HH;   // per (sample, net): W1, W1T, W2, P^T (P = diag(u) Wa W2)
 constexpr int STA_IMG = IMG_HC + 2 * IMG_HH;       // per net: Wd, Wa, one unused [256 x 256] slot (the workspace sizes are pinned)
-// Workspace tile of one (net, point tile):  YT QM ZH ZC | ZP ZD | AUX | MASK.  No kernel writes the YT slot: the first tile of a
-// (sample, net) keeps scratch() there (the workspace sizes are pinned).  Pass 2 runs as the forward pass of the combined row
+// Workspace tile of one (net, point tile):  YT QM ZH ZC | ZP ZD | AUX | MASK.  No kernel writes the YT or the ZC slot (y and zc are never
+// formed); the first tile of a (sample, net) keeps scratch() in YT (the workspace sizes are pinned).  Pass 2 runs as the forward pass of the combined row
 // (DESIGN.md section 3) and needs only the ReLU mask m1 of pass 1 (256 bits per point) instead of the h1 / c / g tiles (3 x 1 KB per
 // point), and the weight-gradient kernel builds its J operand [a3 > 0] from the m3 mask bits instead of reading a stored tile.
 constexpr int NBLOB_H = 4, NBLOB_C = 2;
@@ -114,7 +114,7 @@ struct Work {
   float* pet;              // [B*T][C][TP] fp32 transposed coordinate features
   uint8_t* blobs;          // [B][Kn][T][NET_TILE_BYTES]
   float *o, *od, *dov, *dod;   // [B*T*TP][Kn], [..][Kn][3]
-  float *vc, *vg, *sdo;        // [Kn][H] column sums of zc / of the never-formed gz, and [Kn] sum of dov
+  float* sdo;                  // [Kn] sum of dov
   const NetScales* sc;         // [B][Kn] scaling plan (fp16 variant only)
   uint8_t* scr;                // per-(sample, net) scratch of the reverse sweep: scr + (b Kn + k) scr_stride (see scratch())
   size_t scr_stride;
@@ -141,7 +141,7 @@ template <int PL> __device__ __forceinline__ uint8_t* blob_mask(uint8_t* nt) { r
 // Per-(sample, net) scratch of the reverse sweep (fp32), in the YT slot of workspace tile index (b Kn + k) Tc, Tc = the tiles per
 // sample of a full chunk: no kernel writes a YT slot (DESIGN.md section 4), and the address is the same for every chunk of a call.
 //   c2 = 2 W2^T wo (pass 1, epilogue 4) | sum_p zh | sum_p dov | (b = 0 only) sum_{b,p} zd  - the last three accumulate over chunks
-// and are turned into dW2, db2 and dWd by unfold_kernel after the last chunk.  P = diag(u) Wa W2 (fp32, [H][H]) is formed in the
+// and enter vc (fold_s_kernel) and dW2, db2, dWd (fold_gemm_kernel, unfold_b2_kernel) after the last chunk.  P = diag(u) Wa W2 (fp32, [H][H]) is formed in the
 // QM .. ZC slots of the same tile before pass 1 of the first chunk writes them.
 enum { SCR_C2 = 0, SCR_SZH = H, SCR_SDO = 2 * H, SCR_SZD = 2 * H + 32 };   // float offsets
 __host__ __device__ __forceinline__ float* scratch(uint8_t* scr, size_t stride, int bk) { return reinterpret_cast<float*>(scr + (size_t)bk * stride); }
@@ -233,7 +233,7 @@ struct NetScales {                       // one per (sample, net)
   float M1, Mc, l1W1, l1W12;             // bounds of |h1|, |c|; L1(W1), L1(W1) L1(W2)
   float rowB;                            // max(1, L1(W1), L1(W1) L1(W2)): growth of the pass-2 tangent row over its chain
   float cap;                             // largest sH1 * sW2 this (sample, net) can carry (plan_kernel takes the min over samples)
-  float sZP, sZH, sZC, sZD, sDV;         // Z-side tiles and the seed tile of the CURRENT chunk (zscale_kernel)
+  float sZP, sZH, sZC, sZD, sDV;         // Z-side tiles and the seed tile of the CURRENT chunk (zscale_kernel; no kernel reads sZC)
 };
 constexpr float S_PE = 1024.f;           // coordinate / data features lie in [-1, 1]
 constexpr float F16_TOP = 32768.f;       // bound -> 2^15 (fp16 max is 65504)
@@ -865,7 +865,7 @@ __device__ __forceinline__ void unpack_planes(const uint4 (&q)[PL], float* v) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// Pass 2 of the split modes as the FORWARD PASS OF THE COMBINED ROW (DESIGN.md section 3).
+// Pass 2 of the split modes as the FORWARD PASS OF THE COMBINED ROW (DESIGN.md section 3), one GEMM per net.
 // The Z-side operands of the weight gradients are  zh = dov h1 + ht,  zc = dov c + ct,  gz = dov g + gt  with the tangent chain
 // ht = (xt W1^T) m1, ct = ht W2^T, gt = (ct Wa^T) m3.  Because h1 = m1 (PE W1^T + b1), c = h1 W2^T + PE6 Wd^T + bsum and
 // g = m3 (c Wa^T + ba) are (masked) affine in their inputs, the sums collapse:
@@ -873,28 +873,23 @@ __device__ __forceinline__ void unpack_planes(const uint4 (&q)[PL], float* v) {
 //        zc = zh W2^T + zd Wd^T + dov bsum       zd = dov PE6       (the operand of dWd)
 //        gz = m3 ( zc Wa^T + dov ba )
 // i.e. pass 2 is pass 1's value chain applied to the row zp with the FROZEN masks and dov-scaled biases.  It needs from pass 1
-// one bit mask per point (32 bytes) instead of the h1 / c / g tiles (3 KB), no separate tangent row, and every tile it produces
-// is at once the next A operand and the stored wgrad operand (one split instead of two).
-// gz itself is never formed: it enters the gradients only through its column sum vg = sum_p gz (dWb, dwo), and
-//        vg[j] = sum_i Wa[j,i] S[j,i] + ba[j] sum_p m3[p,j] dov[p],     S = m3^T zc
-// where S is the contraction the weight-gradient kernel runs anyway for dWa = diag(u) S (wgrad2_kernel, layer 2) - so the third
-// GEMM of the chain (zc Wa^T, K = 256) and its epilogue are not executed at all.
-// Structure = pass1_ts_kernel: two 256-column TMEM regions as ping-pong accumulators, converted in place into the next A operand,
-// the next GEMM starting block by block under the running epilogue.  Per net: the prologue writes zp into R1 (hi planes columns
-// [0,96), lo [96,192)) while G7' (-> R0) consumes it; epilogue 7 converts R0 into zh while G8' (-> R1, first the K = 192 part whose
-// A operand zd is staged in shared memory, 96 KB, layout (*)) consumes it; epilogue 8 reads R1 (zc -> workspace, column sums) and
-// the next net's prologue follows in the same threads.  7 x 16 KB weight ring.
+// one bit mask per point (32 bytes) instead of the h1 / c / g tiles (3 KB) and no separate tangent row.
+// Only zh is formed.  zc and gz enter the gradients through S = m3^T zc (dWa = diag(u) S, dba) and the column sums vc = sum_p zc,
+// vg[j] = sum_i Wa[j,i] S[j,i] + ba[j] sum_p m3[p,j] dov[p], and zc is linear in zh, zd and dov:  S = (m3^T zh) W2^T + (m3^T zd) Wd^T
+// + sm3 (x) bsum.  So fold_s_kernel forms S and vc after the last chunk from m3^T zh, m3^T zd, sm3 and the column sums, which the
+// weight-gradient kernel accumulates for dW2 / dWd anyway, and neither zh W2^T + zd Wd^T nor zc Wa^T is executed here.
+// Pipeline = pass1_ts_kernel's (namespace pp).  Per net: the prologue writes zp into TMEM region R1 (hi planes columns [0,96), lo
+// [96,192)) block by block while G7' (-> R0) consumes it; epilogue 7 reads R0 (zh -> workspace), and the next net's prologue follows
+// in the same threads.  7 x 16 KB weight ring.
 // ------------------------------------------------------------------------------------------------
 namespace p2z {
-enum { V2_B1 = 0, V2_BSUM, NV2 };
 constexpr int NS_MAX = 14;
 template <int PL>
 struct Cfg {
   static constexpr int NS = PL == 2 ? 7 : 14;
   static constexpr int W_BYTES = PL * STAGE_BYTES;       // one K = 16 chunk of a [256 x K] image: 8 KB per plane, hi | lo
   static constexpr int STAGE = W_BYTES;
-  static constexpr int ZD_BYTES = PL * BLOB_C;           // zd staging: one [128 x 192] tile per plane, layout (*)
-  static constexpr int SMEM = NS * STAGE + ZD_BYTES + NV2 * H * 4 + H * 4 + 16;        // + column sums of zc + sum of dov
+  static constexpr int SMEM = NS * STAGE + H * 4 + 16;   // + b1 + sum of dov
 };
 constexpr uint32_t ZP_LO = 96;                 // zp planes inside TMEM region R1: hi [0,96) | lo [96,192)
 struct PipeZ {
@@ -906,7 +901,7 @@ struct PipeZ {
 // K-chunks of zp (K = 192) complete after prologue iteration i of both halves: a half writes 24 columns = 1.5 chunks per iteration
 __host__ __device__ constexpr int zp_first(int i) { return i == 0 ? 0 : i == 1 ? 1 : i == 2 ? 3 : 4; }
 __host__ __device__ constexpr int zp_count(int i) { return (i & 1) ? 2 : 1; }
-static_assert(Cfg<2>::SMEM + (int)sizeof(PipeZ) + 1024 <= 227 * 1024 && Cfg<1>::SMEM <= Cfg<2>::SMEM, "pass2z_kernel: ring + zd tile + vectors must fit one SM's 227 KB");
+static_assert(Cfg<2>::SMEM + (int)sizeof(PipeZ) + 1024 <= 227 * 1024 && Cfg<1>::SMEM <= Cfg<2>::SMEM, "pass2z_kernel: ring + vectors must fit one SM's 227 KB");
 }  // namespace p2z
 
 template <int PL, bool F16>
@@ -915,9 +910,8 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ p2z::PipeZ pipe;
   uint8_t* ring = smem;
-  uint8_t* zdt = smem + PZ::NS * PZ::STAGE;
-  float* svec = reinterpret_cast<float*>(zdt + PZ::ZD_BYTES);
-  float* csum = svec + p2z::NV2 * H;                               // [H] + sdo
+  float* sb1 = reinterpret_cast<float*>(smem + PZ::NS * PZ::STAGE);   // [H] b1
+  float* ssdo = sb1 + H;                                              // sum of dov over this tile
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int b = blockIdx.x / w.T, tl = blockIdx.x % w.T;
@@ -929,22 +923,16 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
     // ---------------- producer: weight chunks (multicast slices) ----------------
     pp::Ring<PL, PZ> wr{ring, pipe.full, pipe.empty, cta.rank, l2_policy_evict_last()};
     for (int k = 0; k < w.Kn; ++k) {
-      const uint8_t* gen = w.img_gen + ((size_t)b * w.Kn + k) * Geo<PL>::GEN;
-      const uint8_t* sta = w.img_sta + (size_t)k * Geo<PL>::STA;
-      const uint8_t *iW1 = gen, *iW2 = gen + PL * 2 * IMG_HC, *iWd = sta;
-      // the MMA warp's order: G7' in prologue-block order | zd Wd^T (no dependence on an epilogue) | G8' in block order
+      const uint8_t* gen = w.img_gen + ((size_t)b * w.Kn + k) * Geo<PL>::GEN;     // the W1 image
+      // the MMA warp's order: G7' in prologue-block order
       for (int i = 0; i < 4; ++i)
         for (int h = 0; h < 2; ++h)
-          for (int j = 0; j < p2z::zp_count(i); ++j) wr.put(iW1 + (size_t)(6 * h + p2z::zp_first(i) + j) * PZ::W_BYTES, PZ::W_BYTES, nullptr);
-      for (int c = 0; c < 12; ++c) wr.put(iWd + (size_t)c * PZ::W_BYTES, PZ::W_BYTES, nullptr);
-      for (int i = 0; i < 16; ++i) wr.put(iW2 + (size_t)pp::block_order(i) * PZ::W_BYTES, PZ::W_BYTES, nullptr);
+          for (int j = 0; j < p2z::zp_count(i); ++j) wr.put(gen + (size_t)(6 * h + p2z::zp_first(i) + j) * PZ::W_BYTES, PZ::W_BYTES, nullptr);
     }
   } else if (warp == Geo<PL>::W_MMA) {
     // ---------------- MMA issuer ----------------
     pp::Mma<PL, F16, PZ> mma{{ring, pipe.full, pipe.empty}, pipe.blk, pipe.acc_ready, smem_u32(ring), w.phase_dbg != nullptr, false};
     const long long t_begin = clock64();
-    const uint64_t zd_base = smem_desc(smem_u32(zdt), CORE_STRIDE, 128);
-    constexpr uint32_t zd_lo = BLOB_C >> 4, zd_step = (2 * CORE_STRIDE) >> 4;
     const uint32_t R0 = tmem, R1 = tmem + pp::REGION;
     for (int k = 0; k < w.Kn; ++k) {
       for (int i = 0; i < 4; ++i) {                                        // G7' = zp W1^T -> R0, under the prologue
@@ -957,8 +945,6 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       }
       mma.bp ^= 1u;
       mma.ready(0);
-      for (int c = 0; c < 12; ++c) mma.ss(R1, H, zd_base + (uint32_t)c * zd_step, zd_lo, false, c > 0 ? 1u : 0u);   // G8' = zd Wd^T (zd: shared memory, complete with the prologue)
-      mma.gemm_ts(R1, R0, H, true); mma.ready(1);                          //       + zh W2^T, under epilogue 7
     }
     if (mma.timed && lane == 0) {
       atomicAdd((unsigned long long*)w.phase_dbg + 8, (unsigned long long)(clock64() - t_begin));
@@ -978,15 +964,11 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
     long long t_pro = 0;
     const long long t_begin = clock64();
     const bool timed = epi.timed;
-    for (int i = tid; i < H + 4; i += Geo<PL>::ET) csum[i] = 0.f;
+    if (tid == 0) *ssdo = 0.f;
     for (int k = 0; k < w.Kn; ++k) {
       uint8_t* nt = net_tile<PL>(w, b, k, tl);
-      epi_bar<PL>();                                                   // previous net's vectors / column sums are flushed
-      if (tid < H) {
-        const size_t vb = ((size_t)b * w.Kn + k) * H;
-        svec[p2z::V2_B1 * H + tid] = __ldg(w.b1 + vb + tid);
-        svec[p2z::V2_BSUM * H + tid] = __ldg(w.bsum + vb + tid);
-      }
+      epi_bar<PL>();                                                   // previous net's b1 / sum of dov are flushed
+      if (tid < H) sb1[tid] = __ldg(w.b1 + ((size_t)b * w.Kn + k) * H + tid);
       epi_bar<PL>();
       const float dv = w.dov[row * w.Kn + k];
       float dd[3];
@@ -994,19 +976,16 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       for (int c = 0; c < 3; ++c) dd[c] = w.dod[(row * w.Kn + k) * 3 + c];          // zero for the values-only backward
       const uint4 m1q = __ldg(reinterpret_cast<const uint4*>(blob_mask<PL>(nt)) + r * 2 + half);
       const uint32_t m1w[4] = {m1q.x, m1q.y, m1q.z, m1q.w};
-      // fp16 variant: every tile carries one power-of-two scale per (sample, net) (zscale_kernel); accumulators carry
-      // (A tile scale) x (weight image scale) and i7 / i8 undo that
-      // zd exists twice: the stored tile (wgrad operand of dWd) with its own scale sZD, and the A operand of G8' whose scale is tied
-      // to the accumulator it shares with zh W2^T: sZH sW2 = sZDa sWd, and plan_kernel made sH1 sW2 = S_PE sWd  =>  sZDa = sZH S_PE / sH1
-      float sZP = 1.f, sZH = 1.f, sZC = 1.f, sZD = 1.f, sZDa = 1.f, sDV = 1.f, i7 = 1.f, i8 = 1.f;
+      // fp16 variant: every tile carries one power-of-two scale per (sample, net) (zscale_kernel); the accumulator of G7' carries
+      // (A tile scale) x (weight image scale) and i7 undoes that
+      float sZP = 1.f, sZH = 1.f, sZD = 1.f, sDV = 1.f, i7 = 1.f;
       if (F16) {
         const NetScales t = w.sc[b * w.Kn + k];
-        sZP = t.sZP; sZH = t.sZH; sZC = t.sZC; sZD = t.sZD; sDV = t.sDV;
-        sZDa = t.sZH * (S_PE / t.sH1);
-        i7 = (1.f / t.sZP) * (1.f / t.sW1); i8 = (1.f / t.sZH) * (1.f / t.sW2);
+        sZP = t.sZP; sZH = t.sZH; sZD = t.sZD; sDV = t.sDV;
+        i7 = (1.f / t.sZP) * (1.f / t.sW1);
       }
-      // the scale of the tile an epilogue produces is folded into its FMA (powers of two: exact): zh sZH = m1 (acc k7 + (dov sZH) b1), ...
-      const float k7 = i7 * sZH, k8 = i8 * sZC, dvH = dv * sZH, dvC = dv * sZC, dvP = dv * sZP, inv_sZC = 1.f / sZC;
+      // the scale of the tile the epilogue produces is folded into its FMA (powers of two: exact): zh sZH = m1 (acc k7 + (dov sZH) b1)
+      const float k7 = i7 * sZH, dvH = dv * sZH, dvP = dv * sZP;
       const float ddP[3] = {dd[0] * sZP, dd[1] * sZP, dd[2] * sZP};
       // seed tile for the bias-gradient MMAs of the wgrad kernel: col 0/1/2 = dov split into three 16-bit terms, col 3 = an exact 1 on
       // valid points (the column sums of zh / zd), rest 0
@@ -1025,7 +1004,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         __stcs(reinterpret_cast<uint4*>(blob_aux<PL>(nt) + gp_off(2, r, 0)), pack8f<F16>(a8));
         __stcs(reinterpret_cast<uint4*>(blob_aux<PL>(nt) + gp_off(2, r, 1)), make_uint4(0u, 0u, 0u, 0u));
       }
-      // ---- prologue: zp = dov PE + sum_c dod_c dPE_c -> A operand (TMEM) + workspace;  zd = dov PE6 -> shared memory + workspace ----
+      // ---- prologue: zp = dov PE + sum_c dod_c dPE_c -> A operand (TMEM) + workspace;  zd = dov PE6 -> workspace ----
       const long long t_p0 = timed ? clock64() : 0ll;
       // the loads of column group it + 1 are in flight while group it is processed (they come from L2: the tile's features are
       // re-read for every net)
@@ -1069,24 +1048,21 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
           if (PL == 2) __stcs(reinterpret_cast<uint4*>(blob_zp<PL>(nt) + BLOB_C + goff), pq[PL - 1]);
           hi[qd * 4 + 0] = pq[0].x; hi[qd * 4 + 1] = pq[0].y; hi[qd * 4 + 2] = pq[0].z; hi[qd * 4 + 3] = pq[0].w;
           lo[qd * 4 + 0] = pq[PL - 1].x; lo[qd * 4 + 1] = pq[PL - 1].y; lo[qd * 4 + 2] = pq[PL - 1].z; lo[qd * 4 + 3] = pq[PL - 1].w;
-          float d6[8], da[8];
+          float d6[8];
           unpack_planes<PL, F16>(p6[qd], d6);
 #pragma unroll
-          for (int e = 0; e < 8; ++e) { da[e] = F16 ? d6[e] * (dv * (sZDa / S_PE)) : d6[e] * dv; d6[e] *= F16 ? dv * (sZD / S_PE) : dv; }
+          for (int e = 0; e < 8; ++e) d6[e] *= F16 ? dv * (sZD / S_PE) : dv;
           split8<PL, F16>(d6, pq);
           __stcs(reinterpret_cast<uint4*>(blob_zd<PL>(nt) + goff), pq[0]);
           if (PL == 2) __stcs(reinterpret_cast<uint4*>(blob_zd<PL>(nt) + BLOB_C + goff), pq[PL - 1]);
-          if (F16) split8<PL, F16>(da, pq);                           // (bf16 / bf16x3: no scales, the same planes serve both)
-          const uint32_t soff = piece_off(r, it * 3 + qd);
-          *reinterpret_cast<uint4*>(zdt + soff) = pq[0];
-          if (PL == 2) *reinterpret_cast<uint4*>(zdt + BLOB_C + soff) = pq[PL - 1];
         }
         tmem_st8(R1 + it * 12, hi); tmem_st4(R1 + it * 12 + 8, hi + 8);
         if (PL == 2) { tmem_st8(R1 + p2z::ZP_LO + it * 12, lo); tmem_st4(R1 + p2z::ZP_LO + it * 12 + 8, lo + 8); }
-        epi.blk_done(it - half * NB, true);               // (and its part of the zd tile is in shared memory)
+        epi.blk_done(it - half * NB);
       }
       if (timed) t_pro += clock64() - t_p0;
-      // ---- epilogue 7: zh = m1 (acc + dov b1) ----
+      // ---- epilogue 7: zh = m1 (acc + dov b1) -> workspace.  G7' has completed: it no longer reads R1, which the next net's prologue
+      // overwrites; the next G7' overwrites R0 only after that prologue's first block, i.e. after these reads ----
       epi.acc_wait(0);
 #pragma unroll 1
       for (int cb = 0; cb < NB; ++cb) {
@@ -1098,7 +1074,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         for (int i = 0; i < NB; ++i) bits = (cb == i) ? m1w[i] : bits;
 #pragma unroll
         for (int j4 = 0; j4 < 8; ++j4) {
-          const float4 bv = *reinterpret_cast<const float4*>(svec + p2z::V2_B1 * H + cg * 32 + j4 * 4);
+          const float4 bv = *reinterpret_cast<const float4*>(sb1 + cg * 32 + j4 * 4);
           const float bb[4] = {bv.x, bv.y, bv.z, bv.w};
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
@@ -1107,54 +1083,20 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
             v[j] = ((bits >> j) & 1u) ? z : 0.f;
           }
         }
-        epi.emit(cg, v, blob_h<PL>(nt, B_ZH), true, R0 + cg * 32);
-        epi.blk_done(cb, true);
+        epi.emit(cg, v, blob_h<PL>(nt, B_ZH), false, 0u);
       }
-      // ---- epilogue 8: zc = acc + dov (b2 + bd + e) -> workspace (Z operand of dWa);  column sum -> vc ----
-      epi.acc_wait(1);
-#pragma unroll 1
-      for (int cb = 0; cb < NB; ++cb) {
-        const int cg = c0 + cb;
-        float v[32], z[32];
-        tmem_ld32(R1 + cg * 32, v);
-#pragma unroll
-        for (int j4 = 0; j4 < 8; ++j4) {
-          const float4 bv = *reinterpret_cast<const float4*>(svec + p2z::V2_BSUM * H + cg * 32 + j4 * 4);
-          const float bb[4] = {bv.x, bv.y, bv.z, bv.w};
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const int j = j4 * 4 + e;
-            z[j] = v[j] = F16 ? fmaf(v[j], k8, dvC * bb[e]) : fmaf(dv, bb[e], v[j]);           // zc sZC
-          }
-        }
-#pragma unroll
-        for (int qd = 0; qd < 4; ++qd) {
-          uint4 pq[PL];
-          split8<PL, F16>(v + qd * 8, pq);
-          const uint32_t off = gp_off(32, r, cg * 4 + qd);
-          __stcs(reinterpret_cast<uint4*>(blob_h<PL>(nt, B_ZC) + off), pq[0]);
-          if (PL == 2) __stcs(reinterpret_cast<uint4*>(blob_h<PL>(nt, B_ZC) + BLOB_H + off), pq[PL - 1]);
-        }
-        const float cs = warp_colsum32(z, lane);
-        atomicAdd(csum + cg * 32 + lane, cs * inv_sZC);
-      }
-      tc_fence_before();                                                // my reads of R1 precede the prologue's tcgen05.st of the next net
-      // ---- flush this net's column sums ----
+      // ---- sum of dov over this tile ----
       if (half == 0) {
         float sd = dv;
 #pragma unroll
         for (int m = 16; m; m >>= 1) sd += __shfl_xor_sync(0xffffffffu, sd, m);
-        if (lane == 0) atomicAdd(csum + H, sd);
+        if (lane == 0) atomicAdd(ssdo, sd);
       }
       epi_bar<PL>();
-      for (int i = tid; i < H; i += Geo<PL>::ET) {
-        atomicAdd(w.vc + (size_t)k * H + i, csum[i]);
-        csum[i] = 0.f;
-      }
       if (tid == 0) {
-        atomicAdd(w.sdo + k, csum[H]);
-        atomicAdd(scratch(w.scr, w.scr_stride, b * w.Kn + k) + SCR_SDO, csum[H]);
-        csum[H] = 0.f;
+        atomicAdd(w.sdo + k, *ssdo);
+        atomicAdd(scratch(w.scr, w.scr_stride, b * w.Kn + k) + SCR_SDO, *ssdo);
+        *ssdo = 0.f;
       }
     }
     if (timed && tid == 0) {
@@ -1174,13 +1116,10 @@ struct WgradWork {
   int B, Kn, T, splits;
   const uint8_t* blobs;
   const NetScales* sc;
-  const float* uvec;       // [Kn][H] u = Wb^T wo
-  const float *Wa, *ba;    // [Kn][H][H], [Kn][H] fp32 (split modes: vg = sum_p gz from the dWa contraction, see wgrad2_kernel)
-  float* vg;               // [Kn][H]
   uint8_t* scr;            // per-(sample, net) scratch (see scratch()): sum_p zh, sum_p zd
   size_t scr_stride;
-  float *gW1, *gW2, *gWa, *gWd;
-  float *gb1, *gb2, *ge, *gbd, *gba;
+  float *gW1, *gW2, *gWd;
+  float *gb1, *gb2, *ge, *gbd;
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -1189,14 +1128,12 @@ struct WgradWork {
 // HBM-bound (it reads every operand tile pass 1 / pass 2 wrote), so the structure follows the bytes:
 //   * tiles are stored [point quarter][k-core][32 rows][16 B] (gp_off), so a 32-point quarter of every operand is contiguous; THREE
 //     stages of 73 KB: the bulk loads of quarter-tiles i+1, i+2 run under the MMAs of quarter-tile i;
-//   * three kinds of work item per (sample, net):  0: dW1 = qm^T zp (+ db1);  1 and 2 have J = [a3 > 0] as one exact 16-bit plane
-//     built from the mask bits of pass 1 (two MMAs per step and Z plane instead of three, no stored J tile):
-//     1: diag(u) m3^T zh AND diag(u) m3^T zd (+ u sm3) in ONE item with a 256 + 192 column accumulator, plus the column sums
-//     sum_p zh, sum_p zd (the Z half-tiles against the seed tile's column of ones) - y = m3 (diag(u) Wa) + 2wo is never stored, and
-//     unfold_kernel turns these into dW2 = y^T zh, dWd = y^T zd, db2 after the last chunk;
-//     2: S = m3^T zc.  Its epilogue derives three results from S and the seed product sm3 = sum_p m3 dov:
-//     dWa = diag(u) S,  dba = u sm3,  and the column sum of the never-formed tile gz = m3 (zc Wa^T + dov ba):
-//     vg[j] = sum_i Wa[j,i] S[j,i] + ba[j] sm3[j]  - which is why pass 2 has no third GEMM;
+//   * two kinds of work item per (sample, net):  0: dW1 = qm^T zp (+ db1);
+//     1: J = [a3 > 0] as one exact 16-bit plane built from the mask bits of pass 1 (two MMAs per step and Z plane instead of three,
+//     no stored J tile): m3^T zh AND m3^T zd (+ the seed product sm3 = sum_p m3 dov) in ONE item with a 256 + 192 column
+//     accumulator, plus the column sums sum_p zh, sum_p zd (the Z half-tiles against the seed tile's column of ones).  Neither
+//     y = m3 (diag(u) Wa) + 2wo nor zc = zh W2^T + zd Wd^T + dov bsum is ever formed: after the last chunk fold_s_kernel turns
+//     these sums into dWa, dba, vg and vc, and fold_gemm_kernel / unfold_b2_kernel into dW2 = y^T zh, dWd = y^T zd and db2;
 //   * bias gradients are seed-tile products (an N = 16 MMA of the same J planes against the three 16-bit terms of dov);
 //   * the two CTAs of a cluster are the two output halves of one item: they contract against the SAME Z quarter-tiles, each fetches
 //     half of every Z plane (and of the seed tile) and multicasts it to both - one L2 / DRAM read instead of two;
@@ -1211,10 +1148,10 @@ constexpr int ZH_PLANE = PT * H * 2;                // 16384
 constexpr int ZC_PLANE = PT * C * 2;                // 12288
 constexpr int X_BYTES = PT * 16 * 2;                // 1024 seed tile
 constexpr int ROW_PAD = 16;                         // bytes between staged output rows: 1040-byte pitch -> conflict-free 16-byte stores
-constexpr int ITEMS = 3;                            // work-item kinds per (sample, net)
+constexpr int ITEMS = 2;                            // work-item kinds per (sample, net)
 constexpr int NSTG_MAX = 5;
 template <int PL>
-struct Cfg {                                        // stage = J planes | Z1 planes (zp / zh / zc) | Z2 planes (zd) | seed tile
+struct Cfg {                                        // stage = J planes | Z1 planes (zp / zh) | Z2 planes (zd) | seed tile
   static constexpr int NSTG = PL == 2 ? 3 : 5;
   static constexpr int OFF_Z1 = PL * J_PLANE, OFF_Z2 = OFF_Z1 + PL * ZH_PLANE, OFF_X = OFF_Z2 + PL * ZC_PLANE;
   static constexpr int STAGE = OFF_X + X_BYTES;     // 74752 / 37888
@@ -1235,17 +1172,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
   int item = blockIdx.x;
   const int mh = item & 1; item >>= 1;                               // output half == cluster rank
   const int split = item % w.splits; item /= w.splits;
-  const int kind = item % wg2::ITEMS; item /= wg2::ITEMS;            // 0: dW1   1: dW2 + dWd (mask)   2: dWa (mask)
+  const int kind = item % wg2::ITEMS; item /= wg2::ITEMS;            // 0: dW1   1: dW2 + dWd (mask)
   const int k = item % w.Kn, b = item / w.Kn;
-  const int N1 = kind == 0 ? C : H;                                   // columns of the first Z tile (zp | zh | zc)
-  const bool two = kind == 1;                                         // second Z tile: zd, N = 192
-  const bool build_j = kind > 0;
+  const int N1 = kind == 0 ? C : H;                                   // columns of the first Z tile (zp | zh)
+  const bool mask_j = kind == 1;                                      // J built from the m3 mask bits; second Z tile: zd, N = 192
   const uint32_t z1plane = (uint32_t)wg2::PT * N1 * 2;                // bytes of one plane of a Z1 quarter-tile
   const int jsel = B_QM;
   const int t0 = (int)((long long)w.T * split / w.splits), t1 = (int)((long long)w.T * (split + 1) / w.splits);
   const int nst = 4 * (t1 - t0);                                      // quarter-tiles
   if (tid == 0) {
-    for (int s = 0; s < WG::NSTG; ++s) { mbar_init(&full[s], build_j ? 129 : 1); mbar_init(&empty[s], 2); }
+    for (int s = 0; s < WG::NSTG; ++s) { mbar_init(&full[s], mask_j ? 129 : 1); mbar_init(&empty[s], 2); }
     mbar_init(&acc_ready, 1);
     fence_barrier_init();
   }
@@ -1263,7 +1199,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
         const int t = t0 + (i >> 2), pq = i & 3;                      // tile, point quarter
         const uint8_t* nt = w.blobs + (((size_t)b * w.Kn + k) * w.T + t) * Geo<PL>::NET_TILE;
         const uint8_t* jsrc = nt + off_h<PL>(jsel) + (size_t)pq * (BLOB_H / 4) + (size_t)mh * wg2::J_PLANE;
-        const uint8_t* z1src = (kind == 0 ? nt + off_zp<PL>() : nt + off_h<PL>(kind == 1 ? B_ZH : B_ZC)) + (size_t)pq * z1plane;
+        const uint8_t* z1src = (kind == 0 ? nt + off_zp<PL>() : nt + off_h<PL>(B_ZH)) + (size_t)pq * z1plane;
         const uint32_t z1stride = kind == 0 ? BLOB_C : BLOB_H;          // plane stride of the Z1 tile in the workspace
         const uint8_t* z2src = nt + off_zd<PL>() + (size_t)pq * wg2::ZC_PLANE;
         const uint8_t* xsrc = nt + off_aux<PL>() + (size_t)pq * wg2::X_BYTES;
@@ -1271,13 +1207,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
         uint8_t* st = smem + s * WG::STAGE;
         mbar_wait(&empty[s], ((i / WG::NSTG) & 1) ^ 1);              // BOTH CTAs are done with the previous occupant (multicast commits)
         if (elect_one()) {
-          mbar_arrive_expect_tx(&full[s], (build_j ? 0 : PL * wg2::J_PLANE) + PL * z1plane + (two ? PL * wg2::ZC_PLANE : 0) + wg2::X_BYTES);
+          mbar_arrive_expect_tx(&full[s], (mask_j ? 0 : PL * wg2::J_PLANE) + PL * z1plane + (mask_j ? PL * wg2::ZC_PLANE : 0) + wg2::X_BYTES);
           const uint32_t zh = z1plane / 2, z2h = wg2::ZC_PLANE / 2, xh = wg2::X_BYTES / 2;
 #pragma unroll
           for (int p = 0; p < PL; ++p) {
-            if (!build_j) bulk_g2s(st + p * wg2::J_PLANE, jsrc + (size_t)p * BLOB_H, wg2::J_PLANE, &full[s]);
+            if (!mask_j) bulk_g2s(st + p * wg2::J_PLANE, jsrc + (size_t)p * BLOB_H, wg2::J_PLANE, &full[s]);
             bulk_g2s_mc(st + WG::OFF_Z1 + p * wg2::ZH_PLANE + mh * zh, z1src + (size_t)p * z1stride + mh * zh, zh, &full[s], (uint16_t)3);
-            if (two) bulk_g2s_mc(st + WG::OFF_Z2 + p * wg2::ZC_PLANE + mh * z2h, z2src + (size_t)p * BLOB_C + mh * z2h, z2h, &full[s], (uint16_t)3);
+            if (mask_j) bulk_g2s_mc(st + WG::OFF_Z2 + p * wg2::ZC_PLANE + mh * z2h, z2src + (size_t)p * BLOB_C + mh * z2h, z2h, &full[s], (uint16_t)3);
           }
           bulk_g2s_mc(st + WG::OFF_X + mh * xh, xsrc + mh * xh, xh, &full[s], (uint16_t)3);
         }
@@ -1305,15 +1241,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
             // every J plane is fetched from shared memory once per step for all MMAs that read it (A collector)
             if (PL == 1) {                                   // one plane per operand: J Z1 (+ J Z2) + J seeds
               mma_f16_c<A_FILL>(tmem, ad, b1, idesc1, first);
-              if (two) mma_f16_c<A_USE>(tmem + COL_D2, ad, b2, idesc2, first);
+              if (mask_j) mma_f16_c<A_USE>(tmem + COL_D2, ad, b2, idesc2, first);
               mma_f16_c<A_LAST>(tmem + COL_X, ad, xd, idesc_x, first);
-            } else if (build_j) {                            // exact one-plane J (the mask): J Z_lo + J Z_hi (+ J Z2 likewise) + J seeds
+            } else if (mask_j) {                             // exact one-plane J (the mask): J Z_lo + J Z_hi, J Z2 likewise, + J seeds
               mma_f16_c<A_FILL>(tmem, ad, b1 + b1_lo, idesc1, first);
               mma_f16_c<A_USE>(tmem, ad, b1, idesc1, 1u);
-              if (two) {
-                mma_f16_c<A_USE>(tmem + COL_D2, ad, b2 + b2_lo, idesc2, first);
-                mma_f16_c<A_USE>(tmem + COL_D2, ad, b2, idesc2, 1u);
-              }
+              mma_f16_c<A_USE>(tmem + COL_D2, ad, b2 + b2_lo, idesc2, first);
+              mma_f16_c<A_USE>(tmem + COL_D2, ad, b2, idesc2, 1u);
               mma_f16_c<A_LAST>(tmem + COL_X, ad, xd, idesc_x, first);
             } else {
               mma_f16_c<A_FILL>(tmem, ad + a_lo, b1, idesc1, first);
@@ -1322,7 +1256,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
               mma_f16_c<A_USE>(tmem, ad, b1, idesc1, 1u);
               mma_f16_c<A_LAST>(tmem + COL_X, ad, xd, idesc_x, 1u);
             }
-            if (two) {                                       // column sums: the Z half-tiles (all planes) against the column of ones
+            if (mask_j) {                                    // column sums: the Z half-tiles (all planes) against the column of ones
               const uint64_t zh_a = b1 + zh_half, zd_a = b2 + zd_half;
               mma_f16_c<A_DISCARD>(tmem + COL_SZH, zh_a, xd, idesc_x, first);
               if (PL == 2) mma_f16_c<A_DISCARD>(tmem + COL_SZH, zh_a + b1_lo, xd, idesc_x, 1u);
@@ -1335,7 +1269,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
       }
       if (elect_one()) mma_commit(&acc_ready);
     } else if (warp < 4) {
-      if (build_j) {
+      if (mask_j) {
         // J quarter-tile = [16 k-cores][32 points][8 features], one plane: thread = (point, 32-feature group gq): 4 pieces from one mask word
         const int pt = tid & 31, gq = tid >> 5;
         for (int i = 0; i < nst; ++i) {
@@ -1366,49 +1300,40 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
       if (F16) {
         const NetScales t = w.sc[gk];
         const float sj = kind == 0 ? t.sQ : 1.f;                       // (the mask carries no scale)
-        const float sz1 = kind == 0 ? t.sZP : (kind == 1 ? t.sZH : t.sZC);
+        const float sz1 = kind == 0 ? t.sZP : t.sZH;
         un1 = (1.f / sj) * (1.f / sz1); un2 = 1.f / t.sZD; un_x = (1.f / sj) * (1.f / t.sDV);   // separately: sj * sz may leave the fp32 range
       }
-      // kinds 1, 2: row `out` of m3^T z is scaled by u[out]; kind 2: this row of S = m3^T zc also gives the dot product with Wa[out,:]
-      // that vg needs
-      const float urow = build_j ? __ldg(w.uvec + (size_t)k * H + out) : 1.f;
-      const float* warow = w.Wa + ((size_t)k * H + out) * H;
-      float dot0 = 0.f, dot1 = 0.f;
+      // kind 1 accumulates m3^T z itself, not diag(u) m3^T z: fold_s_kernel needs the rows with u = 0 for vg (a net with wo = 0 has
+      // u = 0), and fold_gemm_kernel / unfold_b2_kernel apply diag(u) when they fold the sums into dW2, dWd, db2
       uint8_t* myrow = smem + (size_t)tid * (H * 4 + wg2::ROW_PAD);
       const uint32_t lane_base = tmem + ((uint32_t)(warp * 32) << 16);
       float v[32];
       {
-        float* dst = (kind == 0 ? w.gW1 + gk * H * C : kind == 1 ? w.gW2 + gk * H * H : w.gWa + (size_t)k * H * H) + (size_t)out * N1;
-        const float sc = un1 * urow;
+        float* dst = (kind == 0 ? w.gW1 + gk * H * C : w.gW2 + gk * H * H) + (size_t)out * N1;
+        const float sc = un1;
         for (int cb = 0; cb < N1 / 32; ++cb) {
           tmem_ld32(lane_base + cb * 32, v);
-          if (kind == 2) {
-#pragma unroll
-            for (int j4 = 0; j4 < 8; ++j4) {
-              const float4 wv = __ldg(reinterpret_cast<const float4*>(warow + cb * 32) + j4);
-              dot0 = fmaf(v[j4 * 4], wv.x, dot0); dot1 = fmaf(v[j4 * 4 + 1], wv.y, dot1);
-              dot0 = fmaf(v[j4 * 4 + 2], wv.z, dot0); dot1 = fmaf(v[j4 * 4 + 3], wv.w, dot1);
-            }
-          }
 #pragma unroll
           for (int j4 = 0; j4 < 8; ++j4)
             *reinterpret_cast<float4*>(myrow + cb * 128 + j4 * 16) =
-                (F16 || build_j) ? make_float4(v[j4 * 4] * sc, v[j4 * 4 + 1] * sc, v[j4 * 4 + 2] * sc, v[j4 * 4 + 3] * sc)
-                                 : make_float4(v[j4 * 4], v[j4 * 4 + 1], v[j4 * 4 + 2], v[j4 * 4 + 3]);
+                F16 ? make_float4(v[j4 * 4] * sc, v[j4 * 4 + 1] * sc, v[j4 * 4 + 2] * sc, v[j4 * 4 + 3] * sc)
+                    : make_float4(v[j4 * 4], v[j4 * 4 + 1], v[j4 * 4 + 2], v[j4 * 4 + 3]);
         }
         fence_proxy_async();                                           // my generic-proxy row -> visible to the bulk engine
         bulk_red_add_f32(dst, myrow, (uint32_t)N1 * 4u);
         bulk_commit();
       }
-      if (two) {                                                       // second output of the merged item: dWd rows (the staging row is reused)
+      if (mask_j) {                                                    // second output of the merged item: dWd rows (the staging row is reused)
         float* dst = w.gWd + (size_t)k * H * C + (size_t)out * C;
         bulk_wait_read_all();
-        const float sc = un2 * urow;
+        const float sc = un2;
         for (int cb = 0; cb < C / 32; ++cb) {
           tmem_ld32(lane_base + COL_D2 + cb * 32, v);
 #pragma unroll
           for (int j4 = 0; j4 < 8; ++j4)
-            *reinterpret_cast<float4*>(myrow + cb * 128 + j4 * 16) = make_float4(v[j4 * 4] * sc, v[j4 * 4 + 1] * sc, v[j4 * 4 + 2] * sc, v[j4 * 4 + 3] * sc);
+            *reinterpret_cast<float4*>(myrow + cb * 128 + j4 * 16) =
+                F16 ? make_float4(v[j4 * 4] * sc, v[j4 * 4 + 1] * sc, v[j4 * 4 + 2] * sc, v[j4 * 4 + 3] * sc)
+                    : make_float4(v[j4 * 4], v[j4 * 4 + 1], v[j4 * 4 + 2], v[j4 * 4 + 3]);
         }
         fence_proxy_async();
         bulk_red_add_f32(dst, myrow, (uint32_t)C * 4u);
@@ -1420,11 +1345,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
         const float bsum = (x[0] + x[1] + x[2]) * un_x;                // the three 16-bit terms of the seed
         if (kind == 0) {
           atomicAdd(w.gb1 + gk * H + out, bsum);
-        } else if (kind == 2) {                                        // bsum = sum_p m3[p,out] dov[p]
-          atomicAdd(w.gba + (size_t)k * H + out, urow * bsum);
-          atomicAdd(w.vg + (size_t)k * H + out, fmaf(__ldg(w.ba + (size_t)k * H + out), bsum, (dot0 + dot1) * un1));
-        } else {                                                       // u sm3; and the column sums of zh (features 128 mh + tid) and zd
-          atomicAdd(w.gb2 + gk * H + out, urow * bsum);                // (features 64 mh + tid: CTA 0 keeps [0, 96), CTA 1 [96, 192))
+        } else {                                                       // sm3; and the column sums of zh (features 128 mh + tid) and zd
+          atomicAdd(w.gb2 + gk * H + out, bsum);                       // (features 64 mh + tid: CTA 0 keeps [0, 96), CTA 1 [96, 192))
           tmem_ld16(lane_base + COL_SZH, x);
           float* scr = scratch(w.scr, w.scr_stride, (int)gk);
           atomicAdd(scr + SCR_SZH + out, F16 ? x[3] * (1.f / w.sc[gk].sZH) : x[3]);
@@ -1583,7 +1505,8 @@ __global__ void __launch_bounds__(256) seedmax_kernel(int Kn, size_t rows_per_sa
   }
 }
 
-// Z-side scales of this chunk from the seed maxima: zp = dov PE + xt, zh = dov h1 + ht, zc = dov c + ct, zd = dov PE6
+// Z-side scales of this chunk from the seed maxima: zp = dov PE + xt, zh = dov h1 + ht, zc = dov c + ct, zd = dov PE6.  zc is no
+// longer formed and sZC is read by no kernel; it is still computed so that the plan stays the one oracle/rescale.py restates.
 __global__ void zscale_kernel(int n, const int* __restrict__ seedmax, NetScales* __restrict__ tab) {
   const int bk = blockIdx.x * blockDim.x + threadIdx.x;
   if (bk >= n) return;
@@ -1597,10 +1520,10 @@ __global__ void zscale_kernel(int n, const int* __restrict__ seedmax, NetScales*
 }
 
 // ---- the fold of the reverse sweep (DESIGN.md section 3), fp32 on the CUDA cores ----------------------------------------
-// out[m][n] = rs[m] sum_l A(m, l) X[l][n] + xv[m] yv[n]  for one [H x N] X per batch (blockIdx.y), A = Wa of net batch % Kn:
-// A(m, l) = Wa[m][l] (AT = false: P = diag(u) Wa W2 before pass 1) or Wa[l][m] (AT = true: Wa^T (diag(u) m3^T z) + 2wo (x) sum_p z
-// after the last chunk).  rs, xv: [Kn][H] or nullptr; yv: [N] per batch, sY floats apart.  A CTA owns the 32-column block
-// blockIdx.x of all H rows and has read its whole block of X before it writes, so X may be out (in place).
+// out[m][n] = sum_l A(m, l) X[l][n] + xv[m] yv[n]  for one [H x N] X per batch (blockIdx.y), A = diag(rs) Wa of net batch % Kn:
+// A(m, l) = rs[m] Wa[m][l] (AT = false: P = diag(u) Wa W2 before pass 1) or rs[l] Wa[l][m] (AT = true: Wa^T diag(u) (m3^T z) +
+// 2wo (x) sum_p z after the last chunk).  rs, xv: [Kn][H] or nullptr; yv: [N] per batch, sY floats apart.  A CTA owns the
+// 32-column block blockIdx.x of all H rows and has read its whole block of X before it writes, so X may be out (in place).
 template <bool AT>
 __global__ void __launch_bounds__(256) fold_gemm_kernel(int Kn, int N, const float* __restrict__ Wa, const float* X, size_t sX, float* out,
                                                         size_t sOut, const float* __restrict__ rs, const float* __restrict__ xv,
@@ -1621,8 +1544,15 @@ __global__ void __launch_bounds__(256) fold_gemm_kernel(int Kn, int N, const flo
   for (int l0 = 0; l0 < H; l0 += 16) {
     __syncthreads();
     if (AT) {
-      for (int i = tid; i < 4 * H; i += 256)
-        *reinterpret_cast<float4*>(&As[i / (H / 4)][(i % (H / 4)) * 4]) = __ldg(reinterpret_cast<const float4*>(A + (size_t)(l0 + i / (H / 4)) * H) + i % (H / 4));
+      for (int i = tid; i < 4 * H; i += 256) {
+        const int l = i / (H / 4);
+        float4 v = __ldg(reinterpret_cast<const float4*>(A + (size_t)(l0 + l) * H) + i % (H / 4));
+        if (rs) {
+          const float s = rs[(size_t)k * H + l0 + l];
+          v.x *= s; v.y *= s; v.z *= s; v.w *= s;
+        }
+        *reinterpret_cast<float4*>(&As[l][(i % (H / 4)) * 4]) = v;
+      }
     } else {
       for (int i = tid; i < 4 * H; i += 256) {
         const int m = i >> 2, q = i & 3;
@@ -1651,7 +1581,7 @@ __global__ void __launch_bounds__(256) fold_gemm_kernel(int Kn, int N, const flo
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int m = ty * 8 + i;
-    const float r = rs ? rs[(size_t)k * H + m] : 1.f, xm = xv ? xv[(size_t)k * H + m] : 0.f;
+    const float r = (!AT && rs) ? rs[(size_t)k * H + m] : 1.f, xm = xv ? xv[(size_t)k * H + m] : 0.f;   // (AT: applied while staging)
     *reinterpret_cast<float4*>(out + (size_t)batch * sOut + (size_t)m * N + n0 + tx * 4) =
         make_float4(fmaf(r, acc[i][0], xm * y[0]), fmaf(r, acc[i][1], xm * y[1]), fmaf(r, acc[i][2], xm * y[2]), fmaf(r, acc[i][3], xm * y[3]));
   }
@@ -1670,12 +1600,13 @@ __global__ void __launch_bounds__(H) c2_kernel(int Kn, const float* __restrict__
   if (i == 0) t[SCR_SDO] = 0.f;
 }
 
-// Per (sample, net), after the last chunk: db2 = Wa^T (u sm3) + 2wo sum_p dov (G.b2 holds u sm3), de = db2, dbd = sum_b db2
-__global__ void __launch_bounds__(H) unfold_b2_kernel(int Kn, const float* __restrict__ Wa, const float* __restrict__ wo2, uint8_t* scr,
-                                                      size_t stride, float* gb2, float* ge, float* gbd) {
+// Per (sample, net), after the last chunk: db2 = Wa^T (u sm3) + 2wo sum_p dov (G.b2 holds sm3 = m3^T dov), de = db2, dbd = sum_b db2
+__global__ void __launch_bounds__(H) unfold_b2_kernel(int Kn, const float* __restrict__ Wa, const float* __restrict__ uvec,
+                                                      const float* __restrict__ wo2, uint8_t* scr, size_t stride, float* gb2, float* ge,
+                                                      float* gbd) {
   __shared__ float v[H];
   const int bk = blockIdx.x, k = bk % Kn, j = threadIdx.x;
-  v[j] = gb2[(size_t)bk * H + j];
+  v[j] = __ldg(uvec + (size_t)k * H + j) * gb2[(size_t)bk * H + j];
   __syncthreads();
   const float* wa = Wa + (size_t)k * H * H;
   float s = __ldg(wo2 + (size_t)k * H + j) * scratch(scr, stride, bk)[SCR_SDO];
@@ -1683,6 +1614,130 @@ __global__ void __launch_bounds__(H) unfold_b2_kernel(int Kn, const float* __res
   gb2[(size_t)bk * H + j] = s;
   ge[(size_t)bk * H + j] = s;
   atomicAdd(gbd + (size_t)k * H + j, s);
+}
+
+// Per net, after the last chunk and before the unfold rewrites G.W2 / G.Wd / G.b2 in place: S = m3^T zc summed over the samples,
+// from the sums the weight-gradient kernel accumulated (zc = zh W2^T + zd Wd^T + dov bsum itself is never formed):
+//     S = sum_b (m3^T zh)_b W2_b^T + (sum_b m3^T zd) Wd^T + sum_b sm3_b (x) bsum_b          sm3 = m3^T dov
+// ->  dWa = diag(u) S,  dba = u sum_b sm3_b,  and the column sum of the never-formed tile gz = m3 (zc Wa^T + dov ba):
+//     vg[j] = sum_i Wa[j,i] S[j,i] + ba[j] sum_b sm3_b[j].
+// S is formed from the raw sums, not from diag(u) S: vg needs the rows where u = 0 (every row of a net with wo = 0).  The same
+// contraction with a mask of ones gives  vc = sum_p zc = sum_b [(sum_p zh)_b W2_b^T + (sum_p dov)_b bsum_b] + (sum_{b,p} zd) Wd^T.
+// Grid (H / RB + 1, Kn), 128 threads: CTA x < H / RB owns rows RB x .. RB x + RB - 1 of S_k, CTA H / RB the row vc_k (its other
+// rows are zero); each loops over the samples itself, so every sum has one fixed order and no atomics.  Thread (warp wr, lane):
+// rows 4 wr .. 4 wr + 3 of the block, columns lane + 32 e.  The K = KB slices of X (the rows of m3^T z) and of Y (W2_b, Wd) are
+// staged transposed in shared memory; the next slice's loads are in flight while the current one is contracted.
+namespace fs {
+constexpr int RB = 16, KB = 32, THREADS = 128;
+}
+__global__ void __launch_bounds__(fs::THREADS) fold_s_kernel(int B, int Kn, const float* __restrict__ W2, const float* __restrict__ Wd,
+                                                             const float* __restrict__ Wa, const float* __restrict__ ba,
+                                                             const float* __restrict__ uvec, const float* __restrict__ bsum,
+                                                             const float* __restrict__ gW2, const float* __restrict__ gWd,
+                                                             const float* __restrict__ gb2, uint8_t* scr, size_t stride, float* __restrict__ gWa,
+                                                             float* __restrict__ gba, float* __restrict__ vg, float* __restrict__ vc) {
+  using namespace fs;
+  __shared__ float Ys[KB][H + 1];                                    // pitch H + 1: the transposing stores are conflict-free
+  __shared__ __align__(16) float Xs[KB][RB];
+  const int tid = threadIdx.x, lane = tid & 31, wr = tid >> 5, k = blockIdx.y;
+  const bool vrow = blockIdx.x == H / RB;
+  const int j0 = vrow ? 0 : blockIdx.x * RB;
+  const bool idle = vrow && wr > 0;                                  // the vc CTA's rows 4 .. 15 are zero: warps 1 .. 3 only stage slices
+  constexpr int SPB = H / KB;                                        // K-slices per sample (W2 term); then C / KB for the Wd term
+  const int nsteps = B * SPB + C / KB;
+  float4 yr[KB * H / 4 / THREADS], xr;
+  auto load = [&](const int s) {
+    const float *X, *Y, *xv;
+    int ld, l0;
+    if (s < B * SPB) {
+      const size_t bk = (size_t)(s / SPB) * Kn + k;
+      X = gW2 + bk * H * H; Y = W2 + bk * H * H; ld = H; l0 = (s % SPB) * KB;
+      xv = scratch(scr, stride, (int)bk) + SCR_SZH;
+    } else {
+      X = gWd + (size_t)k * H * C; Y = Wd + (size_t)k * H * C; ld = C; l0 = (s - B * SPB) * KB;
+      xv = scratch(scr, stride, k) + SCR_SZD;
+    }
+#pragma unroll
+    for (int n = 0; n < KB * H / 4 / THREADS; ++n) {
+      const int idx = tid + THREADS * n, i = idx / (KB / 4), q = idx % (KB / 4);
+      yr[n] = __ldg(reinterpret_cast<const float4*>(Y + (size_t)i * ld + l0) + q);
+    }
+    static_assert(RB * KB / 4 == THREADS, "one float4 of the X slice per thread");
+    const int r = tid / (KB / 4), q = tid % (KB / 4);
+    if (!vrow) xr = *(reinterpret_cast<const float4*>(X + (size_t)(j0 + r) * ld + l0) + q);
+    else xr = r == 0 ? *(reinterpret_cast<const float4*>(xv + l0) + q) : make_float4(0.f, 0.f, 0.f, 0.f);
+  };
+  float acc[4][8], sm3[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+  for (int a = 0; a < 4; ++a)
+#pragma unroll
+    for (int e = 0; e < 8; ++e) acc[a][e] = 0.f;
+  load(0);
+  for (int s = 0; s < nsteps; ++s) {
+    __syncthreads();                                                 // every thread is done with the previous slice
+#pragma unroll
+    for (int n = 0; n < KB * H / 4 / THREADS; ++n) {
+      const int idx = tid + THREADS * n, i = idx / (KB / 4), q = idx % (KB / 4);
+      Ys[4 * q][i] = yr[n].x; Ys[4 * q + 1][i] = yr[n].y; Ys[4 * q + 2][i] = yr[n].z; Ys[4 * q + 3][i] = yr[n].w;
+    }
+    {
+      const int r = tid / (KB / 4), q = tid % (KB / 4);
+      Xs[4 * q][r] = xr.x; Xs[4 * q + 1][r] = xr.y; Xs[4 * q + 2][r] = xr.z; Xs[4 * q + 3][r] = xr.w;
+    }
+    __syncthreads();
+    if (s + 1 < nsteps) load(s + 1);
+    if (idle) continue;                                              // (warp-uniform; the barriers above are every thread's)
+    if (s < B * SPB && s % SPB == 0) {                               // sample b's rank-1 term sm3_b (x) bsum_b (vc: sum_p dov)
+      const size_t bk = (size_t)(s / SPB) * Kn + k;
+      float x[4];
+#pragma unroll
+      for (int a = 0; a < 4; ++a) {
+        x[a] = vrow ? (wr == 0 && a == 0 ? scratch(scr, stride, (int)bk)[SCR_SDO] : 0.f) : gb2[bk * H + j0 + 4 * wr + a];
+        sm3[a] += x[a];
+      }
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float y = __ldg(bsum + bk * H + lane + 32 * e);
+#pragma unroll
+        for (int a = 0; a < 4; ++a) acc[a][e] = fmaf(x[a], y, acc[a][e]);
+      }
+    }
+#pragma unroll 8
+    for (int l = 0; l < KB; ++l) {
+      const float4 xv = *reinterpret_cast<const float4*>(&Xs[l][4 * wr]);
+      const float x[4] = {xv.x, xv.y, xv.z, xv.w};
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float y = Ys[l][lane + 32 * e];
+#pragma unroll
+        for (int a = 0; a < 4; ++a) acc[a][e] = fmaf(x[a], y, acc[a][e]);
+      }
+    }
+  }
+  if (vrow) {
+    if (wr == 0) {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) vc[(size_t)k * H + lane + 32 * e] = acc[0][e];
+    }
+    return;
+  }
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    const size_t j = (size_t)k * H + j0 + 4 * wr + a;
+    const float uj = __ldg(uvec + j);
+    float dot = 0.f;
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      dot = fmaf(__ldg(Wa + j * H + lane + 32 * e), acc[a][e], dot);
+      gWa[j * H + lane + 32 * e] = uj * acc[a][e];
+    }
+#pragma unroll
+    for (int m = 16; m; m >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, m);
+    if (lane == 0) {
+      vg[j] = fmaf(__ldg(ba + j), sm3[a], dot);
+      gba[j] = uj * sm3[a];
+    }
+  }
 }
 
 // fp32 weight matrix [R_src x K_src] -> bf16 image in layout (*) ; transpose = image rows are source columns.
@@ -1951,11 +2006,7 @@ static int run_planes(const Job& J, cudaStream_t st) {
     DPN_CUDA_OK(cudaMemsetAsync(G.e, 0, BKn * H * 4, st));
     DPN_CUDA_OK(cudaMemsetAsync(G.Wd, 0, (size_t)Kn * H * C * 4, st));
     DPN_CUDA_OK(cudaMemsetAsync(G.bd, 0, (size_t)Kn * H * 4, st));
-    DPN_CUDA_OK(cudaMemsetAsync(G.Wa, 0, (size_t)Kn * H * H * 4, st));
-    DPN_CUDA_OK(cudaMemsetAsync(G.ba, 0, (size_t)Kn * H * 4, st));
-    DPN_CUDA_OK(cudaMemsetAsync(c.vc, 0, (size_t)Kn * H * 4, st));
-    DPN_CUDA_OK(cudaMemsetAsync(c.vg, 0, (size_t)Kn * H * 4, st));
-    DPN_CUDA_OK(cudaMemsetAsync(c.sdo, 0, (size_t)Kn * 4, st));
+    DPN_CUDA_OK(cudaMemsetAsync(c.sdo, 0, (size_t)Kn * 4, st));      // (G.Wa, G.ba, vc, vg: written whole by fold_s_kernel)
   }
   for (int p0 = 0; p0 < N; p0 += chunk) {
     const int P = min(chunk, N - p0);
@@ -1978,7 +2029,7 @@ static int run_planes(const Job& J, cudaStream_t st) {
     }
     w.pe_blob = c.pe_blob; w.pe6_blob = c.pe6_blob; w.pet = c.pet; w.blobs = c.blobs;
     w.o = c.o; w.od = c.od; w.dov = c.dov; w.dod = c.dod;
-    w.vc = c.vc; w.vg = c.vg; w.sdo = c.sdo;
+    w.sdo = c.sdo;
     w.sc = c.sc;
     w.scr = c.blobs; w.scr_stride = c.scr_stride;
     w.xfirst = J.shape.mode == DPN_MODE_F16X3A ? 1 : 0;
@@ -2035,11 +2086,10 @@ static int run_planes(const Job& J, cudaStream_t st) {
     pass2z_kernel<PL, F16><<<tiles, Geo<PL>::THREADS, p2z::Cfg<PL>::SMEM, st>>>(w);
     DPN_LAUNCH_OK();
     WgradWork ww;
-    ww.B = B; ww.Kn = Kn; ww.T = T; ww.blobs = c.blobs; ww.sc = c.sc; ww.uvec = c.uvec;
-    ww.Wa = Wt.Wa; ww.ba = Wt.ba; ww.vg = c.vg;
+    ww.B = B; ww.Kn = Kn; ww.T = T; ww.blobs = c.blobs; ww.sc = c.sc;
     ww.scr = c.blobs; ww.scr_stride = c.scr_stride;
-    ww.gW1 = G.W1; ww.gW2 = G.W2; ww.gWa = G.Wa; ww.gWd = G.Wd;
-    ww.gb1 = G.b1; ww.gb2 = G.b2; ww.ge = G.e; ww.gbd = G.bd; ww.gba = G.ba;
+    ww.gW1 = G.W1; ww.gW2 = G.W2; ww.gWd = G.Wd;
+    ww.gb1 = G.b1; ww.gb2 = G.b2; ww.ge = G.e; ww.gbd = G.bd;
     const int items = B * Kn * 2 * wg2::ITEMS;                            // x 2 output halves
     // point-splits per (sample, net, layer, out-half): fill whole waves of resident CTAs (148 SMs x CTAs per SM); every split
     // adds one fp32 red.add pass over the gradient tile, so prefer the smallest count within 2 % of the best wave efficiency
@@ -2075,16 +2125,21 @@ static int run_planes(const Job& J, cudaStream_t st) {
   }
 #endif
   if (want_bwd) {
-    // dW2 = Wa^T (diag(u) m3^T zh) + 2wo (x) sum_p zh, dWd likewise with zd, db2 = de, dbd (linear: once, after the last chunk)
+    // Linear in the sums over points, so once, after the last chunk.  First dWa, dba, vg, vc from G.W2 = m3^T zh, G.Wd = sum_b m3^T zd
+    // and G.b2 = sm3, which the unfold then rewrites in place: dW2 = Wa^T diag(u) (m3^T zh) + 2wo (x) sum_p zh, dWd likewise with zd,
+    // db2 = de, dbd.
     const DpnGrads& G = *J.grads;
     const float* s0 = scratch(c.blobs, c.scr_stride, 0);
-    fold_gemm_kernel<true><<<dim3(H / 32, B * Kn), 256, 0, st>>>(Kn, H, Wt.Wa, G.W2, (size_t)H * H, G.W2, (size_t)H * H, nullptr, c.wo2,
+    fold_s_kernel<<<dim3(H / fs::RB + 1, Kn), fs::THREADS, 0, st>>>(B, Kn, Wt.W2, Wt.Wd, Wt.Wa, Wt.ba, c.uvec, c.bsum, G.W2, G.Wd, G.b2,
+                                                                     c.blobs, c.scr_stride, G.Wa, G.ba, c.vg, c.vc);
+    DPN_LAUNCH_OK();
+    fold_gemm_kernel<true><<<dim3(H / 32, B * Kn), 256, 0, st>>>(Kn, H, Wt.Wa, G.W2, (size_t)H * H, G.W2, (size_t)H * H, c.uvec, c.wo2,
                                                                  s0 + SCR_SZH, c.scr_stride / 4);
     DPN_LAUNCH_OK();
-    fold_gemm_kernel<true><<<dim3(C / 32, Kn), 256, 0, st>>>(Kn, C, Wt.Wa, G.Wd, (size_t)H * C, G.Wd, (size_t)H * C, nullptr, c.wo2,
+    fold_gemm_kernel<true><<<dim3(C / 32, Kn), 256, 0, st>>>(Kn, C, Wt.Wa, G.Wd, (size_t)H * C, G.Wd, (size_t)H * C, c.uvec, c.wo2,
                                                              s0 + SCR_SZD, c.scr_stride / 4);
     DPN_LAUNCH_OK();
-    unfold_b2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.Wa, c.wo2, c.blobs, c.scr_stride, G.b2, G.e, G.bd);
+    unfold_b2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.Wa, c.uvec, c.wo2, c.blobs, c.scr_stride, G.b2, G.e, G.bd);
     DPN_LAUNCH_OK();
     if ((rc = f32::launch_finalize(Kn, Wt, c.vc, c.vg, c.sdo, G, st))) return rc;
   }
