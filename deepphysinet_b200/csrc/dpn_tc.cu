@@ -59,13 +59,12 @@ constexpr int AUX_BYTES = TP * 16 * 2;        // 4096   [128 x 16] 16-bit seed t
 constexpr int IMG_HC = H * C * 2;             // 98304
 constexpr int IMG_HH = H * H * 2;             // 131072
 constexpr int GEN_IMG = 2 * IMG_HC + 2 * IMG_HH;   // per (sample, net): W1, W1T, W2, P^T (P = diag(u) Wa W2)
-constexpr int STA_IMG = IMG_HC + 2 * IMG_HH;       // per net: Wd, Wa, one unused [256 x 256] slot (the workspace sizes are pinned)
-// Workspace tile of one (net, point tile):  YT QM ZH ZC | ZP ZD | AUX | MASK.  No kernel writes the YT or the ZC slot (y and zc are never
-// formed); the first tile of a (sample, net) keeps scratch() in YT (the workspace sizes are pinned).  Pass 2 runs as the forward pass of the combined row
+constexpr int STA_IMG = IMG_HC + IMG_HH;           // per net: Wd, Wa
+// Workspace tile of one (net, point tile):  QM ZH | ZP ZD | AUX | MASK.  Pass 2 runs as the forward pass of the combined row
 // (DESIGN.md section 3) and needs only the ReLU mask m1 of pass 1 (256 bits per point) instead of the h1 / c / g tiles (3 x 1 KB per
 // point), and the weight-gradient kernel builds its J operand [a3 > 0] from the m3 mask bits instead of reading a stored tile.
-constexpr int NBLOB_H = 4, NBLOB_C = 2;
-enum { B_YT = 0, B_QM, B_ZH, B_ZC };
+constexpr int NBLOB_H = 2, NBLOB_C = 2;
+enum { B_QM = 0, B_ZH };
 constexpr int MASK_BYTES = 2 * TP * 32;       // [m1 | m3][128 rows][8 words]
 
 // Sizes that depend on the number of operand planes PL (1: bf16; 2: hi + lo, bf16 or scaled fp16).  Planes of one tile are
@@ -116,8 +115,7 @@ struct Work {
   float *o, *od, *dov, *dod;   // [B*T*TP][Kn], [..][Kn][3]
   float* sdo;                  // [Kn] sum of dov
   const NetScales* sc;         // [B][Kn] scaling plan (fp16 variant only)
-  uint8_t* scr;                // per-(sample, net) scratch of the reverse sweep: scr + (b Kn + k) scr_stride (see scratch())
-  size_t scr_stride;
+  float* scr;                  // [B][Kn][SCR_FLOATS] scratch of the reverse sweep (see scratch())
   long long* phase_dbg;        // optional [kernel(2)][8] cycle counters (debug builds with DPN_PHASE_DEBUG=1), summed over CTAs
   int xfirst;                  // cross-first accumulation of G1 - G3 (DPN_MODE_F16X3A)
   int dbg_flags;               // DEBUG BUILDS ONLY (tools/build_debug.sh, DPN_DEBUG_FLAGS): 1 = no MMAs, 2 = empty epilogues, 4 = no tile stores
@@ -138,13 +136,11 @@ template <int PL> __device__ __forceinline__ uint8_t* blob_zp(uint8_t* nt) { ret
 template <int PL> __device__ __forceinline__ uint8_t* blob_zd(uint8_t* nt) { return nt + off_zd<PL>(); }
 template <int PL> __device__ __forceinline__ uint8_t* blob_aux(uint8_t* nt) { return nt + off_aux<PL>(); }
 template <int PL> __device__ __forceinline__ uint8_t* blob_mask(uint8_t* nt) { return nt + off_mask<PL>(); }
-// Per-(sample, net) scratch of the reverse sweep (fp32), in the YT slot of workspace tile index (b Kn + k) Tc, Tc = the tiles per
-// sample of a full chunk: no kernel writes a YT slot (DESIGN.md section 4), and the address is the same for every chunk of a call.
+// Per-(sample, net) scratch of the reverse sweep (fp32, SCR_FLOATS per (sample, net), bk = b Kn + k):
 //   c2 = 2 W2^T wo (pass 1, epilogue 4) | sum_p zh | sum_p dov | (b = 0 only) sum_{b,p} zd  - the last three accumulate over chunks
-// and enter vc (fold_s_kernel) and dW2, db2, dWd (fold_gemm_kernel, unfold_b2_kernel) after the last chunk.  P = diag(u) Wa W2 (fp32, [H][H]) is formed in the
-// QM .. ZC slots of the same tile before pass 1 of the first chunk writes them.
-enum { SCR_C2 = 0, SCR_SZH = H, SCR_SDO = 2 * H, SCR_SZD = 2 * H + 32 };   // float offsets
-__host__ __device__ __forceinline__ float* scratch(uint8_t* scr, size_t stride, int bk) { return reinterpret_cast<float*>(scr + (size_t)bk * stride); }
+// and enter vc (fold_s_kernel) and dW2, db2, dWd (fold_gemm_kernel, unfold_b2_kernel) after the last chunk.
+enum { SCR_C2 = 0, SCR_SZH = H, SCR_SDO = 2 * H, SCR_SZD = 2 * H + 32, SCR_FLOATS = 2 * H + 32 + C };   // float offsets
+__host__ __device__ __forceinline__ float* scratch(float* scr, int bk) { return scr + (size_t)bk * SCR_FLOATS; }
 
 // ------------------------------------------------------------------------------------------------
 // Small helpers
@@ -229,11 +225,10 @@ __device__ __forceinline__ void stg8(uint8_t* tile, uint32_t plane, uint32_t off
 struct NetScales {                       // one per (sample, net)
   float sW1, sW2, sWd, sWa;              // weight images (a matrix and its transpose share the factor)
   float sP;                              // the image of P^T, P = diag(u) Wa W2 (B operand of G4, whose A operand is the bare m3 mask)
-  float sH1, sC, sG, spare0, spare1, sQ; // tiles written by pass 1: h1, c, g, q*m1 (spare0 / 1 keep the pinned workspace size)
-  float M1, Mc, l1W1, l1W12;             // bounds of |h1|, |c|; L1(W1), L1(W1) L1(W2)
-  float rowB;                            // max(1, L1(W1), L1(W1) L1(W2)): growth of the pass-2 tangent row over its chain
+  float sH1, sC, sQ;                     // tiles written by pass 1: h1, c, q*m1
+  float M1, l1W1;                        // bound of |h1|; L1(W1)
   float cap;                             // largest sH1 * sW2 this (sample, net) can carry (plan_kernel takes the min over samples)
-  float sZP, sZH, sZC, sZD, sDV;         // Z-side tiles and the seed tile of the CURRENT chunk (zscale_kernel; no kernel reads sZC)
+  float sZP, sZH, sZD, sDV;              // Z-side tiles and the seed tile of the CURRENT chunk (zscale_kernel)
 };
 constexpr float S_PE = 1024.f;           // coordinate / data features lie in [-1, 1]
 constexpr float F16_TOP = 32768.f;       // bound -> 2^15 (fp16 max is 65504)
@@ -681,7 +676,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
         svec[V_BA * H + tid] = __ldg(w.ba + vk + tid);
         svec[V_U * H + tid] = __ldg(w.uvec + vk + tid);
         svec[V_WO2 * H + tid] = __ldg(w.wo2 + vk + tid) * (1.f / sC);
-        if (sweep) svec[V_C2 * H + tid] = scratch(w.scr, w.scr_stride, b * w.Kn + k)[SCR_C2 + tid] * sQ;
+        if (sweep) svec[V_C2 * H + tid] = scratch(w.scr, b * w.Kn + k)[SCR_C2 + tid] * sQ;
       }
       epi_bar<PL>();
       uint32_t m1w[NB];
@@ -1095,7 +1090,7 @@ __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(Geo<2>::THREAD
       epi_bar<PL>();
       if (tid == 0) {
         atomicAdd(w.sdo + k, *ssdo);
-        atomicAdd(scratch(w.scr, w.scr_stride, b * w.Kn + k) + SCR_SDO, *ssdo);
+        atomicAdd(scratch(w.scr, b * w.Kn + k) + SCR_SDO, *ssdo);
         *ssdo = 0.f;
       }
     }
@@ -1116,8 +1111,7 @@ struct WgradWork {
   int B, Kn, T, splits;
   const uint8_t* blobs;
   const NetScales* sc;
-  uint8_t* scr;            // per-(sample, net) scratch (see scratch()): sum_p zh, sum_p zd
-  size_t scr_stride;
+  float* scr;              // per-(sample, net) scratch (see scratch()): sum_p zh, sum_p zd
   float *gW1, *gW2, *gWd;
   float *gb1, *gb2, *ge, *gbd;
 };
@@ -1348,11 +1342,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(192, 1) wgrad2_kerne
         } else {                                                       // sm3; and the column sums of zh (features 128 mh + tid) and zd
           atomicAdd(w.gb2 + gk * H + out, bsum);                       // (features 64 mh + tid: CTA 0 keeps [0, 96), CTA 1 [96, 192))
           tmem_ld16(lane_base + COL_SZH, x);
-          float* scr = scratch(w.scr, w.scr_stride, (int)gk);
+          float* scr = scratch(w.scr, (int)gk);
           atomicAdd(scr + SCR_SZH + out, F16 ? x[3] * (1.f / w.sc[gk].sZH) : x[3]);
           tmem_ld16(lane_base + COL_SZD, x);
           if (mh == 0 ? tid < C / 2 : tid >= TP - C / 2)
-            atomicAdd(scratch(w.scr, w.scr_stride, k) + SCR_SZD + mh * (C - TP) + tid, F16 ? x[3] * (1.f / w.sc[gk].sZD) : x[3]);
+            atomicAdd(scratch(w.scr, k) + SCR_SZD + mh * (C - TP) + tid, F16 ? x[3] * (1.f / w.sc[gk].sZD) : x[3]);
         }
       }
       bulk_wait_read_all();                                            // the engine has read my row: shared memory may go away
@@ -1383,12 +1377,11 @@ __device__ __forceinline__ float block_max256(float v, float* red) {      // 256
 // One block per (sample, net): L1 norms / maxima of its matrices -> activation bounds and tile scales.
 __global__ void __launch_bounds__(1024) bounds_kernel(int Kn, const float* __restrict__ W1, const float* __restrict__ b1,
                                                      const float* __restrict__ W2, const float* __restrict__ Wd,
-                                                     const float* __restrict__ Wa, const float* __restrict__ ba,
-                                                     const float* __restrict__ bsum, const float* __restrict__ uvec,
-                                                     const float* __restrict__ wo2, const uint8_t* __restrict__ Pm, size_t p_stride,
-                                                     NetScales* __restrict__ tab) {   // Pm: fp32 P of (b, k) at Pm + bk p_stride, or nullptr
+                                                     const float* __restrict__ Wa, const float* __restrict__ bsum,
+                                                     const float* __restrict__ uvec, const float* __restrict__ wo2,
+                                                     const float* __restrict__ Pm, NetScales* __restrict__ tab) {   // Pm: [B][Kn][H][H] fp32 P, or nullptr
   __shared__ float red[8];
-  __shared__ float srow[8][H];                                       // per matrix row: L1 norm / maximum of W1, Wd, W2, Wa
+  __shared__ float srow[7][H];                                       // per matrix row: L1 norm / maximum of W1, Wd, W2; maximum of Wa
   // 1024 threads: the block reads ~1.4 MB and one SM's memory-level parallelism is what bounds it (48 blocks on 148 SMs)
   __shared__ float scol[2][4][H];                                    // partial column L1 norms of W2, Wa
   const int bk = blockIdx.x, k = bk % Kn, j = threadIdx.x & 255, part = threadIdx.x >> 8, lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
@@ -1398,25 +1391,25 @@ __global__ void __launch_bounds__(1024) bounds_kernel(int Kn, const float* __res
   const float* wa = Wa + (size_t)k * H * H;
   // row-wise quantities: one warp per row, lanes along the row (coalesced), shuffle reduction
   for (int row = wrp; row < H; row += 32) {
-    float a1 = 0.f, x1 = 0.f, ad = 0.f, xd = 0.f, a2 = 0.f, x2 = 0.f, aa = 0.f, xa = 0.f;
+    float a1 = 0.f, x1 = 0.f, ad = 0.f, xd = 0.f, a2 = 0.f, x2 = 0.f, xa = 0.f;
     for (int i = lane; i < C; i += 32) {
       const float a = fabsf(w1m[(size_t)row * C + i]), d = fabsf(wdm[(size_t)row * C + i]);
       a1 += a; x1 = fmaxf(x1, a); ad += d; xd = fmaxf(xd, d);
     }
     for (int i = lane; i < H; i += 32) {
       const float a = fabsf(w2[(size_t)row * H + i]), c = fabsf(wa[(size_t)row * H + i]);
-      a2 += a; x2 = fmaxf(x2, a); aa += c; xa = fmaxf(xa, c);
+      a2 += a; x2 = fmaxf(x2, a); xa = fmaxf(xa, c);
     }
 #pragma unroll
     for (int m = 16; m; m >>= 1) {
       a1 += __shfl_xor_sync(0xffffffffu, a1, m); x1 = fmaxf(x1, __shfl_xor_sync(0xffffffffu, x1, m));
       ad += __shfl_xor_sync(0xffffffffu, ad, m); xd = fmaxf(xd, __shfl_xor_sync(0xffffffffu, xd, m));
       a2 += __shfl_xor_sync(0xffffffffu, a2, m); x2 = fmaxf(x2, __shfl_xor_sync(0xffffffffu, x2, m));
-      aa += __shfl_xor_sync(0xffffffffu, aa, m); xa = fmaxf(xa, __shfl_xor_sync(0xffffffffu, xa, m));
+      xa = fmaxf(xa, __shfl_xor_sync(0xffffffffu, xa, m));
     }
     if (lane == 0) {
       srow[0][row] = a1; srow[1][row] = x1; srow[2][row] = ad; srow[3][row] = xd;
-      srow[4][row] = a2; srow[5][row] = x2; srow[6][row] = aa; srow[7][row] = xa;
+      srow[4][row] = a2; srow[5][row] = x2; srow[6][row] = xa;
     }
   }
   // column-wise L1 norms: thread (part, j) walks down a quarter of column j (coalesced across the block)
@@ -1434,35 +1427,33 @@ __global__ void __launch_bounds__(1024) bounds_kernel(int Kn, const float* __res
   c2 = (scol[0][0][j] + scol[0][1][j]) + (scol[0][2][j] + scol[0][3][j]);
   ca = (scol[1][0][j] + scol[1][1][j]) + (scol[1][2][j] + scol[1][3][j]);
   const float r1 = srow[0][j], m1 = srow[1][j], rd = srow[2][j], md = srow[3][j];
-  const float r2 = srow[4][j], m2 = srow[5][j], ra = srow[6][j], ma = srow[7][j];
+  const float r2 = srow[4][j], m2 = srow[5][j], ma = srow[6][j];
   const float l1W1 = block_max256(r1, red), M1 = block_max256(r1 + fabsf(b1[(size_t)bk * H + j]), red);
-  const float l1W2 = block_max256(r2, red), l1Wd = block_max256(rd, red), l1Wa = block_max256(ra, red);
+  const float l1W2 = block_max256(r2, red), l1Wd = block_max256(rd, red);
   const float cW2 = block_max256(c2, red), cWa = block_max256(ca, red);
   const float mW1 = block_max256(m1, red), mW2 = block_max256(m2, red), mWd = block_max256(md, red), mWa = block_max256(ma, red);
-  const float mBs = block_max256(fabsf(bsum[(size_t)bk * H + j]), red), mBa = block_max256(fabsf(ba[(size_t)k * H + j]), red);
+  const float mBs = block_max256(fabsf(bsum[(size_t)bk * H + j]), red);
   const float Mu = block_max256(fabsf(uvec[(size_t)k * H + j]), red), mWo2 = block_max256(fabsf(wo2[(size_t)k * H + j]), red);
   float mp = 0.f;                                                    // max |P|
   if (Pm) {
-    const float* pr = reinterpret_cast<const float*>(Pm + (size_t)bk * p_stride);
+    const float* pr = Pm + (size_t)bk * H * H;
     for (int i = 0; i < H; ++i) mp = fmaxf(mp, fabsf(pr[(size_t)i * H + j]));
   }
   const float mP = block_max256(mp, red);
   if (j == 0) {
     NetScales t;
-    const float Mc = l1W2 * M1 + l1Wd + mBs, Mg = l1Wa * Mc + mBa;
+    const float Mc = l1W2 * M1 + l1Wd + mBs;
     const float My = Mu * cWa + mWo2, Mq = My * cW2;
     t.sW1 = scale_for(mW1 * 32.f);                   // weights: maximum -> 2^10
     t.sWa = scale_for(mWa * 32.f);
     t.sP = scale_for(mP * 32.f);
     t.sWd = scale_for(mWd * 32.f);                   // preliminary: plan_kernel couples sWd, sH1 and sW2
     t.sW2 = scale_for(mW2);                          // preliminary: the LARGEST admissible factor
-    t.sH1 = scale_for(M1); t.sC = scale_for(Mc); t.sG = scale_for(Mg);
-    t.spare0 = t.spare1 = 1.f;
+    t.sH1 = scale_for(M1); t.sC = scale_for(Mc);
     t.sQ = scale_for(Mq);
-    t.M1 = M1; t.Mc = Mc; t.l1W1 = l1W1; t.l1W12 = l1W1 * l1W2;
-    t.rowB = fmaxf(1.f, fmaxf(l1W1, l1W1 * l1W2));
+    t.M1 = M1; t.l1W1 = l1W1;
     t.cap = t.sH1 * t.sW2;
-    t.sZP = t.sZH = t.sZC = t.sZD = t.sDV = 1.f;
+    t.sZP = t.sZH = t.sZD = t.sDV = 1.f;
     tab[bk] = t;
   }
 }
@@ -1505,8 +1496,7 @@ __global__ void __launch_bounds__(256) seedmax_kernel(int Kn, size_t rows_per_sa
   }
 }
 
-// Z-side scales of this chunk from the seed maxima: zp = dov PE + xt, zh = dov h1 + ht, zc = dov c + ct, zd = dov PE6.  zc is no
-// longer formed and sZC is read by no kernel; it is still computed so that the plan stays the one oracle/rescale.py restates.
+// Z-side scales of this chunk from the seed maxima: zp = dov PE + xt, zh = dov h1 + ht, zd = dov PE6
 __global__ void zscale_kernel(int n, const int* __restrict__ seedmax, NetScales* __restrict__ tab) {
   const int bk = blockIdx.x * blockDim.x + threadIdx.x;
   if (bk >= n) return;
@@ -1514,7 +1504,6 @@ __global__ void zscale_kernel(int n, const int* __restrict__ seedmax, NetScales*
   const float DV = __int_as_float(seedmax[bk * 2]), RR = 16.f * __int_as_float(seedmax[bk * 2 + 1]);   // |dPE/dz| <= 2^4
   t.sZP = scale_for(DV + RR);
   t.sZH = scale_for(DV * t.M1 + RR * t.l1W1);
-  t.sZC = scale_for(DV * t.Mc + RR * t.l1W12);
   t.sZD = scale_for(DV);
   t.sDV = scale_for(DV);
 }
@@ -1588,12 +1577,12 @@ __global__ void __launch_bounds__(256) fold_gemm_kernel(int Kn, int N, const flo
 }
 
 // Per (sample, net), before pass 1: c2 = 2 W2^T wo, and the sums the weight-gradient kernels accumulate over chunks start at 0
-__global__ void __launch_bounds__(H) c2_kernel(int Kn, const float* __restrict__ W2, const float* __restrict__ wo2, uint8_t* scr, size_t stride) {
+__global__ void __launch_bounds__(H) c2_kernel(int Kn, const float* __restrict__ W2, const float* __restrict__ wo2, float* scr) {
   const int bk = blockIdx.x, k = bk % Kn, i = threadIdx.x;
   const float* w2 = W2 + (size_t)bk * H * H;
   float s = 0.f;
   for (int j = 0; j < H; ++j) s = fmaf(__ldg(wo2 + (size_t)k * H + j), __ldg(w2 + (size_t)j * H + i), s);
-  float* t = scratch(scr, stride, bk);
+  float* t = scratch(scr, bk);
   t[SCR_C2 + i] = s;
   t[SCR_SZH + i] = 0.f;
   if (i < C) t[SCR_SZD + i] = 0.f;
@@ -1602,14 +1591,13 @@ __global__ void __launch_bounds__(H) c2_kernel(int Kn, const float* __restrict__
 
 // Per (sample, net), after the last chunk: db2 = Wa^T (u sm3) + 2wo sum_p dov (G.b2 holds sm3 = m3^T dov), de = db2, dbd = sum_b db2
 __global__ void __launch_bounds__(H) unfold_b2_kernel(int Kn, const float* __restrict__ Wa, const float* __restrict__ uvec,
-                                                      const float* __restrict__ wo2, uint8_t* scr, size_t stride, float* gb2, float* ge,
-                                                      float* gbd) {
+                                                      const float* __restrict__ wo2, float* scr, float* gb2, float* ge, float* gbd) {
   __shared__ float v[H];
   const int bk = blockIdx.x, k = bk % Kn, j = threadIdx.x;
   v[j] = __ldg(uvec + (size_t)k * H + j) * gb2[(size_t)bk * H + j];
   __syncthreads();
   const float* wa = Wa + (size_t)k * H * H;
-  float s = __ldg(wo2 + (size_t)k * H + j) * scratch(scr, stride, bk)[SCR_SDO];
+  float s = __ldg(wo2 + (size_t)k * H + j) * scratch(scr, bk)[SCR_SDO];
   for (int l = 0; l < H; ++l) s = fmaf(__ldg(wa + (size_t)l * H + j), v[l], s);
   gb2[(size_t)bk * H + j] = s;
   ge[(size_t)bk * H + j] = s;
@@ -1634,7 +1622,7 @@ __global__ void __launch_bounds__(fs::THREADS) fold_s_kernel(int B, int Kn, cons
                                                              const float* __restrict__ Wa, const float* __restrict__ ba,
                                                              const float* __restrict__ uvec, const float* __restrict__ bsum,
                                                              const float* __restrict__ gW2, const float* __restrict__ gWd,
-                                                             const float* __restrict__ gb2, uint8_t* scr, size_t stride, float* __restrict__ gWa,
+                                                             const float* __restrict__ gb2, float* scr, float* __restrict__ gWa,
                                                              float* __restrict__ gba, float* __restrict__ vg, float* __restrict__ vc) {
   using namespace fs;
   __shared__ float Ys[KB][H + 1];                                    // pitch H + 1: the transposing stores are conflict-free
@@ -1652,10 +1640,10 @@ __global__ void __launch_bounds__(fs::THREADS) fold_s_kernel(int B, int Kn, cons
     if (s < B * SPB) {
       const size_t bk = (size_t)(s / SPB) * Kn + k;
       X = gW2 + bk * H * H; Y = W2 + bk * H * H; ld = H; l0 = (s % SPB) * KB;
-      xv = scratch(scr, stride, (int)bk) + SCR_SZH;
+      xv = scratch(scr, (int)bk) + SCR_SZH;
     } else {
       X = gWd + (size_t)k * H * C; Y = Wd + (size_t)k * H * C; ld = C; l0 = (s - B * SPB) * KB;
-      xv = scratch(scr, stride, k) + SCR_SZD;
+      xv = scratch(scr, k) + SCR_SZD;
     }
 #pragma unroll
     for (int n = 0; n < KB * H / 4 / THREADS; ++n) {
@@ -1692,7 +1680,7 @@ __global__ void __launch_bounds__(fs::THREADS) fold_s_kernel(int B, int Kn, cons
       float x[4];
 #pragma unroll
       for (int a = 0; a < 4; ++a) {
-        x[a] = vrow ? (wr == 0 && a == 0 ? scratch(scr, stride, (int)bk)[SCR_SDO] : 0.f) : gb2[bk * H + j0 + 4 * wr + a];
+        x[a] = vrow ? (wr == 0 && a == 0 ? scratch(scr, (int)bk)[SCR_SDO] : 0.f) : gb2[bk * H + j0 + 4 * wr + a];
         sm3[a] += x[a];
       }
 #pragma unroll
@@ -1862,11 +1850,11 @@ __global__ void gather_o_kernel(const Work w, float* __restrict__ o_out) {
 struct Carve {
   uint8_t *img_gen, *img_sta, *pe_blob, *pe6_blob, *blobs;
   float *pet, *o, *od, *dov, *dod, *uvec, *wo2, *cst, *bsum, *vc, *vg, *sdo;
+  float *scr, *P;               // reverse sweep: [B][Kn][SCR_FLOATS] scratch(), [B][Kn][H][H] P = diag(u) Wa W2
   float *lx, *ly, *lt, *lcd;    // lattice staging (values-only carve only)
   long long* dbg;
   NetScales* sc;
   int* seedmax;
-  size_t scr_stride;            // bytes between the scratch() of consecutive (sample, net): Tc workspace tiles
   size_t bytes;
 };
 
@@ -1901,8 +1889,9 @@ static Carve carve(uint8_t* base, int chunk, int Kn, int B, int pl, bool values_
     c.bytes = off;
     return c;
   }
-  c.scr_stride = T * (pl == 2 ? Geo<2>::NET_TILE : Geo<1>::NET_TILE);
-  c.blobs = take((size_t)B * Kn * c.scr_stride);
+  c.blobs = take((size_t)B * Kn * T * (pl == 2 ? Geo<2>::NET_TILE : Geo<1>::NET_TILE));
+  c.scr = reinterpret_cast<float*>(take((size_t)B * Kn * SCR_FLOATS * 4));
+  c.P = reinterpret_cast<float*>(take((size_t)B * Kn * H * H * 4));
   c.od = reinterpret_cast<float*>(take(rows * Kn * 12));
   c.dov = reinterpret_cast<float*>(take(rows * Kn * 4));
   c.dod = reinterpret_cast<float*>(take(rows * Kn * 12));
@@ -1931,7 +1920,7 @@ static int make_images(const DpnWeights& Wt, const Carve& c, const float* Pm, in
       {Wt.W1, (size_t)H * C, 0, GEN_IMG, H, C, 0, B * Kn, c.img_gen, 0},              // W1  : rows = out, k = in
       {Wt.W1, (size_t)H * C, IMG_HC, GEN_IMG, C, H, 1, B * Kn, c.img_gen, 0},         // W1T : rows = in,  k = out
       {Wt.W2, (size_t)H * H, 2 * IMG_HC, GEN_IMG, H, H, 0, B * Kn, c.img_gen, 1},
-      {Pm, c.scr_stride / 4, 2 * IMG_HC + IMG_HH, GEN_IMG, H, H, 1, Pm ? B * Kn : 0, c.img_gen, 4},   // P^T (G4 of the reverse sweep)
+      {Pm, (size_t)H * H, 2 * IMG_HC + IMG_HH, GEN_IMG, H, H, 1, Pm ? B * Kn : 0, c.img_gen, 4},   // P^T (G4 of the reverse sweep)
       {Wt.Wd, (size_t)H * C, 0, STA_IMG, H, C, 0, Kn, c.img_sta, 2},
       {Wt.Wa, (size_t)H * H, IMG_HC, STA_IMG, H, H, 0, Kn, c.img_sta, 3},
   };
@@ -1977,18 +1966,17 @@ static int run_planes(const Job& J, cudaStream_t st) {
   constexpr bool phase_debug = false;
 #endif
   if ((rc = f32::launch_prep(B, Kn, Wt, c.uvec, c.wo2, c.cst, c.bsum, st))) return rc;
-  // the reverse sweep's fold: P = diag(u) Wa W2 (fp32, in workspace tiles pass 1 has not written yet) and c2 = 2 W2^T wo
-  float* Pm = sweep ? reinterpret_cast<float*>(c.blobs + off_h<PL>(B_QM)) : nullptr;
+  // the reverse sweep's fold: P = diag(u) Wa W2 (fp32) and c2 = 2 W2^T wo
+  float* Pm = sweep ? c.P : nullptr;
   if (sweep) {
-    c2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.W2, c.wo2, c.blobs, c.scr_stride);
+    c2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.W2, c.wo2, c.scr);
     DPN_LAUNCH_OK();
-    fold_gemm_kernel<false><<<dim3(H / 32, B * Kn), 256, 0, st>>>(Kn, H, Wt.Wa, Wt.W2, (size_t)H * H, Pm, c.scr_stride / 4, c.uvec, nullptr,
+    fold_gemm_kernel<false><<<dim3(H / 32, B * Kn), 256, 0, st>>>(Kn, H, Wt.Wa, Wt.W2, (size_t)H * H, Pm, (size_t)H * H, c.uvec, nullptr,
                                                                   nullptr, 0);
     DPN_LAUNCH_OK();
   }
   if (F16) {                                                          // scaling plan before anything is converted to fp16
-    bounds_kernel<<<B * Kn, 1024, 0, st>>>(Kn, Wt.W1, Wt.b1, Wt.W2, Wt.Wd, Wt.Wa, Wt.ba, c.bsum, c.uvec, c.wo2,
-                                           reinterpret_cast<const uint8_t*>(Pm), c.scr_stride, c.sc);
+    bounds_kernel<<<B * Kn, 1024, 0, st>>>(Kn, Wt.W1, Wt.b1, Wt.W2, Wt.Wd, Wt.Wa, c.bsum, c.uvec, c.wo2, Pm, c.sc);
     DPN_LAUNCH_OK();
     plan_kernel<<<1, 32, 0, st>>>(B, Kn, c.sc);
     DPN_LAUNCH_OK();
@@ -2031,7 +2019,7 @@ static int run_planes(const Job& J, cudaStream_t st) {
     w.o = c.o; w.od = c.od; w.dov = c.dov; w.dod = c.dod;
     w.sdo = c.sdo;
     w.sc = c.sc;
-    w.scr = c.blobs; w.scr_stride = c.scr_stride;
+    w.scr = c.scr;
     w.xfirst = J.shape.mode == DPN_MODE_F16X3A ? 1 : 0;
     w.phase_dbg = phase_debug ? c.dbg : nullptr;
 #ifdef DPN_DEBUG_BUILD
@@ -2087,7 +2075,7 @@ static int run_planes(const Job& J, cudaStream_t st) {
     DPN_LAUNCH_OK();
     WgradWork ww;
     ww.B = B; ww.Kn = Kn; ww.T = T; ww.blobs = c.blobs; ww.sc = c.sc;
-    ww.scr = c.blobs; ww.scr_stride = c.scr_stride;
+    ww.scr = c.scr;
     ww.gW1 = G.W1; ww.gW2 = G.W2; ww.gWd = G.Wd;
     ww.gb1 = G.b1; ww.gb2 = G.b2; ww.ge = G.e; ww.gbd = G.bd;
     const int items = B * Kn * 2 * wg2::ITEMS;                            // x 2 output halves
@@ -2129,17 +2117,16 @@ static int run_planes(const Job& J, cudaStream_t st) {
     // and G.b2 = sm3, which the unfold then rewrites in place: dW2 = Wa^T diag(u) (m3^T zh) + 2wo (x) sum_p zh, dWd likewise with zd,
     // db2 = de, dbd.
     const DpnGrads& G = *J.grads;
-    const float* s0 = scratch(c.blobs, c.scr_stride, 0);
     fold_s_kernel<<<dim3(H / fs::RB + 1, Kn), fs::THREADS, 0, st>>>(B, Kn, Wt.W2, Wt.Wd, Wt.Wa, Wt.ba, c.uvec, c.bsum, G.W2, G.Wd, G.b2,
-                                                                     c.blobs, c.scr_stride, G.Wa, G.ba, c.vg, c.vc);
+                                                                     c.scr, G.Wa, G.ba, c.vg, c.vc);
     DPN_LAUNCH_OK();
     fold_gemm_kernel<true><<<dim3(H / 32, B * Kn), 256, 0, st>>>(Kn, H, Wt.Wa, G.W2, (size_t)H * H, G.W2, (size_t)H * H, c.uvec, c.wo2,
-                                                                 s0 + SCR_SZH, c.scr_stride / 4);
+                                                                 c.scr + SCR_SZH, SCR_FLOATS);
     DPN_LAUNCH_OK();
     fold_gemm_kernel<true><<<dim3(C / 32, Kn), 256, 0, st>>>(Kn, C, Wt.Wa, G.Wd, (size_t)H * C, G.Wd, (size_t)H * C, c.uvec, c.wo2,
-                                                             s0 + SCR_SZD, c.scr_stride / 4);
+                                                             c.scr + SCR_SZD, SCR_FLOATS);
     DPN_LAUNCH_OK();
-    unfold_b2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.Wa, c.uvec, c.wo2, c.blobs, c.scr_stride, G.b2, G.e, G.bd);
+    unfold_b2_kernel<<<B * Kn, H, 0, st>>>(Kn, Wt.Wa, c.uvec, c.wo2, c.scr, G.b2, G.e, G.bd);
     DPN_LAUNCH_OK();
     if ((rc = f32::launch_finalize(Kn, Wt, c.vc, c.vg, c.sdo, G, st))) return rc;
   }

@@ -5,8 +5,8 @@
 namespace dpn {
 namespace tc {
 
-constexpr int DEFAULT_POINTS_IN_FLIGHT = 1048576;  // B * chunk * planes: bounds the workspace (~41 KB per point in the split modes, ~29 KB in bf16 mode):
-                                                   // the B = 8 x 65 536 configuration runs as ONE pass over a 21 GB workspace
+constexpr int DEFAULT_POINTS_IN_FLIGHT = 1048576;  // B * chunk * planes: bounds the workspace (~24 KB per point in the split modes, ~13 KB in bf16 mode):
+                                                   // the B = 8 x 65 536 configuration runs as ONE pass over a 12.1 GiB workspace
 
 int default_chunk(int B, int planes);              // points per sample per pass (multiple of 128)
 size_t workspace_bytes(int chunk, int Kn, int B, int planes);

@@ -222,7 +222,7 @@ typedef struct DpnLattice {
 
 /* Bytes of device workspace dpn_decoder_lattice needs for this shape: the values-only part of the dpn_workspace_bytes carve
  * (weight images, coordinate / data features, outputs) plus per-point staging of x, y, t and coord_data - about 2.3 KB per point
- * in flight in the split modes against 41 KB for dpn_workspace_bytes. */
+ * in flight in the split modes against 24 KB for dpn_workspace_bytes. */
 int dpn_lattice_workspace_bytes(const DpnShape *shape, size_t *bytes);
 
 /* out[b, k, j, i, :] = o * std + mean (inverse_norm WITHOUT clip, as the reference's dense forward :533) of the six nets at node

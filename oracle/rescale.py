@@ -13,9 +13,9 @@ Each returns the new weights and the elementwise factor of every tensor.  Becaus
 to a tensor scaled by f is the old gradient divided by f (transform_grads).  With power-of-two factors every scaled fp32 weight is
 exact and every mask keeps its sign.
 
-scale_plan restates the plan in fp32 so that a test can say which scale or product boundary it targets.  Its L1 norms are summed
-in fp64 and rounded once, where the kernels sum in fp32: a bound that lies within an ulp of a power of two can land one binade
-apart, nowhere else.
+scale_plan restates the plan in fp32 so that a test can say which scale or product boundary it targets.  Its L1 norms and
+P = diag(u) Wa W2 are summed in fp64 and rounded once, where the kernels sum in fp32: a bound that lies within an ulp of a power
+of two can land one binade apart, nowhere else.
 """
 import torch
 
@@ -118,32 +118,31 @@ def scale_plan(W, seeds=None, chunk=None):
     """Per-(sample, net) scales [B, K] of one call, as the f16x3 kernels choose them (keys as NetScales in dpn_tc.cu).
 
     seeds: optional (dov [B,N,K], dod [B,N,K,3] or None), the seeds dL/do and dL/do_c of the call; then 'chunks' holds the Z-side
-    scales (sZP, sZH, sZC, sZD, sDV) of every chunk of `chunk` points (default: one chunk), which zscale_kernel derives from the
-    seed maxima of that chunk.  Also returns the bounds the scales come from and T2 [K], the coupled G2 scale of plan_kernel."""
+    scales (sZP, sZH, sZD, sDV) of every chunk of `chunk` points (default: one chunk), which zscale_kernel derives from the seed
+    maxima of that chunk.  Also returns the bounds the scales come from and T2 [K], the coupled G2 scale of plan_kernel."""
     g = {n: w.detach().double().cpu() for n, w in zip(W._fields, W)}
     B, K = g["W1"].shape[:2]
     bsum = _f32(_f32(g["b2"] + g["bd"]) + g["e"])                        # prep_kernel, in fp32
     uvec = _f32(torch.einsum("kij,ki->kj", g["Wb"], g["wo"]))
     wo2 = 2 * g["wo"]
+    P = _f32(uvec[None, :, :, None] * (g["Wa"][None] @ g["W2"]))         # P = diag(u) Wa W2 of fold_gemm_kernel, rounded to fp32
     rowL1 = lambda w: _f32(w.abs().sum(-1))
     l1W1 = rowL1(g["W1"]).amax(-1)
     M1 = _f32(rowL1(g["W1"]) + g["b1"].abs()).amax(-1)
-    l1W2, l1Wd, l1Wa = rowL1(g["W2"]).amax(-1), rowL1(g["Wd"]).amax(-1), rowL1(g["Wa"]).amax(-1)
+    l1W2, l1Wd = rowL1(g["W2"]).amax(-1), rowL1(g["Wd"]).amax(-1)
     cW2, cWa = _f32(g["W2"].abs().sum(-2)).amax(-1), _f32(g["Wa"].abs().sum(-2)).amax(-1)
     mW1, mW2 = g["W1"].abs().amax((-1, -2)), g["W2"].abs().amax((-1, -2))
     mWd, mWa = g["Wd"].abs().amax((-1, -2)), g["Wa"].abs().amax((-1, -2))
-    mBs, mBa = bsum.abs().amax(-1), g["ba"].abs().amax(-1)
+    mBs = bsum.abs().amax(-1)
     Mu, mWo2 = uvec.abs().amax(-1), wo2.abs().amax(-1)
-    mWaU = _f32(uvec.abs() * g["Wa"].abs().amax(-1)).amax(-1)
+    mP = P.abs().amax((-1, -2))
     Mc = _f32(_f32(l1W2 * M1) + l1Wd + mBs)
-    Mg = _f32(l1Wa * Mc + mBa)
     My = _f32(Mu * cWa + mWo2)
     Mq = _f32(My * cW2)
     bk = lambda v: v.expand(B, K) if v.dim() == 1 else v
-    t = dict(sW1=scale_for(mW1 * 32), sWa=bk(scale_for(mWa * 32)), sWaU=bk(scale_for(mWaU * 32)), sWd=bk(scale_for(mWd * 32)),
-             sW2=scale_for(mW2), sH1=scale_for(M1), sC=scale_for(Mc), sG=scale_for(Mg), sUM=bk(scale_for(Mu)), sY=bk(scale_for(My)),
-             sQ=scale_for(Mq))
-    t.update(M1=M1, Mc=Mc, l1W1=l1W1, l1W12=_f32(l1W1 * l1W2), My=My, Mq=Mq)
+    t = dict(sW1=scale_for(mW1 * 32), sWa=bk(scale_for(mWa * 32)), sP=scale_for(mP * 32), sWd=bk(scale_for(mWd * 32)),
+             sW2=scale_for(mW2), sH1=scale_for(M1), sC=scale_for(Mc), sQ=scale_for(Mq))
+    t.update(M1=M1, Mc=Mc, l1W1=l1W1, My=My, Mq=Mq, mP=mP)
     t["cap"] = t["sH1"] * t["sW2"]
     T2 = torch.minimum(S_PE * t["sWd"][0], t["cap"].amin(0))             # plan_kernel: one coupled scale per net
     t["T2"] = T2
@@ -158,12 +157,12 @@ def scale_plan(W, seeds=None, chunk=None):
             DV = _f32(dov[:, p0:p0 + chunk].abs().amax(1))
             RR = 16 * _f32(dod[:, p0:p0 + chunk].abs().amax((1, 3))) if dod is not None else torch.zeros_like(DV)
             t["chunks"].append(dict(DV=DV, RR=RR, sZP=scale_for(DV + RR), sZH=scale_for(_f32(DV * M1) + _f32(RR * l1W1)),
-                                    sZC=scale_for(_f32(DV * Mc) + _f32(RR * t["l1W12"])), sZD=scale_for(DV), sDV=scale_for(DV)))
+                                    sZD=scale_for(DV), sDV=scale_for(DV)))
     return t
 
 
-# the scale products the epilogues form in one step (pass 1: k1 .. i6) and those they form from split reciprocals
-PASS1_PRODUCTS = dict(k1=("S_PE", "sW1"), k2=("sH1", "sW2"), i3=("sC", "sWa"), i5=("sY", "sW2"), i6=("sQ", "sW1"))
+# the scale products the pass-1 epilogues form in one step (k1, k2, i3, i6; i4 = 1 / sP is a single scale)
+PASS1_PRODUCTS = dict(k1=("S_PE", "sW1"), k2=("sH1", "sW2"), i3=("sC", "sWa"), i6=("sQ", "sW1"))
 
 
 def boundaries(t):
@@ -171,7 +170,7 @@ def boundaries(t):
     product of PASS1_PRODUCTS outside the normal fp32 range [2^-126, 2^127].  Empty: every scale is a free power of two, so a
     uniform power-of-two reparametrisation shifts them exactly."""
     out = []
-    for n in ("sW1", "sW2", "sWd", "sWa", "sWaU", "sH1", "sC", "sG", "sUM", "sY", "sQ"):
+    for n in ("sW1", "sW2", "sWd", "sWa", "sP", "sH1", "sC", "sQ"):
         hit = (t[n] <= CLAMP_LO) | (t[n] >= CLAMP_HI)
         out += [(n, tuple(i)) for i in torch.nonzero(hit).tolist()]
     for n, (a, b) in PASS1_PRODUCTS.items():

@@ -61,8 +61,8 @@ def test_mode_enum_matches_header():
     need = C.c_size_t(0)
     bad = N.DpnShape(B=1, N=128, K=6, mode=max(N.MODES.values()) + 1, n_norm=0, seed_scale=1.0, chunk=0)
     assert N.lib().dpn_workspace_bytes(C.byref(bad), C.byref(need)) != 0
-    # the headline shape runs as one pass in every tensor-core mode; all of them keep the same tiles (YT QM ZH ZC | ZP ZD | seeds | masks),
-    # the split modes as two 16-bit planes, the bf16 mode as one: 18 vs 9.4 GB
+    # the headline shape runs as one pass in every tensor-core mode; all of them keep the same tiles (QM ZH | ZP ZD | seeds | masks),
+    # the split modes as two 16-bit planes, the bf16 mode as one: 12.1 vs 6.4 GiB
     sizes = {}
     for name, mode in N.MODES.items():
         shp = N.DpnShape(B=8, N=65536, K=6, mode=mode, n_norm=0, seed_scale=0.125, chunk=0)

@@ -159,7 +159,7 @@ def test_field_clipped_at_every_point_of_a_sample():
 # the closed interval [lo, hi]
 # ---------------------------------------------------------------------------------------------------------------------------------
 def interval_case(N=640, seed=440, guard=S.GUARD, device="cuda"):
-    """Nets p and T with wo = bo = 0, so o = coord_data exactly and u = Wb^T wo = 0 (the zero-u scale clamps sWaU, sUM, sY, sQ), and
+    """Nets p and T with wo = bo = 0, so o = coord_data exactly and u = Wb^T wo = 0 (so P = diag(u) Wa W2 = 0 and sP, sQ clamp), and
     a normalisation whose std is a power of two and mean a multiple of it, so o * std + mean is exact: p in [65536, 131072] (mean
     90112 = 11 * 8192, std 8192), T in [240, 368] (mean 288 = 18 * 16, std 16).  Four of five points sit on a bound of p and of T
     or one fp32 ulp outside it, the fifth inside.  Both nets then have a zero Jacobian and zero generated-weight gradients; kappa is

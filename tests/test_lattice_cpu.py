@@ -99,13 +99,14 @@ def test_exact_edges_are_inside():
     assert rc != DPN_E_INVALID, err
 
 
-@pytest.mark.parametrize("mode", ["bf16", "bf16x3", "f16x3", "f16x3a"])
-def test_lattice_workspace_is_a_tenth_of_the_full_one(mode):
-    """configs[3] of bench.py (one sample, 48 hourly leads on the 145 x 257 training grid) as one lattice job."""
-    Np = 48 * 145 * 257
-    lat = _bytes("dpn_lattice_workspace_bytes", 1, Np, mode)
-    full = _bytes("dpn_workspace_bytes", 1, Np, mode)
-    assert 10 * lat <= full, (lat, full)
+# configs[3] of bench.py (one sample, 48 hourly leads on the 145 x 257 training grid) as one lattice job: the values-only prefix
+# (weight images, features, outputs, scale plan) plus 36 B per point of lattice staging, about a tenth of dpn_workspace_bytes (1/8 in bf16)
+_LATTICE_PINNED = dict(bf16=1677677568, bf16x3=1247695872, f16x3=1247695872, f16x3a=1247695872)
+
+
+@pytest.mark.parametrize("mode", sorted(_LATTICE_PINNED))
+def test_lattice_workspace_sizes(mode):
+    assert _bytes("dpn_lattice_workspace_bytes", 1, 48 * 145 * 257, mode) == _LATTICE_PINNED[mode]
 
 
 @pytest.mark.parametrize("mode", ["fp32", "bf16", "bf16x3", "f16x3", "f16x3a"])
@@ -115,19 +116,23 @@ def test_refined_lattice_workspace_bound(mode):
     assert _bytes("dpn_lattice_workspace_bytes", 4, 577 * 1025 * 25, mode) < 1.6 * 2 ** 30
 
 
-# dpn_workspace_bytes of the parent commit: the values-only prefix re-orders the carve, it must not change its size.
+# dpn_workspace_bytes.  Tensor-core modes: per (sample, net) and tile of a chunk, QM ZH (2 x 64 KB per plane) | ZP ZD (2 x 48 KB per
+# plane) | seed tile (4 KB) | masks (8 KB); per (sample, net) the fold's scratch (SCR_FLOATS = 736 fp32) and P = diag(u) Wa W2
+# (256 x 256 fp32); every buffer rounded up to 1 KB.  That is the earlier carve without the two 128 KB tile slots no kernel wrote
+# (y and zc are not formed) and the unused [256 x 256] static weight slot, plus the scratch and P buffers those slots used to hold.
+# The values-only prefix and fp32 are as before.
 _PINNED = {
-    (1, 300, 0): dict(fp32=24972800, bf16=14781440, bf16x3=28740608, f16x3=28740608, f16x3a=28740608),
-    (2, 333, 0): dict(fp32=27722240, bf16=27371520, bf16x3=53127168, f16x3=53127168, f16x3a=53127168),
-    (8, 65536, 0): dict(fp32=1362174464, bf16=10090595328, bf16x3=19375801344, f16x3=19375801344, f16x3a=19375801344),
-    (1, 1788720, 0): dict(fp32=1362131456, bf16=20137610240, bf16x3=19337219072, f16x3=19337219072, f16x3a=19337219072),
-    (4, 14785625, 0): dict(fp32=1362149888, bf16=20145888256, bf16x3=19353754624, f16x3=19353754624, f16x3a=19353754624),
-    (3, 8120, 256): dict(fp32=21326336, bf16=25214976, bf16x3=49201152, f16x3=49201152, f16x3a=49201152),
+    (1, 300, 0): dict(fp32=24972800, bf16=12440576, bf16x3=22467584, f16x3=22467584, f16x3a=22467584),
+    (2, 333, 0): dict(fp32=27722240, bf16=23474176, bf16x3=42151936, f16x3=42151936, f16x3a=42151936),
+    (8, 65536, 0): dict(fp32=1362174464, bf16=6881305600, bf16x3=12944499712, f16x3=12944499712, f16x3a=12944499712),
+    (1, 1788720, 0): dict(fp32=1362131456, bf16=13695964160, bf16x3=12894786560, f16x3=12894786560, f16x3a=12894786560),
+    (4, 14785625, 0): dict(fp32=1362149888, bf16=13709011968, bf16x3=12916091904, f16x3=12916091904, f16x3a=12916091904),
+    (3, 8120, 256): dict(fp32=21326336, bf16=24481792, bf16x3=42962944, f16x3=42962944, f16x3a=42962944),
 }
 
 
 @pytest.mark.parametrize("key", sorted(_PINNED))
-def test_full_workspace_sizes_unchanged(key):
+def test_full_workspace_sizes(key):
     B, Np, chunk = key
     for mode, want in _PINNED[key].items():
         assert _bytes("dpn_workspace_bytes", B, Np, mode, chunk) == want, (key, mode)

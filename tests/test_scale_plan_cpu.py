@@ -93,16 +93,16 @@ def _const_weights(B=2, K=2):
     return W
 
 
-def test_scale_plan_by_hand():
+def test_kernel_scale_plan_by_hand():
     """mW1 = 2^-3 -> sW1 = pow2_floor(2^15 / 2^2) = 2^13;  M1 = 192 / 8 = 24 -> sH1 = 2^10;  mW2 = 2^-8 -> cap = 2^10 2^23 = 2^33;
     mWd = 2^-4 -> S_PE sWd = 2^10 2^14 = 2^24 = T2 -> sWd = 2^14, sW2 = 2^14;  Mc = L1(W2) M1 + L1(Wd) = 24 + 12 -> sC = 2^9;
-    u = 0 and wo = 0 -> sUM, sY, sQ, sWaU at the 2^80 clamp."""
+    u = 0 and wo = 0 -> P = diag(u) Wa W2 = 0, and sQ, sP at the 2^80 clamp."""
     t = R.scale_plan(_const_weights())
-    want = dict(sW1=13, sH1=10, sWd=14, sW2=14, sC=9, sWa=15 - (-6 + 5), sUM=80, sY=80, sQ=80, sWaU=80)
+    want = dict(sW1=13, sH1=10, sWd=14, sW2=14, sC=9, sWa=15 - (-6 + 5), sQ=80, sP=80)
     for n, e in want.items():
         assert torch.equal(t[n], torch.full_like(t[n], 2.0 ** e)), (n, R.log2(t[n]))
     assert torch.equal(t["T2"], torch.full((2,), 2.0 ** 24))
-    assert {n for n, _ in R.boundaries(t)} == {"sUM", "sY", "sQ", "sWaU"}
+    assert {n for n, _ in R.boundaries(t)} == {"sQ", "sP"}
 
 
 def test_cross_sample_minimum():
@@ -137,16 +137,18 @@ def test_clamps_and_z_scales():
     assert torch.equal(c1["sDV"], torch.full((2, 2), 2.0 ** 45)) and torch.equal(c1["sZP"], torch.full((2, 2), 2.0 ** 45))
 
 
-def test_uniform_moves_shift_the_plan_exactly(draw):
+def test_uniform_moves_shift_the_kernel_scales_exactly(draw):
     W, _ = draw
     t0 = R.scale_plan(W)
+    # P = diag(u) Wa W2: R2 divides W2 of (1, 2) by 2^16, so sP rises by 16; R3 keeps u = Wb^T wo and multiplies Wa by 2^16 and
+    # W2 by 2^-16, so P and sP do not move
     t = R.scale_plan(R.r2(W, 16, 1, 2)[0])
-    for n, e in dict(sW1=-16, sH1=-16, sW2=16, sQ=16, sWd=0, sC=0, sWa=0, sWaU=0, sY=0, sG=0, sUM=0).items():
+    for n, e in dict(sW1=-16, sH1=-16, sW2=16, sQ=16, sP=16, sWd=0, sC=0, sWa=0).items():
         want = t0[n].clone()
         want[1, 2] *= 2.0 ** e
         assert torch.equal(t[n], want), n
     t = R.scale_plan(R.r3(W, -16, 4)[0])
-    for n, e in dict(sC=16, sWa=-16, sWaU=-16, sY=-16, sWd=16, sW2=16, sH1=0, sW1=0, sQ=0, sG=0, sUM=0).items():
+    for n, e in dict(sC=16, sWa=-16, sWd=16, sW2=16, sH1=0, sW1=0, sQ=0, sP=0).items():
         want = t0[n].clone()
         want[:, 4] *= 2.0 ** e
         assert torch.equal(t[n], want), n
@@ -154,7 +156,7 @@ def test_uniform_moves_shift_the_plan_exactly(draw):
 
 def test_predicted_boundaries_of_the_uniform_sweeps(draw):
     """The sweeps of tests/test_gpu_scale_plan.py stay inside the plan up to +-40 and name their first boundary; no pass-1
-    product (k1 .. i6) leaves the fp32 range before one of its factors is clamped."""
+    product (k1, k2, i3, i6) leaves the fp32 range before one of its factors is clamped."""
     W, _ = draw
     up = range(1, 100)
     b = {(m, s): R.first_boundary(W, (lambda W, a, m=m, s=s: (R.r2(W, s * a, 0, 0) if m == "R2" else R.r3(W, s * a, 0))[0]), up)
