@@ -72,7 +72,7 @@ _lib = None
 ABI_VERSION = 2
 EXPORTS = ("dpn_abi_version", "dpn_last_error", "dpn_workspace_bytes", "dpn_pde_fwd_bwd", "dpn_pde_margin_fwd_bwd",
            "dpn_decoder_fwd", "dpn_decoder_bwd", "dpn_sample_field", "dpn_generate_queries", "dpn_last_launch_count",
-           "dpn_lattice_workspace_bytes", "dpn_decoder_lattice")
+           "dpn_lattice_workspace_bytes", "dpn_decoder_lattice", "dpn_decoder_jac_fwd", "dpn_decoder_jac_bwd")
 
 
 def lib():
@@ -103,6 +103,10 @@ def lib():
         L.dpn_lattice_workspace_bytes.argtypes = [C.POINTER(DpnShape), C.POINTER(C.c_size_t)]
         L.dpn_decoder_lattice.argtypes = [C.POINTER(DpnShape), C.POINTER(DpnConsts), C.POINTER(DpnLattice), C.POINTER(DpnSampler),
                                           C.c_void_p, C.POINTER(DpnWeights), C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+        L.dpn_decoder_jac_fwd.argtypes = [C.POINTER(DpnShape), C.POINTER(DpnConsts), C.POINTER(DpnPoints), C.POINTER(DpnWeights),
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+        L.dpn_decoder_jac_bwd.argtypes = [C.POINTER(DpnShape), C.POINTER(DpnConsts), C.POINTER(DpnPoints), C.POINTER(DpnWeights),
+                                          C.c_void_p, C.c_void_p, C.POINTER(DpnGrads), C.c_void_p, C.c_size_t, C.c_void_p]
         if L.dpn_abi_version() != ABI_VERSION:
             raise RuntimeError("libdpn_b200.so ABI version mismatch")
         _lib = L

@@ -227,6 +227,46 @@ int dpn_decoder_bwd(const DpnShape* shape, const DpnConsts* consts, const DpnPoi
   return dispatch(job, cuda_stream);
 }
 
+// Argument checks shared by dpn_decoder_jac_fwd / _bwd (all before the device is touched).
+static int check_fields(const char* fn, const DpnShape* shape, const DpnConsts* consts, const DpnPoints* pts, const DpnWeights* w) {
+  int rc = check_shape(shape);
+  if (rc) return rc;
+  if (!consts || !pts || !w) { set_error("%s: consts / points / weights is NULL", fn); return DPN_E_INVALID; }
+  if (pts->coord_pe) { set_error("%s: coord_pe must be NULL: the Jacobian is taken against x, y, t", fn); return DPN_E_INVALID; }
+  if (!(pts->x && pts->y && pts->t)) { set_error("%s: x, y and t are required", fn); return DPN_E_INVALID; }
+  if ((rc = check_common(shape, consts, pts, w))) return rc;
+  if (!pts->ref && shape->K != 6) { set_error("%s: ref may only be NULL for K = 6", fn); return DPN_E_INVALID; }
+  return 0;
+}
+
+int dpn_decoder_jac_fwd(const DpnShape* shape, const DpnConsts* consts, const DpnPoints* pts, const DpnWeights* w, float* o, float* jac,
+                        void* workspace, size_t workspace_bytes, void* cuda_stream) {
+  int rc = check_fields("dpn_decoder_jac_fwd", shape, consts, pts, w);
+  if (rc) return rc;
+  if (!o || !jac) { set_error("dpn_decoder_jac_fwd: o / jac is NULL"); return DPN_E_INVALID; }
+  Job job;
+  memset(&job, 0, sizeof(job));
+  job.kind = JOB_JAC_FWD; job.shape = *shape; job.dc = make_dev_consts(*consts);
+  job.pts = pts; job.w = w; job.o = o; job.jac = jac;
+  job.workspace = workspace; job.workspace_bytes = workspace_bytes;
+  return dispatch(job, cuda_stream);
+}
+
+int dpn_decoder_jac_bwd(const DpnShape* shape, const DpnConsts* consts, const DpnPoints* pts, const DpnWeights* w, const float* d_o,
+                        const float* d_jac, const DpnGrads* grads, void* workspace, size_t workspace_bytes, void* cuda_stream) {
+  int rc = check_fields("dpn_decoder_jac_bwd", shape, consts, pts, w);
+  if (rc) return rc;
+  if (!d_o && !d_jac) { set_error("dpn_decoder_jac_bwd: d_o and d_jac are both NULL"); return DPN_E_INVALID; }
+  if (!grads) { set_error("dpn_decoder_jac_bwd: grads is NULL"); return DPN_E_INVALID; }
+  if ((rc = check_grads(grads))) return rc;
+  Job job;
+  memset(&job, 0, sizeof(job));
+  job.kind = JOB_JAC_BWD; job.shape = *shape; job.dc = make_dev_consts(*consts);
+  job.pts = pts; job.w = w; job.d_o = d_o; job.d_jac = d_jac; job.grads = grads;
+  job.workspace = workspace; job.workspace_bytes = workspace_bytes;
+  return dispatch(job, cuda_stream);
+}
+
 int dpn_lattice_workspace_bytes(const DpnShape* shape, size_t* bytes) {
   int rc = check_shape(shape);
   if (rc) return rc;

@@ -451,9 +451,39 @@ __global__ void __launch_bounds__(256) finalize_kernel(const float* __restrict__
   if (blockIdx.y == 0 && threadIdx.x == 0) gbo[k] = sd;
 }
 
-__global__ void copy_seed_kernel(size_t n, const float* __restrict__ src, float scale, float* __restrict__ dst) {
-  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) dst[i] = src[i] * scale;
+// Caller seeds -> workspace seeds, one thread per point, blockIdx.y = sample (srow / sq as residual_kernel):
+//   dov[p,k] = d_o[q,k] scale;  dod[p,k,c] = d_jac[q,k,c] sc_c scale - the chain rule from the caller's physical units into the
+//   normalised z = (x / (dx (W-1)), y / (dy (H-1)), t / t_span) that od and the residual's dod are taken against.
+__global__ void seed_in_kernel(const DevConsts K, int P, int Kn, const float* __restrict__ d_o, const float* __restrict__ d_jac,
+                               float scale, double scale_d, float* __restrict__ dov, float* __restrict__ dod, size_t srow, size_t sq) {
+  const size_t bs = blockIdx.y;
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= P) return;
+  const size_t row = bs * srow + p, q = bs * sq + p;
+  const double sc[3] = {K.sx, K.sy, K.st};
+  for (int k = 0; k < Kn; ++k) {
+    dov[row * Kn + k] = d_o ? d_o[q * Kn + k] * scale : 0.f;
+    if (dod) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c)
+        dod[(row * Kn + k) * 3 + c] = d_jac ? (float)((double)d_jac[(q * Kn + k) * 3 + c] * sc[c] * scale_d) : 0.f;
+    }
+  }
+}
+
+// The fields of dpn_decoder_jac_fwd: o_out[q,k] = o[p,k], jac[q,k,c] = od[p,k,c] sc_c (physical units, before inverse_norm).
+__global__ void fields_kernel(const DevConsts K, int P, int Kn, const float* __restrict__ o, const float* __restrict__ od,
+                              float* __restrict__ o_out, float* __restrict__ jac, size_t srow, size_t sq) {
+  const size_t bs = blockIdx.y;
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= P) return;
+  const size_t row = bs * srow + p, q = bs * sq + p;
+  const double sc[3] = {K.sx, K.sy, K.st};
+  for (int k = 0; k < Kn; ++k) {
+    o_out[q * Kn + k] = o[row * Kn + k];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) jac[(q * Kn + k) * 3 + c] = (float)((double)od[(row * Kn + k) * 3 + c] * sc[c]);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -522,8 +552,11 @@ int run(const Job& J, cudaStream_t st) {
   Workspace w = carve(reinterpret_cast<char*>(J.workspace), chunk, Kn, B, lattice);
   const DpnWeights& Wt = *J.w;
   const bool pde = J.kind == JOB_PDE;
+  const bool jac_fwd = J.kind == JOB_JAC_FWD;
   const bool want_bwd = J.grads != nullptr;
-  const bool need_sweep = pde || (J.kind == JOB_DEC_BWD);   // reverse sweep (J-side vectors)
+  const bool need_sweep = pde || jac_fwd || J.kind == JOB_DEC_BWD || J.kind == JOB_JAC_BWD;   // reverse sweep (J-side vectors)
+  const bool want_od = pde || jac_fwd;                       // G6 and the Jacobian itself: the backward never reads od
+  const bool tangent = pde || J.d_jac != nullptr;           // seeds on the Jacobian: the tangent row (dod, G7 - G9) in the backward
   const double inv_n = 1.0 / (double)(J.shape.n_norm > 0 ? J.shape.n_norm : N);
   const double seed_scale = J.shape.seed_scale != 0.f ? (double)J.shape.seed_scale : 1.0;
 
@@ -599,11 +632,17 @@ int run(const Job& J, cudaStream_t st) {
       g = mk(P, H, H, w.YT, H, sH, Wt.W2 + gW2, H, (size_t)H * H, w.QM, sH);
       g.mask = w.H1; g.sMask = sH;
       if ((rc = launch_gemm(g, NN, Kn, st))) return rc;
-      if (pde) {
+      if (want_od) {
         g = mk(P, C, H, w.QM, H, sH, Wt.W1 + gW1, C, (size_t)H * C, w.JIN, sC);
         if ((rc = launch_gemm(g, NN, Kn, st))) return rc;
         jac_kernel<<<dim3(gp, Kn), pb, 0, st>>>(DC, P, Kn, w.JIN, pe, w.od);
         DPN_LAUNCH_OK();
+      }
+      if (jac_fwd) {
+        if ((rc = launch_fields(DC, 1, P, Kn, 0, 0, w.o, w.od, J.o + q0 * Kn, J.jac + q0 * Kn * 3, st))) return rc;
+        continue;
+      }
+      if (pde) {
         residual_kernel<<<(P + 255) / 256, 256, 0, st>>>(DC, P, w.o, w.od, J.pts->f + q0, inv_n, seed_scale,
                                                          J.out->loss_terms + (size_t)b * 6, w.dov, w.dod,
                                                          J.out->vals ? J.out->vals + q0 * 6 : nullptr,
@@ -613,16 +652,16 @@ int run(const Job& J, cudaStream_t st) {
                                             w.dov, J.margin->o ? J.margin->o + q0 * 6 : nullptr, st)))
           return rc;
       } else {
-        const size_t n = (size_t)P * Kn;
-        copy_seed_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, J.d_o + q0 * Kn, (float)seed_scale, w.dov);
-        DPN_LAUNCH_OK();
+        if ((rc = launch_seed_in(DC, 1, P, Kn, 0, 0, J.d_o ? J.d_o + q0 * Kn : nullptr, J.d_jac ? J.d_jac + q0 * Kn * 3 : nullptr,
+                                 seed_scale, w.dov, tangent ? w.dod : nullptr, st)))
+          return rc;
       }
       if (!want_bwd) continue;
       const DpnGrads& G = *J.grads;
       // backward inputs and the combined tangent row
-      bwd_in_kernel<<<dim3(gp, Kn), pb, 0, st>>>(DC, P, Kn, pe, w.pe6, w.dov, pde ? w.dod : nullptr, w.JIN, w.ZP, w.ZD);
+      bwd_in_kernel<<<dim3(gp, Kn), pb, 0, st>>>(DC, P, Kn, pe, w.pe6, w.dov, tangent ? w.dod : nullptr, w.JIN, w.ZP, w.ZD);
       DPN_LAUNCH_OK();
-      if (pde) {
+      if (tangent) {
         // G7: HT = (XT W1^T) * [H1>0], ZH = HT + dov H1
         g = mk(P, H, C, w.JIN, C, sC, Wt.W1 + gW1, C, (size_t)H * C, w.HT, sH);
         g.mask = w.H1; g.sMask = sH; g.out2 = w.ZH; g.sOut2 = sH; g.addsrc = w.H1; g.sAdd = sH;
@@ -689,6 +728,20 @@ int launch_margin(int B, int P, size_t srow, size_t sq, const float* o, const fl
                   double seed_scale, double* loss, float* dov, float* o_out, cudaStream_t st) {
   margin_seed_kernel<<<dim3((P + 255) / 256, B), 256, 0, st>>>(P, o, target, M.beta, M.factor * inv_n / 6.0, seed_scale, loss, dov, o_out,
                                                                srow, sq);
+  DPN_LAUNCH_OK();
+  return 0;
+}
+
+int launch_seed_in(const DevConsts& DC, int B, int P, int Kn, size_t srow, size_t sq, const float* d_o, const float* d_jac,
+                   double seed_scale, float* dov, float* dod, cudaStream_t st) {
+  seed_in_kernel<<<dim3((P + 255) / 256, B), 256, 0, st>>>(DC, P, Kn, d_o, d_jac, (float)seed_scale, seed_scale, dov, dod, srow, sq);
+  DPN_LAUNCH_OK();
+  return 0;
+}
+
+int launch_fields(const DevConsts& DC, int B, int P, int Kn, size_t srow, size_t sq, const float* o, const float* od, float* o_out,
+                  float* jac, cudaStream_t st) {
+  fields_kernel<<<dim3((P + 255) / 256, B), 256, 0, st>>>(DC, P, Kn, o, od, o_out, jac, srow, sq);
   DPN_LAUNCH_OK();
   return 0;
 }

@@ -4,7 +4,8 @@
 
 namespace dpn {
 
-enum JobKind { JOB_PDE = 0, JOB_DEC_FWD = 1, JOB_DEC_BWD = 2, JOB_LATTICE = 3 };
+// JOB_JAC_FWD / JOB_JAC_BWD: dpn_decoder_jac_fwd / _bwd - values and Jacobian out, caller seeds on both in.
+enum JobKind { JOB_PDE = 0, JOB_DEC_FWD = 1, JOB_DEC_BWD = 2, JOB_LATTICE = 3, JOB_JAC_FWD = 4, JOB_JAC_BWD = 5 };
 
 // dpn_decoder_lattice, validated by dpn_api.cu: the lattice, the coarse stack it samples and the de-normalisation of the output.
 struct LatticeJob {
@@ -29,10 +30,12 @@ struct Job {
   const DpnWeights* w;
   const DpnPdeOut* out;     // JOB_PDE
   const DpnMargin* margin;  // JOB_PDE, optional: supervised SmoothL1 data loss on the same points
-  const DpnGrads* grads;    // JOB_PDE (optional), JOB_DEC_BWD
-  float* o;                 // JOB_DEC_FWD: normalised [B*N][K];  JOB_LATTICE: physical [B][N][6]
+  const DpnGrads* grads;    // JOB_PDE (optional), JOB_DEC_BWD, JOB_JAC_BWD
+  float* o;                 // JOB_DEC_FWD, JOB_JAC_FWD: normalised [B*N][K];  JOB_LATTICE: physical [B][N][6]
+  float* jac;               // JOB_JAC_FWD: [B*N][K][3] d o / d(x, y, t)
   LatticeJob lat;           // JOB_LATTICE
-  const float* d_o;         // JOB_DEC_BWD
+  const float* d_o;         // JOB_DEC_BWD; JOB_JAC_BWD (may be NULL)
+  const float* d_jac;       // JOB_JAC_BWD (may be NULL): [B*N][K][3]
   void* workspace;
   size_t workspace_bytes;
   int chunk;                // points per sample per internal pass
@@ -77,6 +80,13 @@ int launch_residual(const DevConsts& DC, int B, int P, size_t srow, size_t sq, c
                     double inv_n, double seed_scale, double* loss6, float* dov, float* dod, float* vals, float* jac, cudaStream_t st);
 int launch_margin(int B, int P, size_t srow, size_t sq, const float* o, const float* target, const DpnMargin& M, double inv_n,
                   double seed_scale, double* loss, float* dov, float* o_out, cudaStream_t st);
+// Caller seeds of P points per sample (samples srow workspace rows / sq caller points apart) -> dov [..][Kn], dod [..][Kn][3]
+// (dod may be NULL: values-only backward); a NULL d_o / d_jac is a zero seed.
+int launch_seed_in(const DevConsts& DC, int B, int P, int Kn, size_t srow, size_t sq, const float* d_o, const float* d_jac,
+                   double seed_scale, float* dov, float* dod, cudaStream_t st);
+// o [..][Kn], od [..][Kn][3] of the workspace -> the caller's o [B*N][Kn] and jac = od (sx, sy, st) [B*N][Kn][3].
+int launch_fields(const DevConsts& DC, int B, int P, int Kn, size_t srow, size_t sq, const float* o, const float* od, float* o_out,
+                  float* jac, cudaStream_t st);
 int launch_finalize(int Kn, const DpnWeights& Wt, const float* vc, const float* vg, const float* sdo, const DpnGrads& G,
                     cudaStream_t st);
 

@@ -1823,17 +1823,6 @@ __global__ void __launch_bounds__(TP) encode_kernel(const DevConsts K, const Wor
   }
 }
 
-__global__ void seed_copy_kernel(const Work w, const float* __restrict__ d_o, float scale) {
-  // values-only backward: dov[row][k] = d_o[q][k] * scale for valid rows
-  const size_t row = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= (size_t)w.B * w.T * TP) return;
-  const int tile = (int)(row / TP), r = (int)(row % TP);
-  const int b = tile / w.T, tl = tile % w.T;
-  const int p_local = tl * TP + r;
-  for (int k = 0; k < w.Kn; ++k)
-    w.dov[row * w.Kn + k] = p_local < w.P ? d_o[((size_t)b * w.N + w.p0 + p_local) * w.Kn + k] * scale : 0.f;
-}
-
 __global__ void gather_o_kernel(const Work w, float* __restrict__ o_out) {
   const size_t row = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (row >= (size_t)w.B * w.T * TP) return;
@@ -1955,7 +1944,10 @@ static int run_planes(const Job& J, cudaStream_t st) {
   const DpnWeights& Wt = *J.w;
   const bool pde = J.kind == JOB_PDE;
   const bool want_bwd = J.grads != nullptr;
-  const int sweep = pde ? 2 : (J.kind == JOB_DEC_BWD ? 1 : 0);
+  // sweep 2 forms the Jacobian od (G6), sweep 1 only the reverse sweep the backward needs.  dpn_decoder_jac_bwd recomputes the pass 1
+  // of dpn_decoder_jac_fwd with sweep 1, and the two runs must decide the same ReLU masks: they differ in G6 alone, because the plan
+  // takes Pm (sweep >= 1) and f16x3a its cross-first accumulation (sweep > 0) in both.  Keep every other sweep test that way.
+  const int sweep = (pde || J.kind == JOB_JAC_FWD) ? 2 : ((J.kind == JOB_DEC_BWD || J.kind == JOB_JAC_BWD) ? 1 : 0);
   const double inv_n = 1.0 / (double)(J.shape.n_norm > 0 ? J.shape.n_norm : N);
   const double seed_scale = J.shape.seed_scale != 0.f ? (double)J.shape.seed_scale : 1.0;
   int rc;
@@ -2045,6 +2037,12 @@ static int run_planes(const Job& J, cudaStream_t st) {
       DPN_LAUNCH_OK();
       continue;
     }
+    if (J.kind == JOB_JAC_FWD) {
+      if ((rc = f32::launch_fields(J.dc, B, P, Kn, (size_t)T * TP, (size_t)N, c.o, c.od, J.o + (size_t)p0 * Kn, J.jac + (size_t)p0 * Kn * 3,
+                                   st)))
+        return rc;
+      continue;
+    }
     if (want_bwd || pde) {
       DPN_CUDA_OK(cudaMemsetAsync(c.dov, 0, rows * Kn * 4, st));
       DPN_CUDA_OK(cudaMemsetAsync(c.dod, 0, rows * Kn * 12, st));
@@ -2058,9 +2056,11 @@ static int run_planes(const Job& J, cudaStream_t st) {
       if (J.margin && (rc = f32::launch_margin(B, P, srow, (size_t)N, c.o, J.margin->target + q0 * 6, *J.margin, inv_n, seed_scale,
                                                J.margin->loss, c.dov, J.margin->o ? J.margin->o + q0 * 6 : nullptr, st)))
         return rc;
-    } else {
-      seed_copy_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(w, J.d_o, (float)seed_scale);
-      DPN_LAUNCH_OK();
+    } else {                                                          // caller seeds; padding rows keep the zeros of the memsets
+      const size_t q0 = (size_t)p0;
+      if ((rc = f32::launch_seed_in(J.dc, B, P, Kn, (size_t)T * TP, (size_t)N, J.d_o ? J.d_o + q0 * Kn : nullptr,
+                                    J.d_jac ? J.d_jac + q0 * Kn * 3 : nullptr, seed_scale, c.dov, J.d_jac ? c.dod : nullptr, st)))
+        return rc;
     }
     if (!want_bwd) continue;
     const DpnGrads& G = *J.grads;

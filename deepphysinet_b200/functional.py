@@ -11,6 +11,7 @@ import ctypes as C
 from typing import NamedTuple, Optional
 
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _native as N
 from .config import PhysicsConsts
@@ -196,6 +197,59 @@ class DecoderValuesFn(torch.autograd.Function):
         return (None,) * 8 + tuple(g.to(dt) for g, dt in zip(grads, ctx.dtypes))
 
 
+class DecoderFieldsFn(torch.autograd.Function):
+    """(o [B,N,K], jac [B,N,K,3]) = DecoderFieldsFn.apply(x, y, t, coord_data, ref, consts, mode, *weights)
+
+    o are the normalised outputs of the K coordinate nets (as DecoderValuesFn), jac = d o / d(x, y, t) in physical units, before
+    inverse_norm / clip - what torch.autograd.grad(o_k, x) gives in the reference (interface_physics.py:90-95).  Both outputs are
+    differentiable w.r.t. the 13 DecoderWeights tensors; x, y, t, coord_data and ref are not (their gradients are None, as in
+    PDEResidualFn), so a loss written on (o, jac) in PyTorch trains the weights with the library's backward kernels.
+    The backward recomputes the forward from the saved inputs (dpn_decoder_jac_bwd) and is once-differentiable."""
+
+    @staticmethod
+    def forward(ctx, x, y, t, coord_data, ref, consts: PhysicsConsts, mode, *weights):
+        W = DecoderWeights(*weights)
+        B, K = _check_weights(W)
+        dev = W.W1.device
+        cd = _prep(coord_data, (B, -1, 6))
+        Np = cd.shape[1]
+        xs = [_prep(a, (B, Np)) for a in (x, y, t)]
+        rf = _prep(ref, (B, Np, K))
+        ws = [_prep(w) for w in W]
+        o = torch.empty(B, Np, K, device=dev)
+        jac = torch.empty(B, Np, K, 3, device=dev)
+        shape = _shape(B, Np, K, mode)
+        pts = N.DpnPoints(x=N.ptr(xs[0]), y=N.ptr(xs[1]), t=N.ptr(xs[2]), f=None, coord_pe=None, coord_data=cd.data_ptr(), ref=N.ptr(rf))
+        wsbuf, nbytes = N.workspace(shape, dev)
+        N.check(N.lib().dpn_decoder_jac_fwd(C.byref(shape), C.byref(N.make_consts(consts)), C.byref(pts), C.byref(_weights_struct(ws)),
+                                            N.ptr(o), N.ptr(jac), N.ptr(wsbuf), nbytes, N.stream_ptr()), "dpn_decoder_jac_fwd")
+        ctx.need = any(ctx.needs_input_grad[7:])
+        ctx.saved = (xs, cd, rf, ws, consts, mode, B, Np, K) if ctx.need else None
+        ctx.dtypes = [w.dtype for w in weights]
+        ctx.set_materialize_grads(False)                       # an unused output arrives as None and goes to the library as NULL
+        return o, jac
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_o, g_jac):
+        if not ctx.need:
+            return (None,) * 20
+        xs, cd, rf, ws, consts, mode, B, Np, K = ctx.saved
+        if g_o is None and g_jac is None:
+            return (None,) * 7 + tuple(torch.zeros_like(w, dtype=dt) for w, dt in zip(ws, ctx.dtypes))
+        dev = ws[0].device
+        grads = [torch.empty_like(w) for w in ws]
+        shape = _shape(B, Np, K, mode)
+        pts = N.DpnPoints(x=N.ptr(xs[0]), y=N.ptr(xs[1]), t=N.ptr(xs[2]), f=None, coord_pe=None, coord_data=cd.data_ptr(), ref=N.ptr(rf))
+        go = _prep(g_o, (B, Np, K))
+        gj = _prep(g_jac, (B, Np, K, 3))
+        wsbuf, nbytes = N.workspace(shape, dev)
+        N.check(N.lib().dpn_decoder_jac_bwd(C.byref(shape), C.byref(N.make_consts(consts)), C.byref(pts), C.byref(_weights_struct(ws)),
+                                            N.ptr(go), N.ptr(gj), C.byref(_grads_struct(grads)), N.ptr(wsbuf), nbytes, N.stream_ptr()),
+                "dpn_decoder_jac_bwd")
+        return (None,) * 7 + tuple(g.to(dt) for g, dt in zip(grads, ctx.dtypes))
+
+
 _DEFAULT_MODE = "f16x3"
 
 
@@ -266,6 +320,16 @@ def decoder_values(coord_pe, coord_data, W: DecoderWeights, ref=None, xyz=None, 
     x, y, t = xyz if xyz is not None else (None, None, None)
     o = DecoderValuesFn.apply(coord_pe, x, y, t, coord_data, ref, consts, mode or _DEFAULT_MODE, *W)
     return o[0] if coord_data.dim() == 2 else o
+
+
+def decoder_fields(x, y, t, coord_data, W: DecoderWeights, ref=None, consts: Optional[PhysicsConsts] = None, mode=None):
+    """(o, jac): the normalised outputs o [B,N,K] of the K nets and jac = d o / d(x, y, t) [B,N,K,3] in physical units (per metre,
+    per metre, per second), both differentiable w.r.t. the DecoderWeights tensors - the inputs of a PDE loss written in PyTorch
+    (deepphysinet_b200.physics).  x, y, t [B,N], coord_data [B,N,6], ref [B,N,K] (default: coord_data[..., k] for net k, K = 6);
+    [N] / [N,6] inputs give [N,K] / [N,K,3] (B = 1).  Gradients w.r.t. x, y, t, coord_data and ref are not computed (None)."""
+    consts = consts or PhysicsConsts()
+    o, jac = DecoderFieldsFn.apply(x, y, t, coord_data, ref, consts, mode or _DEFAULT_MODE, *W)
+    return (o[0], jac[0]) if coord_data.dim() == 2 else (o, jac)
 
 
 def sample_field(coarse, x, y, t, consts: Optional[PhysicsConsts] = None, cells_per_coarse=4.0, t_step=6 * 3600.0,

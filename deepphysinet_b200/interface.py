@@ -12,6 +12,7 @@ import torch
 import torch.nn as nn
 
 from . import functional as Fn
+from . import physics
 from .config import FACTOR_KEYS, TERM_NAMES, VAR_ORDER, PhysicsConsts
 from .pe import SineCosPE
 from .physics_net import PhysicsNet
@@ -97,9 +98,9 @@ class InterfacePhysics(nn.Module):
         """Same contract as interface_physics.py:271-320: returns the scalar PDE loss (sum of the six weighted
         residual MSEs) whose .backward() reaches every physics_net parameter.  Host tensors are moved to
         `device` exactly as the reference does (:273-276); batches of samples ([B,N,...]) are allowed and
-        give the mean over samples."""
-        if not isinstance(criterion, nn.MSELoss) or getattr(criterion, "reduction", "mean") != "mean":
-            raise NotImplementedError("the fused residual kernel implements nn.MSELoss() (losses/builder.py:10); got %r" % (criterion,))
+        give the mean over samples.  nn.MSELoss() (losses/builder.py:10) runs the fused residual kernel; any other
+        criterion runs the decoder fields (functional.decoder_fields) and the PyTorch physics (physics.residual_terms), which
+        call criterion(lhs, rhs) per sample and equation as the reference does."""
         dev = torch.device(device)
         f, x, y, t = (a.to(dev, non_blocking=True) for a in (f, x, y, t))
         field_data = field_data.to(dev, non_blocking=True)
@@ -108,8 +109,16 @@ class InterfacePhysics(nn.Module):
         B = field_data.shape[0]
         W = self.physics_net.decoder_weights(field_data, forecast_h)
         shp = (B, -1)
-        total, terms = Fn.pde_residual(x.reshape(shp), y.reshape(shp), t.reshape(shp), f.reshape(shp),
-                                       input_data.reshape(B, -1, 6), W, consts=self.consts(loss_factor), mode=self.mode)
+        consts = self.consts(loss_factor)
+        if isinstance(criterion, nn.MSELoss) and criterion.reduction == "mean":
+            total, terms = Fn.pde_residual(x.reshape(shp), y.reshape(shp), t.reshape(shp), f.reshape(shp),
+                                           input_data.reshape(B, -1, 6), W, consts=consts, mode=self.mode)
+        else:
+            o, jac = Fn.decoder_fields(x.reshape(shp), y.reshape(shp), t.reshape(shp), input_data.reshape(B, -1, 6), W,
+                                       consts=consts, mode=self.mode)
+            terms = physics.residual_terms(o, jac, f.reshape(shp), consts, criterion)
+            total = terms.sum(dim=1).mean()
+            terms = terms.detach()
         self.last_terms = terms
         if global_step % log_step == 1 and local_rank == 0:
             vals = terms.mean(dim=0).tolist()            # .item()-style sync, as in the reference's logging branch

@@ -169,6 +169,25 @@ int dpn_decoder_bwd(const DpnShape *shape, const DpnConsts *consts, const DpnPoi
                     const DpnWeights *w, const float *d_o, const DpnGrads *grads,
                     void *workspace, size_t workspace_bytes, void *cuda_stream);
 
+/* Differentiable decoder fields: the values of the K nets AND their first derivatives in x, y, t, so that any loss built from
+ * them (another criterion than MSE, a modified or extra equation, weights that need gradients) can be written by the caller and
+ * still run the decoder, the reverse sweep and the weight gradients here.  Arguments of both calls:
+ *   pts    x, y, t required; coord_pe must be NULL (the Jacobian is taken against x, y, t); f unused; ref as in dpn_decoder_fwd
+ *          (NULL only for K = 6)
+ *   shape  K = 1..6 in every mode; chunk honoured; n_norm ignored (the caller's loss owns its normalisation)
+ *   workspace  dpn_workspace_bytes(shape)
+ * o [B*N,K] normalised outputs, exactly as dpn_decoder_fwd;
+ * jac [B*N,K,3] = d o / d(x, y, t) in physical units (per metre, per metre, per second): what torch.autograd.grad(o_k, x)
+ * returns in the reference (interface_physics.py:90-95) BEFORE inverse_norm / clip. */
+int dpn_decoder_jac_fwd(const DpnShape *shape, const DpnConsts *consts, const DpnPoints *pts, const DpnWeights *w,
+                        float *o, float *jac, void *workspace, size_t workspace_bytes, void *cuda_stream);
+
+/* grads = seed_scale * d( sum d_o*o + sum d_jac*jac ) / d(every DpnWeights tensor), overwritten; o and jac as dpn_decoder_jac_fwd
+ * returns them (recomputed here, not read back).  d_o [B*N,K] or d_jac [B*N,K,3] may be NULL (a zero seed), not both. */
+int dpn_decoder_jac_bwd(const DpnShape *shape, const DpnConsts *consts, const DpnPoints *pts, const DpnWeights *w,
+                        const float *d_o, const float *d_jac, const DpnGrads *grads,
+                        void *workspace, size_t workspace_bytes, void *cuda_stream);
+
 /* Query-point producer (SURVEY 8(f) N2).  Replaces the CPU xarray trilinear interpolation of the normalised coarse
  * field stack (dataset/physics_dataset.py:477-486, :406-415, :567-576) and get_coriolis (:521-526).
  *   coarse     [B, Tt, Hc, Wc, 6]  normalised coarse field, channel-last (u10,v10,pres,t2,q2,rio)
